@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    # the reference-style CPU path (oracle port) on the host cores
+    python bench.py --steps K --warmup W --dump-outputs bench_outputs   # also write the headline's posteriors (seeded row sample)
 
 Headline workload = BASELINE.json configs[2], the configuration the metric's "at 1/2/4/8 B200" is quoted on: Alarm-shaped
 network (37 nodes, card <= 4), 16,777,216 evidence rows in total, row-sharded over the ranks (STRONG scaling), evidence =
@@ -38,6 +39,8 @@ ALARM_ROWS = 1 << 24
 L2_BYTES = 126 * 1024 * 1024
 METRIC = "posterior queries/sec (batched VE)"
 MIN_REGION_S = 0.060
+# --dump-outputs: 3 batches x 4 targets x 2^18 rows x 2 fp32 = 24 MiB of posteriors (the ring always holds >= 3 batches)
+DUMP_ROWS, DUMP_BATCHES, DUMP_SEED = 1 << 18, 3, 1250
 # identical in both arms (the driver compares them): what is computed, not how
 CONFIG = {"workload": "alarm-37node batched VE (BASELINE.json configs[2]): 16,777,216 evidence rows in total, 12 evidence "
                       "leaves drawn from the joint, 4 binary targets (HYPOVOLEMIA, LVFAILURE, KINKEDTUBE, PULMEMBOLUS)",
@@ -388,6 +391,35 @@ def verify_sharded_fit(env, spec, tables, seed, n_per_rank):
     return f"rank 0 recounted the {env.world} concatenated shards alone: tables and n_total bit-equal"
 
 
+def dump_headline_outputs(env, out_dir, out_ring, targets, first_row):
+    """--dump-outputs: the posteriors the last timed step of the headline left in the first DUMP_BATCHES batches of the ring
+    (every step covers the whole ring), at DUMP_ROWS rows drawn with a fixed seed from the 16M-row batch.  Row ids are global,
+    so the files do not depend on the number of GPUs.  Writes `<target>_batch<r>.npy` (float32 [DUMP_ROWS, card]) and
+    `rows.npy` (the sampled row ids, float64) on rank 0."""
+    import numpy as np
+
+    torch = env.torch
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(ALARM_ROWS, size=DUMP_ROWS, replace=False))
+    n_local = out_ring[0][0].shape[0]
+    mine = (idx >= first_row) & (idx < first_row + n_local)
+    src = torch.from_numpy(idx[mine] - first_row).to(env.dev)
+    dst = torch.from_numpy(np.nonzero(mine)[0]).to(env.dev)
+    arrays = {}
+    for r in range(DUMP_BATCHES):
+        for t, o in zip(targets, out_ring[r]):
+            a = torch.zeros((DUMP_ROWS, o.shape[1]), dtype=torch.float32, device=env.dev)
+            a[dst] = o.index_select(0, src)
+            if env.world > 1:
+                env.dist.all_reduce(a)          # every sampled row lives on exactly one rank: the sum is that rank's row
+            arrays[f"{t}_batch{r}"] = a
+    if env.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "rows.npy"), idx.astype(np.float64))
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+    env.barrier()
+
+
 # ---------------------------------------------------------------------------------------------- headline: Alarm VE
 def bench_alarm_ve(env, args):
     torch = env.torch
@@ -450,6 +482,8 @@ def bench_alarm_ve(env, args):
     q_s = env.max_over_ranks(e0.elapsed_time(e1) / 1e3)
     clocks = sampler.stop() if sampler else None
     env.barrier()
+    if args.dump_outputs:            # before any later leg writes into the ring's posteriors
+        dump_headline_outputs(env, args.dump_outputs, out_ring, tgs, s)
     launches = args.steps * P
     value = ALARM_ROWS * len(tgs) * launches / q_s
     roof = roofline(env, rows * bpr, q_s / launches, "gather_tiles_kernel<2,4>" if rows >= (1 << 21) else "gather_inter_kernel<2,4>",
@@ -1057,7 +1091,14 @@ def main():
     ap.add_argument("--cpu-budget-s", type=float, default=10.0)
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline posteriors of the last step (a fixed, seeded sample of rows) "
+                         "to DIR/<target>_batch<r>.npy, with the sampled row ids in DIR/rows.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

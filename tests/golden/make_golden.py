@@ -1,7 +1,8 @@
 """Generate golden fixtures by running the UNMODIFIED reference on CPU.
 
-Run in the build container only (``/root/reference`` does not exist on the GPU
-box): ``python tests/golden/make_golden.py``.  Writes ``tests/golden/*.npz``.
+Needs a source checkout of the reference (the directory that holds ``cbn/``) and no
+GPU: ``CBN_REFERENCE=<checkout> python tests/golden/make_golden.py``.  Writes
+``tests/golden/*.npz``.
 The reference imports ``gpytorch`` eagerly (cbn/parameter_learning/__init__.py:2)
 which is not installed; a dummy module tree in ``sys.modules`` is enough because
 only ``BruteForce`` is exercised (SURVEY.md section 8c).  No reference file is edited
@@ -14,7 +15,7 @@ import types
 
 import numpy as np
 
-REF = os.environ.get("CBN_REFERENCE", "/root/reference")
+REF = os.environ.get("CBN_REFERENCE", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -29,6 +30,8 @@ def _stub_gpytorch():
 
 
 def main():
+    if not REF or not os.path.isdir(os.path.join(REF, "cbn")):
+        sys.exit("set CBN_REFERENCE to a checkout of the reference (the directory that holds cbn/)")
     _stub_gpytorch()
     sys.path.insert(0, REF)
     import networkx as nx

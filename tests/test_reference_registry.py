@@ -1,7 +1,8 @@
 """INTEGRATION.md section 2, executed: the engine's classes are registered in the reference's OWN registries
 (cbn/parameter_learning/__init__.py:7-13, cbn/inference/__init__.py:3) and the reference's Node / factories dispatch into
-them.  Needs the reference tree (/root/reference: present in the build container, absent on the GPU box) -- and the build
-container has no GPU, so the call chain is followed up to the device boundary, where the engine must fail loudly
+them.  Needs a source checkout of the reference (Giovannibriglia/ContinuousBayesianNetwork, the directory that holds
+`cbn/`) named by the CBN_REFERENCE environment variable; the repository does not ship it, so without one the test
+skips.  Without a GPU the call chain is followed up to the device boundary, where the engine must fail loudly
 (there is no CPU fallback); what happens behind that boundary is covered by the golden-vector tests in test_fit_gpu.py,
 which make exactly the calls the reference's Node makes (estimator.fit(node_data, parents_data), get_prob(points, query))."""
 import os
@@ -11,12 +12,12 @@ import types
 import pytest
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("CBN_REFERENCE", "")
 
 
 def _import_reference():
-    if not os.path.isdir(os.path.join(REF, "cbn")):
-        pytest.skip("reference tree not present")
+    if not REF or not os.path.isdir(os.path.join(REF, "cbn")):
+        pytest.skip("no reference checkout (set CBN_REFERENCE to the directory that holds cbn/)")
     names = ["gpytorch"] + ["gpytorch." + s for s in ("models", "kernels", "means", "likelihoods", "mlls", "distributions", "settings")]
     for n in names:                       # the reference imports gpytorch eagerly (cbn/parameter_learning/__init__.py:2)
         sys.modules.setdefault(n, types.ModuleType(n))

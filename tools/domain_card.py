@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from continuousbayesiannetwork_b200 import synth
 from continuousbayesiannetwork_b200.engine import tables_from_spec
 dev = "cuda:0"
