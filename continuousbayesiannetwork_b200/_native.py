@@ -135,6 +135,11 @@ SIGNATURES = {
     "cbn_ve_run_f32": (C.c_int, [_P, _P, C.POINTER(_P), C.POINTER(_P), C.c_int64, _P, _P]),
     "cbn_ve_run_codes_map": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, _P, _P]),
     "cbn_ve_run_f32_map": (C.c_int, [_P, _P, C.POINTER(_P), C.POINTER(_P), C.c_int64, _P, _P, _P]),
+    "cbn_ve_run_codes_log_evidence": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, _P]),
+    "cbn_loglik_plan_create": (C.c_int, [_P, C.POINTER(Family), C.c_int32, C.c_int32, _P, _P, C.POINTER(_P)]),
+    "cbn_loglik_plan_destroy": (None, [_P]),
+    "cbn_loglik_run": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, C.c_int32, _P]),
+    "cbn_loglik_plan_tables": (C.c_int, [_P]),
     "cbn_ve_run_codes_host": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P]),
     "cbn_ve_run_codes_host_multi": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P)]),
     "cbn_ve_run_codes_host_multi_ex": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P), C.c_int32]),

@@ -12,6 +12,8 @@ or undefined, SURVEY.md section 3.3):
 * all nodes are fitted by ONE fused pass over an integer-coded sample matrix instead of
   a Python loop of ``torch.unique`` sorts (:138-160).
 * ``evidence=None`` works (prior marginal); ``do`` performs graph surgery.
+* ``log_likelihood(data)`` scores rows: ``log P(observed values of the row)`` for any subset of the nodes, the others
+  summed out exactly (held-out log-likelihood, anomaly scores, probability of evidence); the reference has no such query.
 """
 from __future__ import annotations
 
@@ -204,6 +206,47 @@ class BayesianNetwork:
             dom = self.tables.domains[self.tables.index[tn]]
             out[tn] = (pdf, dom.unsqueeze(0).expand(pdf.shape[0], -1))
         return out
+
+    def log_likelihood(self, data) -> torch.Tensor:
+        """Natural log of the probability of each row's observed values under the fitted CPTs: float32 [n_rows] on the
+        device.
+
+        :param data: a DataFrame or a dict name -> values (tensor / array) holding domain VALUES, as ``infer`` takes them.
+                     The observed set is the set of columns passed, the same for every row; every other node is summed
+                     out exactly, so a subset of the nodes gives ``log P(e)``.  A column that is not a node raises
+                     ``ValueError`` (a typo must not silently marginalise a variable), as do columns of different lengths.
+        :return: ``log P(row)``; ``-inf`` for a value outside the fitted domain (NaN included) or for values of
+                 probability zero under the CPTs (a never-observed parent configuration among them); 0 for every row
+                 when no column is passed.  ``log P(e, T=t) - log P(e)`` equals ``log`` of ``infer``'s posterior
+                 ``P(t | e)``.  The value of a row depends on that row only (any batching gives identical bits).
+        """
+        cols, n_rows = self._observed_columns(data)
+        if not cols:
+            return torch.zeros(n_rows, dtype=torch.float32, device=self.device)
+        log_evidence = getattr(self.inference_obj, "log_evidence", None)
+        if log_evidence is None:
+            raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not compute log P(e)")
+        return log_evidence(cols)
+
+    def _observed_columns(self, data) -> Tuple[Dict[str, torch.Tensor], int]:
+        """``_columns`` for a subset of the nodes: (name -> float32 device column, number of rows)."""
+        dev = self.device
+        names = list(data.keys()) if isinstance(data, dict) else list(data.columns)
+        unknown = [n for n in names if n not in self.nodes_obj]
+        if unknown:
+            raise ValueError(f"columns {unknown} are not nodes of the network")
+        if isinstance(data, dict):
+            cols = {n: torch.as_tensor(data[n]).reshape(-1).to(dev, torch.float32) for n in names}
+            lengths = {int(c.numel()) for c in cols.values()}
+            if len(lengths) > 1:
+                raise ValueError("all columns must have the same number of rows")
+            return cols, (lengths.pop() if lengths else 0)
+        n_rows = len(data)
+        if not names:
+            return {}, n_rows
+        block = np.require(data[names].to_numpy(dtype=np.float32).T, requirements=["C", "W"])
+        dev_block = torch.from_numpy(block).to(dev)
+        return {n: dev_block[i] for i, n in enumerate(names)}, n_rows
 
     def sample(self, N: int, seed: int = 0, first_sample: int = 0) -> Dict[str, torch.Tensor]:
         """``N`` ancestral samples of the whole network from the fitted CPTs, as ``name -> float32 [N]`` device columns of

@@ -14,7 +14,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libcbn_b200.so")
-SOURCES = ["fit.cu", "count.cu", "ve.cu", "comm.cu"]
+SOURCES = ["fit.cu", "count.cu", "ve.cu", "comm.cu", "loglik.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-shared", "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",

@@ -341,9 +341,10 @@ struct cbn_ve_plan {
   // cbn_ve_plan_set_static_evidence: the evidence handed to runs of this plan is never written by the kernel that
   // precedes the run on the stream, so the gather kernels may read it before griddepcontrol.wait
   int static_evidence = 0;
-  // resident CTAs per SM of the kernel variant this plan launches ([0] direct, [1] tile-staged), queried once per plan
-  mutable int occ[2] = {0, 0};
-  mutable size_t occ_smem[2] = {0, 0};
+  // resident CTAs per SM of the kernel variant this plan launches ([0] direct, [1] tile-staged; [2], [3] the same for the
+  // log-evidence launch), queried once per plan
+  mutable int occ[4] = {0, 0, 0, 0};
+  mutable size_t occ_smem[4] = {0, 0, 0, 0};
 };
 
 namespace {
@@ -517,10 +518,43 @@ __device__ __forceinline__ void finish_map4(float (&p)[4][CT], uint32_t bad, int
   }
 }
 
+// Log-evidence epilogue (log-space plans): one float per row, the log of the row's unnormalised sum over the target,
+// max + log sum exp(x - max); -inf for a row with an unseen code or a zero sum
 template <int CT>
+__device__ __forceinline__ void finish_logev4(float (&p)[4][CT], uint32_t bad, int64_t quad, int64_t n_rows, float* __restrict__ out) {
+  pdl_wait();
+  const float NEG_INF = __int_as_float(0xff800000);
+  float v[4];
+#pragma unroll
+  for (int r = 0; r < 4; ++r) {
+    float m = p[r][0];
+#pragma unroll
+    for (int t = 1; t < CT; ++t) m = fmaxf(m, p[r][t]);
+    if (CT > 1 && m != NEG_INF) {
+      float z = 0.0f;
+#pragma unroll
+      for (int t = 0; t < CT; ++t) z += expf(p[r][t] - m);
+      m += logf(z);
+    }
+    v[r] = ((bad >> r) & 1u) ? NEG_INF : m;
+  }
+  const int64_t row0 = quad << 2;
+  if (row0 + 4 <= n_rows && (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
+    st_na_f128(reinterpret_cast<float4*>(out + row0), make_float4(v[0], v[1], v[2], v[3]));
+  } else {
+#pragma unroll
+    for (int r = 0; r < 4; ++r)
+      if (row0 + r < n_rows) out[row0 + r] = v[r];
+  }
+}
+
+// LOGEV: the log-evidence launch (cbn_ve_run_codes_log_evidence) -- a template parameter, so the posterior and MAP
+// launches compile exactly as without it
+template <int CT, bool LOGEV = false>
 __device__ __forceinline__ void finish_any4(float (&p)[4][CT], uint32_t bad, bool normalize, int64_t quad, int64_t n_rows,
                                             const GatherOuts& outs, int which, uint64_t st_pol) {
-  if (outs.map_domain) finish_map4<CT>(p, bad, quad, n_rows, outs.map_domain, outs.out[which]);
+  if constexpr (LOGEV) finish_logev4<CT>(p, bad, quad, n_rows, outs.out[which]);
+  else if (outs.map_domain) finish_map4<CT>(p, bad, quad, n_rows, outs.map_domain, outs.out[which]);
   else finish_rows4<CT>(p, bad, normalize, quad, n_rows, outs.out[which], st_pol, outs.log_space != 0);
 }
 
@@ -541,7 +575,7 @@ __device__ __noinline__ uint4 exact_index4(const GTable& T, const Loader& L, int
 
 // One quad (4 consecutive rows): for every fused target, gather one slice per table, multiply, normalise, store.
 // The four row indices are computed with SIMD-within-a-register arithmetic when the table is small enough.
-template <int CT, typename Loader>
+template <int CT, typename Loader, bool LOGEV = false>
 __device__ __forceinline__ void gather_rows4(const GTable* __restrict__ st, int n_tables, const float* __restrict__ pool,
                                              const Loader& L, int64_t quad, int64_t n_rows, const GatherOuts& outs,
                                              uint64_t st_pol = 0, uint64_t ld_pol = 0) {
@@ -554,7 +588,7 @@ __device__ __forceinline__ void gather_rows4(const GTable* __restrict__ st, int 
     const GTable& T = st[k];
     const int flags = T.flags;
     if (T.out_id != cur) {
-      if (cur >= 0) finish_any4<CT>(p, bad, (outs.normalize_mask >> cur) & 1u, quad, n_rows, outs, cur, st_pol);
+      if (cur >= 0) finish_any4<CT, LOGEV>(p, bad, (outs.normalize_mask >> cur) & 1u, quad, n_rows, outs, cur, st_pol);
       cur = T.out_id;
       bad = 0;
       n_mul = 0;
@@ -650,7 +684,7 @@ __device__ __forceinline__ void gather_rows4(const GTable* __restrict__ st, int 
       }
     }
   }
-  if (cur >= 0) finish_any4<CT>(p, bad, (outs.normalize_mask >> cur) & 1u, quad, n_rows, outs, cur, st_pol);
+  if (cur >= 0) finish_any4<CT, LOGEV>(p, bad, (outs.normalize_mask >> cur) & 1u, quad, n_rows, outs, cur, st_pol);
 }
 
 // one straight 128-bit copy of the plan blob (descriptors + staged tables) into shared memory
@@ -775,7 +809,7 @@ struct TileLoader {
   }
 };
 
-template <int CT, int NOUT, int GT_QPT>     // NOUT == 0: generic table list (gather_rows4); NOUT >= 2: one interleaved table
+template <int CT, int NOUT, int GT_QPT, bool LOGEV = false>     // NOUT == 0: generic table list (gather_rows4); NOUT >= 2: one interleaved table
 __global__ void __launch_bounds__(GATHER_TPB) gather_tiles_kernel(const unsigned char* __restrict__ blob, int blob_bytes,
                                                                   int desc_bytes, int n_tables, const __grid_constant__ TileCols cols,
                                                                   int n_stages, int hints, const uint8_t* __restrict__ ev, int64_t ld,
@@ -853,7 +887,7 @@ __global__ void __launch_bounds__(GATHER_TPB) gather_tiles_kernel(const unsigned
           const float* base = T.smem_off >= 0 ? pool + T.smem_off : T.data;
           gather_inter_rows4<CT, NOUT>(T, base, L, q, n_rows, outs, st_pol, ld_pol);
         } else {
-          gather_rows4<CT>(st, n_tables, pool, L, q, n_rows, outs, st_pol, ld_pol);
+          gather_rows4<CT, TileLoader<GT_TILE_ROWS>, LOGEV>(st, n_tables, pool, L, q, n_rows, outs, st_pol, ld_pol);
         }
       }
     }
@@ -864,8 +898,9 @@ __global__ void __launch_bounds__(GATHER_TPB) gather_tiles_kernel(const unsigned
 
 constexpr int gather_min_blocks(int ct) { return ct <= 2 ? 6 : (ct <= 4 ? 5 : 3); }
 
-template <int CT>
-__global__ void __launch_bounds__(GATHER_TPB, gather_min_blocks(CT)) gather_codes_kernel(
+// (the log-evidence variant of CT = 2 gets the register budget of CT = 3: at 40 registers it would spill)
+template <int CT, bool LOGEV = false>
+__global__ void __launch_bounds__(GATHER_TPB, gather_min_blocks(LOGEV && CT == 2 ? 3 : CT)) gather_codes_kernel(
     const unsigned char* __restrict__ blob, int blob_bytes, int desc_bytes, int n_tables, const uint8_t* __restrict__ ev,
     int64_t ld, int64_t n_rows, int early_ev, const __grid_constant__ GatherOuts outs) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -877,7 +912,7 @@ __global__ void __launch_bounds__(GATHER_TPB, gather_min_blocks(CT)) gather_code
   CodeLoader L{ev, ld};
   const int64_t nquads = (n_rows + 3) >> 2;
   for (int64_t q = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; q < nquads; q += int64_t(gridDim.x) * blockDim.x)
-    gather_rows4<CT>(st, n_tables, pool, L, q, n_rows, outs);
+    gather_rows4<CT, CodeLoader, LOGEV>(st, n_tables, pool, L, q, n_rows, outs);
 }
 
 template <int CT>
@@ -1153,22 +1188,23 @@ int gather_blocks(cbn_ctx* ctx, int64_t n_rows, int per_sm) {
   const int64_t nquads = (n_rows + 3) >> 2;
   return (int)balanced_grid((nquads + GATHER_TPB - 1) / GATHER_TPB, int64_t(ctx->sm_count) * per_sm);
 }
-template <int CT>
+template <int CT, bool LOGEV = false>
 int launch_codes(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, const GatherOuts& outs,
                  cudaStream_t s) {
   static bool attr_set[64] = {};
   if (!attr_set[ctx->device & 63]) {
-    CBN_CUDA(ctx, cudaFuncSetAttribute(gather_codes_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+    CBN_CUDA(ctx, cudaFuncSetAttribute(gather_codes_kernel<CT, LOGEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
     attr_set[ctx->device & 63] = true;
   }
   // one wave: as many CTAs as fit (register / shared-memory bound), the rest of the rows by the grid-stride loop
-  if (p->occ[0] == 0 || p->occ_smem[0] != p->blob_bytes) {   // resident CTAs per SM for this plan (queried once)
+  const int slot = LOGEV ? 2 : 0;
+  if (p->occ[slot] == 0 || p->occ_smem[slot] != p->blob_bytes) {   // resident CTAs per SM for this plan (queried once)
     int occ = 1;
-    CBN_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gather_codes_kernel<CT>, GATHER_TPB, p->blob_bytes));
-    p->occ[0] = std::max(occ, 1); p->occ_smem[0] = p->blob_bytes;
+    CBN_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gather_codes_kernel<CT, LOGEV>, GATHER_TPB, p->blob_bytes));
+    p->occ[slot] = std::max(occ, 1); p->occ_smem[slot] = p->blob_bytes;
   }
-  const int per_sm = p->occ[0];
-  CBN_CUDA(ctx, launch_pdl(gather_codes_kernel<CT>, gather_blocks(ctx, n_rows, per_sm), GATHER_TPB, p->blob_bytes, s,
+  const int per_sm = p->occ[slot];
+  CBN_CUDA(ctx, launch_pdl(gather_codes_kernel<CT, LOGEV>, gather_blocks(ctx, n_rows, per_sm), GATHER_TPB, p->blob_bytes, s,
                            p->d_blob, (int)p->blob_bytes, (int)p->desc_bytes, p->n_tables, ev, ld, n_rows, p->static_evidence, outs));
   return CBN_OK;
 }
@@ -1208,7 +1244,7 @@ int launch_inter(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t 
 }
 
 // tile-staged launch: persistent CTAs, as many as fit per SM for this plan's shared-memory footprint
-template <int CT, int NOUT, int QPT>
+template <int CT, int NOUT, int QPT, bool LOGEV = false>
 int launch_tiles_q(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, const GatherOuts& outs,
                    cudaStream_t s) {
   TileCols cols{};
@@ -1233,18 +1269,19 @@ int launch_tiles_q(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_
   const size_t smem = blob_pad + n_stages * stage_bytes;
   static bool attr_set[64] = {};
   if (!attr_set[ctx->device & 63]) {
-    CBN_CUDA(ctx, cudaFuncSetAttribute(gather_tiles_kernel<CT, NOUT, QPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+    CBN_CUDA(ctx, cudaFuncSetAttribute(gather_tiles_kernel<CT, NOUT, QPT, LOGEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
     attr_set[ctx->device & 63] = true;
   }
-  if (p->occ[1] == 0 || p->occ_smem[1] != smem) {
+  const int slot = LOGEV ? 3 : 1;
+  if (p->occ[slot] == 0 || p->occ_smem[slot] != smem) {
     int occ = 1;
-    CBN_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gather_tiles_kernel<CT, NOUT, QPT>, GATHER_TPB, smem));
-    p->occ[1] = std::max(occ, 1); p->occ_smem[1] = smem;
+    CBN_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gather_tiles_kernel<CT, NOUT, QPT, LOGEV>, GATHER_TPB, smem));
+    p->occ[slot] = std::max(occ, 1); p->occ_smem[slot] = smem;
   }
   const int64_t n_tiles = (n_rows + GT_TILE_ROWS - 1) / GT_TILE_ROWS;
-  const int per_sm = p->occ[1];
+  const int per_sm = p->occ[slot];
   const int blocks = (int)balanced_grid(n_tiles, int64_t(ctx->sm_count) * per_sm);
-  CBN_CUDA(ctx, launch_pdl(gather_tiles_kernel<CT, NOUT, QPT>, blocks, GATHER_TPB, smem, s, p->d_blob, (int)p->blob_bytes,
+  CBN_CUDA(ctx, launch_pdl(gather_tiles_kernel<CT, NOUT, QPT, LOGEV>, blocks, GATHER_TPB, smem, s, p->d_blob, (int)p->blob_bytes,
                            (int)p->desc_bytes, p->n_tables, cols, n_stages, hints, ev, ld, n_rows, p->static_evidence, outs));
   return CBN_OK;
 }
@@ -1556,7 +1593,9 @@ __host__ __device__ inline int rows_code_words(int n_evidence) { return (((n_evi
 __host__ __device__ inline int rows_base_words(int n_inputs) { return (n_inputs + 3) & ~3; }
 __host__ __device__ inline int rows_scale_words(int n_steps) { return (n_steps + 3) & ~3; }
 
-template <bool LOG>
+// LE: log-evidence mode (log space only) -- instead of the posterior row, out[row] = log of the row's unnormalised sum:
+// LSE_t(last) plus the maxima that the consuming steps took out of every earlier temporary (-sum of their scales)
+template <bool LOG, bool LE = false>
 __global__ void __launch_bounds__(ROWS_TPB, 4) ve_rows_kernel(const RowInputDev* __restrict__ inputs, int n_inputs,
                                                            const RowStepDev* __restrict__ steps, int n_steps, int temp_floats,
                                                            const int* __restrict__ off_pool, int off_ints, int n_evidence,
@@ -1628,8 +1667,25 @@ __global__ void __launch_bounds__(ROWS_TPB, 4) ve_rows_kernel(const RowInputDev*
         __syncwarp();          // this step's stores and its scale become visible to the other lanes
       }
     }
-    // normalise the last temporary over the target and write the posterior row
     const float* last = temps + sst[n_steps - 1].temp_off;
+    if constexpr (LE) {
+      float mx = NEG_INF, z = 0.0f;
+      if (!bad) {
+        for (int t = lane; t < card_t; t += 32) mx = fmaxf(mx, last[t]);
+        mx = warp_max(mx);
+        if (mx != NEG_INF) {
+          for (int t = lane; t < card_t; t += 32) z += expf(last[t] - mx);
+          z = warp_sum(z);
+          float taken = 0.0f;
+          for (int j = 0; j + 1 < n_steps; ++j) taken -= tscale[j];
+          mx += logf(z) + taken;
+        }
+      }
+      if (lane == 0) out[row] = mx;
+      __syncwarp();
+      continue;
+    }
+    // normalise the last temporary over the target and write the posterior row
     float z = 0.0f, mx = NEG_INF;
     if (LOG && !bad) {
       for (int t = lane; t < card_t; t += 32) mx = fmaxf(mx, last[t]);
@@ -1800,7 +1856,8 @@ __device__ __noinline__ float rowt_step_any(const RowStepDev& S, const int* __re
   return mx;
 }
 
-template <bool LOG>
+// LE: log-evidence mode, as in ve_rows_kernel; the maxima subtracted in place are summed in one register
+template <bool LOG, bool LE = false>
 __global__ void __launch_bounds__(ROWT_TPB) ve_rows_thread_kernel(const RowInputDev* __restrict__ inputs, int n_inputs,
                                                                   const RowStepDev* __restrict__ steps, int n_steps, int temp_floats,
                                                                   const int* __restrict__ off_pool, int off_ints,
@@ -1822,6 +1879,7 @@ __global__ void __launch_bounds__(ROWT_TPB) ve_rows_thread_kernel(const RowInput
   for (int64_t row0 = int64_t(blockIdx.x) * ROWT_TPB; row0 < n_rows; row0 += int64_t(gridDim.x) * ROWT_TPB) {
     const int64_t row = min(row0 + tid, n_rows - 1);       // threads past the end repeat the last row and do not store
     bool bad = false;
+    float taken = 0.0f;                                      // LE: sum of the maxima subtracted from the temporaries
     for (int j = 0; j < n_steps; ++j) {
       const RowStepDev& S = sst[j];
       const int* offs = soff + S.off_at;
@@ -1836,14 +1894,25 @@ __global__ void __launch_bounds__(ROWT_TPB) ve_rows_thread_kernel(const RowInput
       if (j + 1 < n_steps) {       // keep the temporary in range (a per-row constant cancels in the final normalisation)
         if (LOG) {
           if (mx != NEG_INF) for (int o = 0; o < S.out_size; ++o) tsm[(S.temp_off + o) * ROWT_TPB + tid] -= mx;
+          if (LE && mx != NEG_INF) taken += mx;
         } else if (mx > 0.0f) {
           const float inv = 1.0f / mx;
           for (int o = 0; o < S.out_size; ++o) tsm[(S.temp_off + o) * ROWT_TPB + tid] *= inv;
         }
       }
     }
-    // normalise the last temporary over the target and write the posterior row
     const int last = sst[n_steps - 1].temp_off;
+    if constexpr (LE) {
+      float mxl = NEG_INF, z = 0.0f;
+      for (int t = 0; t < card_t; ++t) mxl = fmaxf(mxl, tsm[(last + t) * ROWT_TPB + tid]);
+      if (mxl != NEG_INF) {
+        for (int t = 0; t < card_t; ++t) z += expf(tsm[(last + t) * ROWT_TPB + tid] - mxl);
+        mxl += logf(z) + taken;
+      }
+      if (row0 + tid < n_rows) out[row] = bad ? NEG_INF : mxl;
+      continue;
+    }
+    // normalise the last temporary over the target and write the posterior row
     float z = 0.0f, mxl = NEG_INF;
     if (LOG) for (int t = 0; t < card_t; ++t) mxl = fmaxf(mxl, tsm[(last + t) * ROWT_TPB + tid]);
     for (int t = 0; t < card_t; ++t) {
@@ -1979,42 +2048,39 @@ extern "C" int cbn_ve_plan_create_rows(cbn_ctx* ctx, int32_t n_evidence, const i
   if (e == cudaSuccess) e = cudaFuncSetAttribute(ve_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(ve_rows_thread_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(ve_rows_thread_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(ve_rows_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(ve_rows_thread_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
   if (e != cudaSuccess) { cbn_ve_plan_destroy(p); return cbn_fail(ctx, CBN_ERR_CUDA, "per-row plan upload: %s", cudaGetErrorString(e)); }
   *out = p;
   return CBN_OK;
 }
 
-static int ve_run_rows(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, float* out, cudaStream_t s) {
+template <bool LOG, bool LE>
+static int ve_run_rows_t(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, float* out, cudaStream_t s) {
   static int thread_mode = -1;
   if (thread_mode < 0) { const char* e = getenv("CBN_ROWS_THREAD"); thread_mode = e ? atoi(e) : 1; }
   if (p->rows_per_thread && thread_mode) {
     const int per = (int)std::max<size_t>(1, std::min<size_t>(8, (200 * 1024) / (p->rows_thread_smem + 1024)));
     const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((n_rows + ROWT_TPB - 1) / ROWT_TPB, int64_t(ctx->sm_count) * per));
-    if (p->rows_flags & CBN_ROWS_LOG_SPACE)
-      ve_rows_thread_kernel<true><<<blocks, ROWT_TPB, p->rows_thread_smem, s>>>(
-          (const RowInputDev*)p->d_row_inputs, p->rows_n_inputs, (const RowStepDev*)p->d_row_steps, p->rows_n_steps, p->rows_temp_floats,
-          (const int*)p->d_row_offsets, p->rows_off_ints, ev, ld, n_rows, p->card_t, out);
-    else
-      ve_rows_thread_kernel<false><<<blocks, ROWT_TPB, p->rows_thread_smem, s>>>(
-          (const RowInputDev*)p->d_row_inputs, p->rows_n_inputs, (const RowStepDev*)p->d_row_steps, p->rows_n_steps, p->rows_temp_floats,
-          (const int*)p->d_row_offsets, p->rows_off_ints, ev, ld, n_rows, p->card_t, out);
+    ve_rows_thread_kernel<LOG, LE><<<blocks, ROWT_TPB, p->rows_thread_smem, s>>>(
+        (const RowInputDev*)p->d_row_inputs, p->rows_n_inputs, (const RowStepDev*)p->d_row_steps, p->rows_n_steps, p->rows_temp_floats,
+        (const int*)p->d_row_offsets, p->rows_off_ints, ev, ld, n_rows, p->card_t, out);
     CBN_CHECK_LAUNCH(ctx);
     return CBN_OK;
   }
   const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(4, (200 * 1024) / (p->blob_bytes + 1024)));
   const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((n_rows + ROWS_WARPS - 1) / ROWS_WARPS, int64_t(ctx->sm_count) * per_sm));
-  if (p->rows_flags & CBN_ROWS_LOG_SPACE)
-    ve_rows_kernel<true><<<blocks, ROWS_TPB, p->blob_bytes, s>>>((const RowInputDev*)p->d_row_inputs, p->rows_n_inputs,
-                                                                (const RowStepDev*)p->d_row_steps, p->rows_n_steps, p->rows_temp_floats,
-                                                                (const int*)p->d_row_offsets, p->rows_off_ints, p->n_evidence,
-                                                                ev, ld, n_rows, p->card_t, out);
-  else
-    ve_rows_kernel<false><<<blocks, ROWS_TPB, p->blob_bytes, s>>>((const RowInputDev*)p->d_row_inputs, p->rows_n_inputs,
+  ve_rows_kernel<LOG, LE><<<blocks, ROWS_TPB, p->blob_bytes, s>>>((const RowInputDev*)p->d_row_inputs, p->rows_n_inputs,
                                                                  (const RowStepDev*)p->d_row_steps, p->rows_n_steps, p->rows_temp_floats,
                                                                  (const int*)p->d_row_offsets, p->rows_off_ints, p->n_evidence,
                                                                  ev, ld, n_rows, p->card_t, out);
   CBN_CHECK_LAUNCH(ctx);
   return CBN_OK;
+}
+
+static int ve_run_rows(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, float* out, cudaStream_t s) {
+  if (p->rows_flags & CBN_ROWS_LOG_SPACE) return ve_run_rows_t<true, false>(ctx, p, ev, ld, n_rows, out, s);
+  return ve_run_rows_t<false, false>(ctx, p, ev, ld, n_rows, out, s);
 }
 
 extern "C" int cbn_ve_run_codes(cbn_ctx* ctx, const cbn_ve_plan* plan, const uint8_t* ev_codes, int64_t ld,
@@ -2041,6 +2107,49 @@ extern "C" int cbn_ve_run_codes_multi(cbn_ctx* ctx, const cbn_ve_plan* plan, con
   if (n_rows == 0) return CBN_OK;
   DeviceGuard g(ctx->device);
   return ve_run_codes_impl(ctx, plan, ev_codes, ld, n_rows, outs, (cudaStream_t)stream);
+}
+
+// ---- log of the evidence probability per row (log-space plans; see the header) ---------------------------------------
+extern "C" int cbn_ve_run_codes_log_evidence(cbn_ctx* ctx, const cbn_ve_plan* plan, const uint8_t* ev_codes, int64_t ld,
+                                             int64_t n_rows, float* log_out, cbn_stream stream) {
+  const char* fn = "cbn_ve_run_codes_log_evidence";
+  if (!ctx) return cbn_fail(nullptr, CBN_ERR_INVALID, "%s: ctx is NULL", fn);
+  if (!plan || n_rows < 0) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: bad argument", fn);
+  const bool log_plan = plan->kind == 1 ? (plan->rows_flags & CBN_ROWS_LOG_SPACE) != 0 : plan->log_space != 0;
+  if (!log_plan) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: the plan's tables are not logarithms (compile it in log space)", fn);
+  if (plan->kind == 0 && (plan->n_out != 1 || plan->interleaved || plan->card_t > GATHER_MAX_CT))
+    return cbn_fail(ctx, CBN_ERR_UNSUPPORTED, "%s: needs a single-target plan with at most %d target values", fn, GATHER_MAX_CT);
+  if (n_rows == 0) return CBN_OK;
+  if (!log_out) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: log_out is NULL", fn);
+  if (plan->n_evidence > 0 && (!ev_codes || ld < n_rows || (ld % 16) != 0 || !is_aligned(ev_codes, 16)))
+    return cbn_fail(ctx, CBN_ERR_INVALID, "%s: evidence matrix needs ld >= n_rows, ld %% 16 == 0, 16-byte aligned base", fn);
+  DeviceGuard g(ctx->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (plan->kind == 1) return ve_run_rows_t<true, true>(ctx, plan, ev_codes, ld, n_rows, log_out, s);
+  GatherOuts outs{};
+  outs.out[0] = log_out;
+  outs.normalize_mask = 0;
+  outs.log_space = 1;
+  if (use_tiles(plan, n_rows)) switch (plan->card_t) {
+    case 1: return launch_tiles_q<1, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 2: return launch_tiles_q<2, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 3: return launch_tiles_q<3, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 4: return launch_tiles_q<4, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 5: return launch_tiles_q<5, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 6: return launch_tiles_q<6, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 7: return launch_tiles_q<7, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    default: return launch_tiles_q<8, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+  }
+  switch (plan->card_t) {
+    case 1: return launch_codes<1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 2: return launch_codes<2, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 3: return launch_codes<3, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 4: return launch_codes<4, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 5: return launch_codes<5, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 6: return launch_codes<6, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    case 7: return launch_codes<7, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+    default: return launch_codes<8, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+  }
 }
 
 extern "C" int cbn_ve_run_f32(cbn_ctx* ctx, const cbn_ve_plan* plan, const float* const* ev_cols,

@@ -7,7 +7,7 @@ import torch
 
 from .. import _native as N
 from ..base.inference import BaseInference
-from ..ve import FusedPlan, QueryPlan, RowPlan, VECompiler
+from ..ve import EvidencePlan, FusedPlan, QueryPlan, RowPlan, VECompiler
 
 
 class ExactInference(BaseInference):
@@ -80,6 +80,32 @@ class ExactInference(BaseInference):
                 else:
                     out[chunk[0]] = plans[i].run_codes(codes, nq)
         return out
+
+    def evidence_plan(self, evidence_names: Sequence[str]) -> EvidencePlan:
+        assert self.compiler is not None, "inference engine is not bound to a fitted network"
+        return self.compiler.compile_evidence(list(evidence_names))
+
+    def log_evidence(self, evidence: Dict[str, torch.Tensor]) -> torch.Tensor:
+        """``log P(e)`` per row: float32 [n_rows] on the device (natural log).  ``evidence``: name -> tensor [n_rows] or
+        [n_rows, 1] of category VALUES, the same observed set for every row; every other node is summed out exactly.
+        -inf for a value outside the fitted domain (NaN included) or evidence of probability zero; an empty dict gives an
+        empty result.  Not part of the reference's surface."""
+        t = self.tables
+        evidence = evidence or {}
+        names = list(evidence.keys())
+        for n in names:
+            if n not in t.index:
+                raise ValueError(f"{n} is not a node of the network")
+        cols = [torch.as_tensor(evidence[n]).reshape(-1) for n in names]
+        nq = int(cols[0].numel()) if cols else 0
+        if any(int(c.numel()) != nq for c in cols):
+            raise ValueError("all evidence columns must have the same number of rows")
+        plan = self.evidence_plan(names)
+        ld = (max(nq, 1) + 15) // 16 * 16
+        codes = torch.empty((max(len(names), 1), ld), dtype=torch.uint8, device=t.device)
+        for e, (n, c) in enumerate(zip(names, cols)):
+            t.encode(c.to(t.device, torch.float32, non_blocking=True), t.index[n], codes[e])
+        return plan.run_codes(codes, nq)
 
     def infer_map(self, target_node: str, evidence: Dict[str, torch.Tensor]) -> Optional[torch.Tensor]:
         """MAP value of the target per row through the fused kernel (``cbn_ve_run_f32_map``); ``None`` when the plan is

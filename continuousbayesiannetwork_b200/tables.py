@@ -46,6 +46,8 @@ class DiscreteTables:
         self.counts: Optional[torch.Tensor] = None   # int64 [total_cells]
         self.joint: Optional[torch.Tensor] = None    # float32 [total_cells]
         self.cond: Optional[torch.Tensor] = None     # float32 [total_cells]
+        self._log_cond: Optional[torch.Tensor] = None
+        self.cond_version = 0                        # bumped whenever cond changes: plans derived from it are stale
         self._count_plan = None
         self._dom_matrix = None
         self._layout_cards: Optional[List[int]] = None
@@ -75,6 +77,7 @@ class DiscreteTables:
             self.reset_counts()
             self.joint = None
             self.cond = None
+            self._drop_log_cond()
             return
         self._destroy_plan()
         self._layout_cards = list(self.cards)
@@ -102,8 +105,24 @@ class DiscreteTables:
         self._n_dev = self._counts_buf[off:off + 1]
         self.joint = None
         self.cond = None
+        self._drop_log_cond()
         self._n_host, self._n_host_valid = 0, True
         self._reduced = False
+
+    def _drop_log_cond(self):
+        self._log_cond = None
+        self.cond_version += 1
+
+    @property
+    def log_cond(self) -> torch.Tensor:
+        """``log(cond)`` (natural log, -inf for zero entries), same layout as ``cond``; computed on first use and dropped
+        whenever the conditional tables change (``finalize``, ``set_cond_tables``), together with the log-evidence plans
+        built from it."""
+        if self.cond is None:
+            raise ValueError("the network is not fitted")
+        if self._log_cond is None:
+            self._log_cond = torch.log(self.cond)
+        return self._log_cond
 
     def reset_counts(self):
         """Empty tables (and sample count) for a fresh fit; the layout and the count plan are kept."""
@@ -291,6 +310,7 @@ class DiscreteTables:
             self.joint = torch.zeros(self.total_cells, dtype=torch.float32, device=self.device)
             self.cond = torch.zeros(self.total_cells, dtype=torch.float32, device=self.device)
         self._ensure_plan()
+        self._drop_log_cond()
         N.check(N.lib().cbn_cpt_from_plan_dev(self.ctx.handle, self._count_plan, self.counts.data_ptr(), self._n_dev.data_ptr(),
                                               self.joint.data_ptr(), self.cond.data_ptr(), N.stream_ptr(self.device)),
                 self.ctx.handle)
@@ -298,6 +318,7 @@ class DiscreteTables:
     def set_cond_tables(self, cpts: Sequence):
         """Install ground-truth conditional tables (synthetic workloads; no counting)."""
         self.cond = torch.zeros(self.total_cells, dtype=torch.float32, device=self.device)
+        self._drop_log_cond()
         for i, t in enumerate(cpts):
             t = torch.as_tensor(t, dtype=torch.float32).reshape(-1)
             assert t.numel() == self.n_cells[i]

@@ -333,6 +333,95 @@ class RowPlan:
         return self.run_codes(codes, n_rows, out)
 
 
+@dataclass
+class EvidenceSplit:
+    """How ``VECompiler.compile_evidence`` splits ``log P(e)``: the families summed by the observed-families kernel
+    (network ids of the CPT owners) and the statistics of the VE plan for the rest (None: there is no rest)."""
+    evidence: List[int]
+    observed_families: List[int]
+    ve_stats: Optional[PlanStats]
+    per_row: bool = False
+
+
+class LogLikPlan:
+    """Owner of a ``cbn_loglik_plan``: ``out[row] (+)= sum_f log cond_f[index_f(row)]`` over families whose variables are
+    all columns of the code matrix handed to ``run`` (``columns[v]``: the column of network variable v)."""
+
+    def __init__(self, tables_owner, families: Sequence[int], columns: Dict[int, int], n_cols: int):
+        self.ctx = tables_owner.ctx
+        self.device = tables_owner.device
+        self.handle = None
+        t = tables_owner
+        fams = (N.Family * max(len(families), 1))()
+        for i, v in enumerate(families):
+            vs = t.family_vars(t.names[v])
+            fams[i] = N.make_family([columns[u] for u in vs], [t.cards[u] for u in vs], t.offsets[v])
+        h = C.c_void_p()
+        # the plan derives its own (merged) tables from the log tables and does not keep a reference to them
+        N.check(N.lib().cbn_loglik_plan_create(self.ctx.handle, fams, len(families), int(n_cols), t.log_cond.data_ptr(),
+                                               N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
+        self.handle = h
+        self.lookups_per_row = N.lib().cbn_loglik_plan_tables(h)
+
+    def __del__(self):
+        try:
+            if self.handle is not None:
+                N.lib().cbn_loglik_plan_destroy(self.handle)
+                self.handle = None
+        except Exception:
+            pass
+
+    def run(self, codes: torch.Tensor, n_rows: int, out: torch.Tensor, accumulate: bool = False) -> torch.Tensor:
+        assert codes.dtype == torch.uint8 and codes.is_cuda and out.dtype == torch.float32
+        N.check(N.lib().cbn_loglik_run(self.ctx.handle, self.handle, codes.data_ptr(), codes.stride(0), int(n_rows),
+                                       out.data_ptr(), 1 if accumulate else 0, N.stream_ptr(self.device)), self.ctx.handle)
+        return out
+
+
+class EvidencePlan:
+    """A compiled ``log P(e)`` query (``VECompiler.compile_evidence``): the observed-families kernel over the CPTs that
+    lie inside the evidence set, plus at most one VE plan (gather or per-row) for the rest."""
+
+    def __init__(self, tables_owner, evidence: List[int], observed_families: List[int], ve_plan, split: EvidenceSplit):
+        self.owner = tables_owner
+        self.ctx = tables_owner.ctx
+        self.device = tables_owner.device
+        self.evidence = list(evidence)
+        self.observed_families = list(observed_families)
+        self.ve_plan = ve_plan
+        self.split = split
+        slot = {v: i for i, v in enumerate(self.evidence)}
+        self.loglik = LogLikPlan(tables_owner, self.observed_families, slot, len(self.evidence)) if self.observed_families else None
+
+    def algorithmic_bytes_per_row(self) -> int:
+        return len(self.evidence) + 4
+
+    def set_static_evidence(self, on: bool = True):
+        if self.ve_plan is not None:
+            self.ve_plan.set_static_evidence(on)
+
+    def run_codes(self, ev_codes: torch.Tensor, n_rows: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """ev_codes: uint8 [len(evidence), ld] on the device (row e = evidence variable e of the plan).  Returns float32
+        [n_rows]: log P(e_row), -inf for an unseen value or evidence of probability zero."""
+        assert ev_codes.dtype == torch.uint8 and ev_codes.is_cuda
+        if out is None:
+            out = torch.empty(n_rows, dtype=torch.float32, device=self.device)
+        if n_rows == 0:
+            return out
+        accumulate = False
+        if self.ve_plan is not None:
+            ld = ev_codes.stride(0) if ev_codes.dim() == 2 else 0
+            N.check(N.lib().cbn_ve_run_codes_log_evidence(self.ctx.handle, self.ve_plan.handle, ev_codes.data_ptr(), ld,
+                                                          int(n_rows), out.data_ptr(), N.stream_ptr(self.device)),
+                    self.ctx.handle)
+            accumulate = True
+        if self.loglik is not None:
+            self.loglik.run(ev_codes, n_rows, out, accumulate=accumulate)
+        elif self.ve_plan is None:          # no evidence: log 1
+            out.zero_()
+        return out
+
+
 class _Greedy:
     """Greedy min-size elimination with incremental bookkeeping: the scope a variable's elimination would create is
     cached and only recomputed for the variables that share a factor with the one just eliminated (the full rescan is
@@ -420,6 +509,9 @@ class VECompiler:
         self._cache: Dict[tuple, QueryPlan] = {}
         self._has_zero: Dict[int, bool] = {}
         self.last_row_schedule: Optional[dict] = None
+        self._ev_child: Optional["VECompiler"] = None       # the evidence-mode compiler (log space, no range control)
+        self._ev_cache: Dict[tuple, "EvidencePlan"] = {}
+        self._ev_cache_version = None
 
     # ---------------------------------------------------------------- graph helpers
     def _parents(self, v: int) -> List[int]:
@@ -627,6 +719,96 @@ class VECompiler:
         self._cache[key] = plan
         return plan
 
+    # ---------------------------------------------------------------- evidence mode: log P(e)
+    def compile_evidence(self, evidence_names: Sequence[str], dry: bool = False):
+        """Compile ``log P(e)`` for the evidence set ``evidence_names`` (one value per row of every variable).
+
+        Only ``ancestors(E)`` matter: barren descendants sum to 1.  A CPT whose scope lies inside ``E`` is a constant of
+        the sum and goes to the observed-families kernel (``cbn_loglik_run``) with its variables remapped to evidence
+        slots.  Every other CPT belongs to a component of hidden variables, and ALL components are eliminated completely
+        (none is dropped as in the posterior compile): what is left are tables over evidence subsets only (card_t = 1),
+        gathered by ``cbn_ve_run_codes_log_evidence``.  When the elimination exceeds the table budget the remaining
+        hidden variables go to the per-row executor, as for posteriors.
+
+        The elimination runs in log space WITHOUT range control: log-sum-exp contractions have no range problem in fp32,
+        and dropping the per-slice rescaling is what keeps the normaliser.  The network's posterior plans keep their own
+        configuration and cache; evidence plans are cached separately, keyed by the evidence tuple, and dropped when the
+        tables are re-fitted.
+
+        ``dry=True`` works on ``DryTables`` and returns the ``EvidenceSplit`` only (no device work)."""
+        if not self.log_space or self.rescale:
+            if self._ev_child is None:
+                self._ev_child = VECompiler(self.t, table_budget_cells=self.table_budget, merge_budget_cells=self.merge_budget,
+                                            check_support=False, row_temp_floats=self.row_temp_floats, log_space=True,
+                                            rescale=False, profile_compile=self.profile_compile,
+                                            row_unit_layout=self.row_unit_layout)
+            return self._ev_child.compile_evidence(evidence_names, dry=dry)
+        t = self.t
+        cards = t.cards
+        for e in evidence_names:
+            if e not in t.index:
+                raise ValueError(f"{e} is not a node of the network")
+        E = [t.index[e] for e in evidence_names]
+        if len(set(E)) != len(E):
+            raise ValueError("an evidence variable is listed twice")
+        key = tuple(E)
+        if not dry:
+            version = getattr(t, "cond_version", 0)
+            if self._ev_cache_version != version:          # re-fitted tables: every cached plan is stale
+                self._ev_cache = {}
+                self._ev_cache_version = version
+            if key in self._ev_cache:
+                return self._ev_cache[key]
+            # structure-only pass first: a query that does not fit fails here, before any table is contracted
+            self.compile_evidence(evidence_names, dry=True)
+            self._events = []
+        Eset = set(E)
+        self._ev_set = Eset
+        order_key = {v: i for i, v in enumerate(E)}
+
+        def sort_scope(scope) -> List[int]:
+            # evidence axes (plan order) first, then hidden
+            return sorted(set(scope), key=lambda v: (0 if v in Eset else 1, order_key.get(v, v)))
+
+        stats = PlanStats()
+        relevant = self._ancestors(E)
+        stats.n_relevant = len(relevant)
+        observed: List[int] = []
+        factors: List[Factor] = []
+        for v in sorted(relevant):
+            scope = t.family_vars(t.names[v])
+            if all(u in Eset for u in scope):
+                observed.append(v)
+                continue
+            tensor = None if dry else t.table_view(t.log_cond, t.names[v]).reshape(-1)
+            factors.append(Factor(list(scope), tensor))
+        hidden = [v for v in sorted(relevant) if v not in Eset]
+        stats.n_hidden = len(hidden)
+        stats.relevant_evidence = list(E)
+        ve_plan, per_row = None, False
+        if factors:
+            finals, left = self._eliminate(factors, hidden, sort_scope, stats, dry, None, partial=True)
+            if left:
+                per_row = True
+                stats.per_row_hidden = len(left)
+                stats.final_tables = [(tuple(f.scope), f.size(cards)) for f in finals]
+                stats.per_row_slice_cells = sum(int(f.size(cards) // max(1, _prod(cards[v] for v in f.scope if v in Eset)))
+                                                for f in finals)
+                ve_plan = self._row_plan(None, E, finals, left, stats, dry)
+            else:
+                finals = self._merge_finals(finals, sort_scope, stats, dry, None)
+                stats.final_tables = [(tuple(f.scope), f.size(cards)) for f in finals]
+                if not dry:
+                    ve_plan = QueryPlan(t, None, E, 1, finals, True, stats, log_space=True)
+        split = EvidenceSplit(evidence=list(E), observed_families=observed, ve_stats=stats if factors else None,
+                              per_row=per_row)
+        if dry:
+            return split
+        stats.contraction_gpu_ms = self._drain_events()
+        plan = EvidencePlan(t, E, observed, ve_plan, split)
+        self._ev_cache[key] = plan
+        return plan
+
     def _drain_events(self) -> float:
         if not self._events:
             return 0.0
@@ -737,12 +919,13 @@ class VECompiler:
             next_key += 1
             stats.n_steps += 1
         rest = list(live.keys())
-        # final product over what is left (free scope is empty or [T])
+        # final product over what is left (free scope is empty or [T]; evidence mode has no target)
+        last_scope = [T] if T is not None else []
         while len(rest) > MAXIN:
-            ops.append((rest[:MAXIN], next_key, [T], None))
+            ops.append((rest[:MAXIN], next_key, last_scope, None))
             rest = rest[MAXIN:] + [next_key]
             next_key += 1
-        ops.append((rest, next_key, [T], None))
+        ops.append((rest, next_key, last_scope, None))
 
         # pass 2: layouts, offset tables, temporaries
         inner = {}                                             # factor key -> the variable its consumer sums over
@@ -816,7 +999,7 @@ class VECompiler:
                                   "steps": steps, "offsets": offsets}
         if dry:
             return None
-        return RowPlan(self.t, T, E, cards[T], laid, steps, offsets, stats, self.log_space)
+        return RowPlan(self.t, T, E, cards[T] if T is not None else 1, laid, steps, offsets, stats, self.log_space)
 
     def _merge_finals(self, finals: List[Factor], sort_scope, stats: PlanStats, dry: bool, T: int) -> List[Factor]:
         """Multiply final tables together while the product stays within the merge budget: fewer gathers

@@ -300,6 +300,15 @@ CBN_API int cbn_ve_run_codes_map(cbn_ctx* ctx, const cbn_ve_plan* plan, const ui
                          const float* target_domain, float* map_out, cbn_stream stream);
 CBN_API int cbn_ve_run_f32_map(cbn_ctx* ctx, const cbn_ve_plan* plan, const float* const* ev_cols, const float* const* domains,
                        int64_t n_rows, const float* target_domain, float* map_out, cbn_stream stream);
+/* Log of the row's unnormalised sum: log_out[row] = log sum_t prod_k table_k[...]  (log-space plans: max + log sum exp(x - max)),
+ * plus, for per-row plans, the scales the schedule took out of its temporaries.  With a plan compiled by the evidence mode
+ * (the hidden variables of the evidence's ancestors eliminated in log space without range control, card_t = 1) this is
+ * log P(e_row).  -inf for unseen codes and zero sums.  Gather plans: single-target, card_t <= 8, tables in log space
+ * (CBN_GATHER_LOG_SPACE); per-row plans: CBN_ROWS_LOG_SPACE.  Other plans: CBN_ERR_INVALID.  log_out: device float
+ * [n_rows].  Nothing in the reference computes this (its inference slot is empty): new surface, like cbn_sample_forward. */
+CBN_API int cbn_ve_run_codes_log_evidence(cbn_ctx* ctx, const cbn_ve_plan* plan, const uint8_t* ev_codes, int64_t ld,
+                                          int64_t n_rows, float* log_out, cbn_stream stream);
+
 /* same as cbn_ve_run_codes but with HOST buffers (pinned or pageable): chunks are
  * copied in, processed and copied out on internal streams, double-buffered.
  * Synchronous: returns when `posterior_host` is complete. */
@@ -322,6 +331,32 @@ CBN_API int cbn_ve_run_codes_host_multi_ex(cbn_ctx* ctx, const cbn_ve_plan* plan
  * (bayesian_network.py:296).  max_out: device float (caller zero-initialises). */
 CBN_API int cbn_batch_max(cbn_ctx* ctx, const float* x, int64_t n, float* max_out, cbn_stream stream);
 CBN_API int cbn_scale_by_inv(cbn_ctx* ctx, float* x, int64_t n, const float* denom, cbn_stream stream);
+
+/* ---- log-probability of fully observed families ---------------------------------------------------------------------
+ * The read-side twin of cbn_count_run: for every row of a code matrix,
+ *     out[row] (+)= sum_f log_tables[ fams[f].table_offset + index_f(row) ]
+ * over families whose variables are all columns of the matrix.  With every family of the network this is the
+ * complete-data log-likelihood log P(x_row); with the families that lie inside an evidence set it is the observed share
+ * of log P(e_row) (cbn_ve_run_codes_log_evidence computes the rest).  Nothing in the reference computes this: new
+ * surface, like cbn_sample_forward.
+ *
+ * cbn_loglik_plan_create: fams[f].var[] are COLUMNS of the code matrix handed to cbn_loglik_run (not network ids);
+ * log_tables (device) holds the natural logs of the conditional tables, laid out as the count tables.  Families that
+ * share variables are merged into union tables holding the sums of their members' entries; the plan derives them from
+ * log_tables on `stream` and returns after that stream has drained: from then on the caller's buffer is not needed and
+ * the plan is immutable.
+ * cbn_loglik_run: out: device float [n]; accumulate = 1 adds into out (plain stream order: the launch does not overlap
+ * the kernel before it, so out may come from a gather kernel launched with programmatic dependent launch).  A code that
+ * is CBN_UNSEEN or >= the variable's cardinality makes the row -inf; no table is read out of range.  The terms of a row
+ * are added in a fixed order: the value of a row depends on that row only. */
+typedef struct cbn_loglik_plan cbn_loglik_plan;
+CBN_API int cbn_loglik_plan_create(cbn_ctx* ctx, const cbn_family* fams, int32_t n_fams, int32_t n_cols,
+                                   const float* log_tables, cbn_stream stream, cbn_loglik_plan** out);
+CBN_API void cbn_loglik_plan_destroy(cbn_loglik_plan* plan);
+CBN_API int cbn_loglik_run(cbn_ctx* ctx, const cbn_loglik_plan* plan, const uint8_t* codes, int64_t ld, int64_t n,
+                           float* out, int32_t accumulate, cbn_stream stream);
+/* introspection for the bench: table lookups per row after merging (<= number of families) */
+CBN_API int cbn_loglik_plan_tables(const cbn_loglik_plan* plan);
 
 /* ---- ancestral sampling (synthetic workloads; BruteForce._sample's network analogue,
  * brute_force.py:246-265).  Counter-based: sample i of variable v depends only on
