@@ -86,6 +86,19 @@ class RowStep(C.Structure):
     ]
 
 
+class MpeStep(C.Structure):
+    _fields_ = [
+        ("slot", C.c_int32),
+        ("card", C.c_int32),
+        ("argmax", C.c_void_p),
+        ("n_cells", C.c_int64),
+        ("n_ctx", C.c_int32),
+        ("ctx_slot", C.c_int32 * MAX_CONTRACT_DIMS),
+        ("ctx_stride", C.c_int32 * MAX_CONTRACT_DIMS),
+    ]
+
+
+MPE_MAX_SLOTS = 512
 ROWS_LOG_SPACE = 1
 GATHER_NORMALIZE, GATHER_LOG_SPACE = 1, 2
 HOST_OUT_DROP_LAST = 1
@@ -140,6 +153,11 @@ SIGNATURES = {
     "cbn_loglik_plan_destroy": (None, [_P]),
     "cbn_loglik_run": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, C.c_int32, _P]),
     "cbn_loglik_plan_tables": (C.c_int, [_P]),
+    "cbn_factor_contract_max": (C.c_int, [_P, C.POINTER(Contract), _P, _P]),
+    "cbn_mpe_plan_create": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(MpeStep), C.c_int32, _P,
+                                      C.POINTER(_P)]),
+    "cbn_mpe_plan_destroy": (None, [_P]),
+    "cbn_mpe_run": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, _P, C.c_int64, _P]),
     "cbn_ve_run_codes_host": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P]),
     "cbn_ve_run_codes_host_multi": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P)]),
     "cbn_ve_run_codes_host_multi_ex": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P), C.c_int32]),

@@ -14,6 +14,8 @@ or undefined, SURVEY.md section 3.3):
 * ``evidence=None`` works (prior marginal); ``do`` performs graph surgery.
 * ``log_likelihood(data)`` scores rows: ``log P(observed values of the row)`` for any subset of the nodes, the others
   summed out exactly (held-out log-likelihood, anomaly scores, probability of evidence); the reference has no such query.
+* ``most_probable_explanation(data)`` gives, per row, the jointly most probable values of every node not in ``data`` and
+  their log-probability ``log max_h P(h, e)`` (missing-value completion, diagnosis); the reference has no such query.
 """
 from __future__ import annotations
 
@@ -227,6 +229,27 @@ class BayesianNetwork:
         if log_evidence is None:
             raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not compute log P(e)")
         return log_evidence(cols)
+
+    def most_probable_explanation(self, data) -> Tuple[Dict[str, torch.Tensor], torch.Tensor]:
+        """Most probable explanation of each row: the jointly most likely values of every node NOT in ``data``,
+        ``argmax_h P(h, e)``, and their log-probability.
+
+        :param data: a DataFrame or a dict name -> values holding domain VALUES, as ``log_likelihood`` takes them; the
+                     observed set is the set of columns passed, the same for every row.  A column that is not a node
+                     raises ``ValueError``.
+        :return: ``(assignment, log_prob)``.  ``assignment`` maps every other node to float32 [n_rows] domain values on the
+                 device; ``log_prob`` is float32 [n_rows], ``log max_h P(h, e)`` (natural log).  A row with a value outside
+                 the fitted domain (NaN included) or evidence of probability zero gives ``log_prob = -inf`` and NaN in every
+                 assignment column (never a NaN ``log_prob``).  With no columns the result is one row, the explanation of
+                 the prior; with every node observed ``assignment`` is empty and ``log_prob`` equals ``log_likelihood``.
+                 The result is checkable: ``log_likelihood(data`` joined with ``assignment)`` equals ``log_prob`` within
+                 fp32 rounding.  The value of a row depends on that row only (any batching gives identical bits).
+        """
+        cols, _ = self._observed_columns(data)
+        mpe = getattr(self.inference_obj, "most_probable_explanation", None)
+        if mpe is None:
+            raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not compute explanations")
+        return mpe(cols)
 
     def _observed_columns(self, data) -> Tuple[Dict[str, torch.Tensor], int]:
         """``_columns`` for a subset of the nodes: (name -> float32 device column, number of rows)."""

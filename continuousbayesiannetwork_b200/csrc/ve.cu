@@ -25,10 +25,12 @@ __device__ __forceinline__ float lse_pair(float a, float b) {
   return (hi == NEG_INF) ? NEG_INF : hi + log1pf(expf(lo - hi));
 }
 
-// LOG: the tables hold logarithms -- products are sums, the sum over the eliminated variable is a log-sum-exp
-template <bool FAST, bool LOG>
+// LOG: the tables hold logarithms -- products are sums, the sum over the eliminated variable is a log-sum-exp.
+// MAX (requires LOG): max-sum instead -- the reduction keeps the largest term and its index s (strict >, so the smallest s
+// attaining the maximum), written to amax[o]; an all -inf reduction gives -inf and index 0.
+template <bool FAST, bool LOG, bool MAX = false>
 __global__ void __launch_bounds__(256) contract_kernel(const __grid_constant__ cbn_contract d, const __grid_constant__ ContractMagic mg,
-                                                       long long n_out) {
+                                                       long long n_out, uint8_t* __restrict__ amax) {
   for (long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x; o < n_out;
        o += (long long)gridDim.x * blockDim.x) {
     long long base[CBN_MAX_CONTRACT_INPUTS];
@@ -55,6 +57,7 @@ __global__ void __launch_bounds__(256) contract_kernel(const __grid_constant__ c
       }
     }
     float acc = LOG ? __int_as_float(0xff800000) : 0.0f;
+    int arg = 0;
     for (int s = 0; s < d.sum_card; ++s) {
       float prod = LOG ? 0.0f : 1.0f;
 #pragma unroll
@@ -63,9 +66,14 @@ __global__ void __launch_bounds__(256) contract_kernel(const __grid_constant__ c
           const float x = __ldg(d.in[k] + base[k] + (long long)s * d.sum_stride[k]);
           prod = LOG ? prod + x : prod * x;
         }
-      acc = LOG ? lse_pair(acc, prod) : acc + prod;
+      if constexpr (MAX) {
+        if (prod > acc) { acc = prod; arg = s; }
+      } else {
+        acc = LOG ? lse_pair(acc, prod) : acc + prod;
+      }
     }
     d.out[o] = acc;
+    if constexpr (MAX) amax[o] = (uint8_t)arg;
   }
 }
 
@@ -73,9 +81,9 @@ __global__ void __launch_bounds__(256) contract_kernel(const __grid_constant__ c
 // (LO <= 1024 cells).  The per-input offsets of every o_lo are decoded ONCE per CTA into shared memory, o_hi is decoded
 // once per (CTA, o_hi) instead of once per cell, and a cell costs n_in shared-memory reads plus its table loads -- the
 // plain kernel spends most of its time on the multiply-shift decode of up to 13 axes per cell.
-template <bool LOG, int NIN>
+template <bool LOG, int NIN, bool MAX = false>
 __global__ void __launch_bounds__(256) contract_tiled_kernel(const __grid_constant__ cbn_contract d, const __grid_constant__ ContractMagic mg,
-                                                             long long n_hi, int lo_cells, int n_lo_dims) {
+                                                             long long n_hi, int lo_cells, int n_lo_dims, uint8_t* __restrict__ amax) {
   extern __shared__ int lo_off[];          // [NIN][lo_cells]
   const int n_hi_dims = d.n_out_dims - n_lo_dims;
   for (int ol = threadIdx.x; ol < lo_cells; ol += blockDim.x) {
@@ -117,6 +125,7 @@ __global__ void __launch_bounds__(256) contract_tiled_kernel(const __grid_consta
 #pragma unroll
       for (int k = 0; k < NIN; ++k) p[k] = src[k] + hb[k] + lo_off[k * lo_cells + ol];
       float acc = LOG ? __int_as_float(0xff800000) : 0.0f;
+      int arg = 0;
       for (int sv = 0; sv < sum_card; ++sv) {
         float prod = LOG ? 0.0f : 1.0f;
 #pragma unroll
@@ -125,9 +134,14 @@ __global__ void __launch_bounds__(256) contract_tiled_kernel(const __grid_consta
           p[k] += ss[k];
           prod = LOG ? prod + x : prod * x;
         }
-        acc = LOG ? lse_pair(acc, prod) : acc + prod;
+        if constexpr (MAX) {
+          if (prod > acc) { acc = prod; arg = sv; }
+        } else {
+          acc = LOG ? lse_pair(acc, prod) : acc + prod;
+        }
       }
       out[ol] = acc;
+      if constexpr (MAX) amax[oh * lo_cells + ol] = (uint8_t)arg;
     }
   }
 }
@@ -209,21 +223,26 @@ extern "C" int cbn_factor_rescale(cbn_ctx* ctx, float* table, long long n_slices
   return CBN_OK;
 }
 
-extern "C" int cbn_factor_contract(cbn_ctx* ctx, const cbn_contract* desc, cbn_stream stream) {
-  if (!ctx) return cbn_fail(nullptr, CBN_ERR_INVALID, "cbn_factor_contract: ctx is NULL");
+namespace {
+int check_contract(cbn_ctx* ctx, const cbn_contract* desc, const char* fn, long long* n_out_ret) {
   if (!desc || !desc->out || desc->n_in < 1 || desc->n_in > CBN_MAX_CONTRACT_INPUTS || desc->n_out_dims < 0 ||
       desc->n_out_dims > CBN_MAX_CONTRACT_DIMS || desc->sum_card < 1)
-    return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_factor_contract: bad descriptor");
+    return cbn_fail(ctx, CBN_ERR_INVALID, "%s: bad descriptor", fn);
   long long n_out = 1;
   for (int a = 0; a < desc->n_out_dims; ++a) {
-    if (desc->out_card[a] < 1) return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_factor_contract: out_card[%d] < 1", a);
+    if (desc->out_card[a] < 1) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: out_card[%d] < 1", fn, a);
     n_out *= desc->out_card[a];
-    if (n_out > (1ll << 40)) return cbn_fail(ctx, CBN_ERR_UNSUPPORTED, "cbn_factor_contract: output too large");
+    if (n_out > (1ll << 40)) return cbn_fail(ctx, CBN_ERR_UNSUPPORTED, "%s: output too large", fn);
   }
   for (int k = 0; k < desc->n_in; ++k)
-    if (!desc->in[k]) return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_factor_contract: input %d is NULL", k);
-  DeviceGuard g(ctx->device);
-  cudaStream_t s = (cudaStream_t)stream;
+    if (!desc->in[k]) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: input %d is NULL", fn, k);
+  *n_out_ret = n_out;
+  return CBN_OK;
+}
+
+// MAX: the max-sum reduction of cbn_factor_contract_max (log space, no normalisation: checked by the caller)
+template <bool MAX>
+int launch_contract(cbn_ctx* ctx, const cbn_contract* desc, long long n_out, uint8_t* amax, cudaStream_t s) {
   int blocks = (int)std::min<long long>((n_out + 255) / 256, (long long)ctx->sm_count * 16);
   bool fast = n_out < (1ll << 31);
   ContractMagic mg{};
@@ -252,21 +271,51 @@ extern "C" int cbn_factor_contract(cbn_ctx* ctx, const cbn_contract* desc, cbn_s
       tiled = true;
       const int tb = (int)std::min<long long>(n_hi, (long long)ctx->sm_count * 8);
       const size_t sm = size_t(desc->n_in) * size_t(lo) * sizeof(int);
-#define CBN_TILED(L, K) contract_tiled_kernel<L, K><<<tb, 256, sm, s>>>(*desc, mg, n_hi, (int)lo, nlo)
-      switch (desc->n_in) {
-        case 1: if (lg) CBN_TILED(true, 1); else CBN_TILED(false, 1); break;
-        case 2: if (lg) CBN_TILED(true, 2); else CBN_TILED(false, 2); break;
-        case 3: if (lg) CBN_TILED(true, 3); else CBN_TILED(false, 3); break;
-        default: if (lg) CBN_TILED(true, 4); else CBN_TILED(false, 4); break;
-      }
+      if constexpr (MAX) {
+#define CBN_TILED(K) contract_tiled_kernel<true, K, true><<<tb, 256, sm, s>>>(*desc, mg, n_hi, (int)lo, nlo, amax)
+        switch (desc->n_in) {
+          case 1: CBN_TILED(1); break;
+          case 2: CBN_TILED(2); break;
+          case 3: CBN_TILED(3); break;
+          default: CBN_TILED(4); break;
+        }
 #undef CBN_TILED
+      } else {
+#define CBN_TILED(L, K) contract_tiled_kernel<L, K><<<tb, 256, sm, s>>>(*desc, mg, n_hi, (int)lo, nlo, nullptr)
+        switch (desc->n_in) {
+          case 1: if (lg) CBN_TILED(true, 1); else CBN_TILED(false, 1); break;
+          case 2: if (lg) CBN_TILED(true, 2); else CBN_TILED(false, 2); break;
+          case 3: if (lg) CBN_TILED(true, 3); else CBN_TILED(false, 3); break;
+          default: if (lg) CBN_TILED(true, 4); else CBN_TILED(false, 4); break;
+        }
+#undef CBN_TILED
+      }
     }
   }
   if (!tiled) {
-    if (fast) { if (lg) contract_kernel<true, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out); else contract_kernel<true, false><<<blocks, 256, 0, s>>>(*desc, mg, n_out); }
-    else { if (lg) contract_kernel<false, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out); else contract_kernel<false, false><<<blocks, 256, 0, s>>>(*desc, mg, n_out); }
+    if constexpr (MAX) {
+      if (fast) contract_kernel<true, true, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out, amax);
+      else contract_kernel<false, true, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out, amax);
+    } else {
+      if (fast) { if (lg) contract_kernel<true, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out, nullptr); else contract_kernel<true, false><<<blocks, 256, 0, s>>>(*desc, mg, n_out, nullptr); }
+      else { if (lg) contract_kernel<false, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out, nullptr); else contract_kernel<false, false><<<blocks, 256, 0, s>>>(*desc, mg, n_out, nullptr); }
+    }
   }
   CBN_CHECK_LAUNCH(ctx);
+  return CBN_OK;
+}
+}  // namespace
+
+extern "C" int cbn_factor_contract(cbn_ctx* ctx, const cbn_contract* desc, cbn_stream stream) {
+  if (!ctx) return cbn_fail(nullptr, CBN_ERR_INVALID, "cbn_factor_contract: ctx is NULL");
+  long long n_out = 0;
+  int rc = check_contract(ctx, desc, "cbn_factor_contract", &n_out);
+  if (rc) return rc;
+  DeviceGuard g(ctx->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  rc = launch_contract<false>(ctx, desc, n_out, nullptr, s);
+  if (rc) return rc;
+  const bool lg = desc->log_space != 0;
   if (desc->normalize_last && desc->n_out_dims > 0) {
     int card = desc->out_card[desc->n_out_dims - 1];
     long long rows = n_out / card;
@@ -276,6 +325,18 @@ extern "C" int cbn_factor_contract(cbn_ctx* ctx, const cbn_contract* desc, cbn_s
     CBN_CHECK_LAUNCH(ctx);
   }
   return CBN_OK;
+}
+
+extern "C" int cbn_factor_contract_max(cbn_ctx* ctx, const cbn_contract* desc, uint8_t* argmax_out, cbn_stream stream) {
+  if (!ctx) return cbn_fail(nullptr, CBN_ERR_INVALID, "cbn_factor_contract_max: ctx is NULL");
+  long long n_out = 0;
+  int rc = check_contract(ctx, desc, "cbn_factor_contract_max", &n_out);
+  if (rc) return rc;
+  if (!argmax_out || desc->log_space != 1 || desc->normalize_last != 0 || desc->sum_card > 255)
+    return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_factor_contract_max: needs log_space = 1, normalize_last = 0, sum_card <= 255 "
+                    "and an argmax buffer");
+  DeviceGuard g(ctx->device);
+  return launch_contract<true>(ctx, desc, n_out, argmax_out, (cudaStream_t)stream);
 }
 
 // =========================================================================== gather plan

@@ -7,7 +7,7 @@ import torch
 
 from .. import _native as N
 from ..base.inference import BaseInference
-from ..ve import EvidencePlan, FusedPlan, QueryPlan, RowPlan, VECompiler
+from ..ve import EvidencePlan, FusedPlan, MPEPlan, QueryPlan, RowPlan, VECompiler
 
 
 class ExactInference(BaseInference):
@@ -22,7 +22,8 @@ class ExactInference(BaseInference):
         self.normalization = (config or {}).get("normalization", "row")
         if self.normalization not in ("row", "global_max"):
             raise ValueError(f"normalization must be 'row' or 'global_max', got {self.normalization!r}")
-        self._budget = {k: int(config[k]) for k in ("table_budget_cells", "merge_budget_cells", "row_temp_floats")
+        self._budget = {k: int(config[k]) for k in ("table_budget_cells", "merge_budget_cells", "row_temp_floats",
+                                                    "mpe_argmax_budget_bytes")
                         if config and k in config}
         for k in ("log_space", "rescale", "profile_compile", "row_unit_layout"):
             if config and k in config:
@@ -106,6 +107,41 @@ class ExactInference(BaseInference):
         for e, (n, c) in enumerate(zip(names, cols)):
             t.encode(c.to(t.device, torch.float32, non_blocking=True), t.index[n], codes[e])
         return plan.run_codes(codes, nq)
+
+    def mpe_plan(self, evidence_names: Sequence[str]) -> MPEPlan:
+        assert self.compiler is not None, "inference engine is not bound to a fitted network"
+        return self.compiler.compile_mpe(list(evidence_names))
+
+    def most_probable_explanation(self, evidence: Dict[str, torch.Tensor]):
+        """Most probable explanation per row: ``(assignment, log_prob)``.  ``evidence``: name -> tensor [n_rows] or
+        [n_rows, 1] of category VALUES, the same observed set for every row.  ``assignment`` maps every other node to
+        float32 [n_rows] domain values of ``argmax_h P(h, e)`` (NaN where ``log_prob`` is -inf); ``log_prob`` is float32
+        [n_rows] ``log max_h P(h, e)`` (natural log; -inf for a value outside the fitted domain, NaN included, or evidence
+        of probability zero).  No evidence gives one row, the explanation of the prior.  Not part of the reference's
+        surface."""
+        t = self.tables
+        evidence = evidence or {}
+        names = list(evidence.keys())
+        for n in names:
+            if n not in t.index:
+                raise ValueError(f"{n} is not a node of the network")
+        cols = [torch.as_tensor(evidence[n]).reshape(-1) for n in names]
+        nq = int(cols[0].numel()) if cols else 1
+        if any(int(c.numel()) != nq for c in cols):
+            raise ValueError("all evidence columns must have the same number of rows")
+        plan = self.mpe_plan(names)
+        ld = (max(nq, 1) + 15) // 16 * 16
+        codes = torch.empty((max(len(names), 1), ld), dtype=torch.uint8, device=t.device)
+        for e, (n, c) in enumerate(zip(names, cols)):
+            t.encode(c.to(t.device, torch.float32, non_blocking=True), t.index[n], codes[e])
+        hidden, log_prob = plan.run_codes(codes, nq)
+        assignment = {}
+        for h, v in enumerate(plan.hidden):
+            c = hidden[h, :nq].long()
+            dead = c >= t.cards[v]
+            vals = t.domains[v][c.clamp(max=t.cards[v] - 1)]
+            assignment[t.names[v]] = torch.where(dead, torch.full_like(vals, float("nan")), vals)
+        return assignment, log_prob
 
     def infer_map(self, target_node: str, evidence: Dict[str, torch.Tensor]) -> Optional[torch.Tensor]:
         """MAP value of the target per row through the fused kernel (``cbn_ve_run_f32_map``); ``None`` when the plan is

@@ -19,6 +19,10 @@ of the hidden variables is eliminated per row by a schedule of product / sum-out
 Host work here is graph logic only (pruning, ordering with incremental bookkeeping, stride and
 offset tables); every floating-point operation runs on the device (``cbn_factor_contract`` at
 compile time, the gather / per-row kernels per evidence row).
+
+The same elimination with ``max`` in place of the sum (``VECompiler.compile_mpe``) gives the most probable explanation:
+every step also records its argmax table, and a per-row traceback (``cbn_mpe_run``) reads the hidden values back in
+reverse elimination order.
 """
 from __future__ import annotations
 
@@ -422,6 +426,85 @@ class EvidencePlan:
         return out
 
 
+@dataclass
+class MPESplit:
+    """Structure of a most-probable-explanation plan (``VECompiler.compile_mpe``)."""
+    evidence: List[int]
+    hidden: List[int]                                   # network ids; row h of the decoded code matrix is hidden[h]
+    observed_families: List[int]                        # CPTs scored by the observed-families kernel
+    decode: List[Tuple[int, Tuple[int, ...]]]           # (variable, scope of its argmax table) in decode order
+    argmax_bytes: int
+    stats: PlanStats
+
+
+class MPEPlan:
+    """A compiled most probable explanation: the argmax tables of the max-sum elimination, the native traceback plan
+    (``cbn_mpe_plan_create``) and the ``EvidencePlan`` that computes each row's value ``log max_h P(h, e)``."""
+
+    def __init__(self, tables_owner, split: MPESplit, decode, value: EvidencePlan):
+        self.owner = tables_owner
+        self.ctx = tables_owner.ctx
+        self.device = tables_owner.device
+        self.split = split
+        self.evidence = list(split.evidence)
+        self.hidden = list(split.hidden)
+        self.value = value
+        self.argmax = [am for _, _, am in decode]           # referenced by the native plan: kept alive with it
+        self.handle = None
+        cards = tables_owner.cards
+        n_ev = len(self.evidence)
+        slot = {v: i for i, v in enumerate(self.evidence)}
+        slot.update({v: n_ev + h for h, v in enumerate(self.hidden)})
+        if not self.hidden:
+            return
+        steps = (N.MpeStep * len(decode))()
+        for k, (v, scope, am) in enumerate(decode):
+            st = steps[k]
+            st.slot = slot[v]
+            st.card = cards[v]
+            st.argmax = am.data_ptr()
+            st.n_cells = am.numel()
+            st.n_ctx = len(scope)
+            stride = 1
+            for j in range(len(scope) - 1, -1, -1):
+                st.ctx_slot[j] = slot[scope[j]]
+                st.ctx_stride[j] = stride
+                stride *= cards[scope[j]]
+        ev_cards = (C.c_int32 * max(n_ev, 1))(*[cards[v] for v in self.evidence])
+        h = C.c_void_p()
+        N.check(N.lib().cbn_mpe_plan_create(self.ctx.handle, n_ev, ev_cards, len(self.hidden), steps, len(decode),
+                                            N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
+        self.handle = h
+
+    def __del__(self):
+        try:
+            if self.handle is not None:
+                N.lib().cbn_mpe_plan_destroy(self.handle)
+                self.handle = None
+        except Exception:
+            pass
+
+    def set_static_evidence(self, on: bool = True):
+        self.value.set_static_evidence(on)
+
+    def run_codes(self, ev_codes: torch.Tensor, n_rows: int, hidden_out: Optional[torch.Tensor] = None,
+                  value_out: Optional[torch.Tensor] = None):
+        """ev_codes: uint8 [len(evidence), ld] on the device (row e = evidence variable e of the plan, ld a multiple of
+        16).  Returns ``(hidden_codes, log_value)``: uint8 [len(hidden), ld'] (row h = network variable ``hidden[h]``,
+        CBN_UNSEEN in every row whose value is -inf) and float32 [n_rows] ``log max_h P(h, e_row)``."""
+        assert ev_codes.dtype == torch.uint8 and ev_codes.is_cuda
+        value = self.value.run_codes(ev_codes, n_rows, value_out)
+        if hidden_out is None:
+            ld = (max(n_rows, 1) + 15) // 16 * 16
+            hidden_out = torch.empty((len(self.hidden), ld), dtype=torch.uint8, device=self.device)
+        if self.handle is not None and n_rows > 0:
+            ld = ev_codes.stride(0) if ev_codes.dim() == 2 else 0
+            N.check(N.lib().cbn_mpe_run(self.ctx.handle, self.handle, ev_codes.data_ptr(), ld, int(n_rows), value.data_ptr(),
+                                        hidden_out.data_ptr(), hidden_out.stride(0), N.stream_ptr(self.device)),
+                    self.ctx.handle)
+        return hidden_out, value
+
+
 class _Greedy:
     """Greedy min-size elimination with incremental bookkeeping: the scope a variable's elimination would create is
     cached and only recomputed for the variables that share a factor with the one just eliminated (the full rescan is
@@ -491,7 +574,7 @@ class VECompiler:
 
     def __init__(self, tables, table_budget_cells: int = 1 << 28, merge_budget_cells: int = 1 << 24,
                  check_support: bool = True, row_temp_floats: int = 5000, log_space: bool = False, rescale: bool = True,
-                 profile_compile: bool = False, row_unit_layout: bool = True):
+                 profile_compile: bool = False, row_unit_layout: bool = True, mpe_argmax_budget_bytes: int = 1 << 30):
         self.t = tables
         # range control of the compile-time elimination: after every contraction each evidence slice of the result is
         # divided by its maximum (cbn_factor_rescale) -- a factor of the evidence configuration only, which cancels in the
@@ -512,6 +595,8 @@ class VECompiler:
         self._ev_child: Optional["VECompiler"] = None       # the evidence-mode compiler (log space, no range control)
         self._ev_cache: Dict[tuple, "EvidencePlan"] = {}
         self._ev_cache_version = None
+        self.mpe_argmax_budget = int(mpe_argmax_budget_bytes)    # argmax tables of one MPE plan, in bytes
+        self._mpe_cache: Dict[tuple, "MPEPlan"] = {}
 
     # ---------------------------------------------------------------- graph helpers
     def _parents(self, v: int) -> List[int]:
@@ -537,7 +622,9 @@ class VECompiler:
 
     # ---------------------------------------------------------------- device contraction
     def _contract(self, inputs: List[Factor], out_scope: List[int], sum_var: Optional[int], dry: bool,
-                  normalize_last: bool = False) -> Factor:
+                  normalize_last: bool = False, argmax: Optional[torch.Tensor] = None) -> Factor:
+        """``argmax``: uint8 device buffer of the output's size -- maximise over ``sum_var`` instead of summing
+        (``cbn_factor_contract_max``, log space) and record the maximising value of every output cell there."""
         cards = self.t.cards
         if dry:
             return Factor(out_scope, None)
@@ -569,7 +656,11 @@ class VECompiler:
         if self.profile_compile:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-        N.check(N.lib().cbn_factor_contract(self.t.ctx.handle, C.byref(d), N.stream_ptr(self.t.device)), self.t.ctx.handle)
+        if argmax is not None:
+            N.check(N.lib().cbn_factor_contract_max(self.t.ctx.handle, C.byref(d), argmax.data_ptr(), N.stream_ptr(self.t.device)),
+                    self.t.ctx.handle)
+        else:
+            N.check(N.lib().cbn_factor_contract(self.t.ctx.handle, C.byref(d), N.stream_ptr(self.t.device)), self.t.ctx.handle)
         if self.rescale and not normalize_last:
             # evidence axes are the slowest axes of every factor (sort_scope): one contiguous slice per evidence configuration
             lead = 0
@@ -737,26 +828,13 @@ class VECompiler:
 
         ``dry=True`` works on ``DryTables`` and returns the ``EvidenceSplit`` only (no device work)."""
         if not self.log_space or self.rescale:
-            if self._ev_child is None:
-                self._ev_child = VECompiler(self.t, table_budget_cells=self.table_budget, merge_budget_cells=self.merge_budget,
-                                            check_support=False, row_temp_floats=self.row_temp_floats, log_space=True,
-                                            rescale=False, profile_compile=self.profile_compile,
-                                            row_unit_layout=self.row_unit_layout)
-            return self._ev_child.compile_evidence(evidence_names, dry=dry)
+            return self._evidence_child().compile_evidence(evidence_names, dry=dry)
         t = self.t
         cards = t.cards
-        for e in evidence_names:
-            if e not in t.index:
-                raise ValueError(f"{e} is not a node of the network")
-        E = [t.index[e] for e in evidence_names]
-        if len(set(E)) != len(E):
-            raise ValueError("an evidence variable is listed twice")
+        E = self._evidence_ids(evidence_names)
         key = tuple(E)
         if not dry:
-            version = getattr(t, "cond_version", 0)
-            if self._ev_cache_version != version:          # re-fitted tables: every cached plan is stale
-                self._ev_cache = {}
-                self._ev_cache_version = version
+            self._drop_stale_plans()
             if key in self._ev_cache:
                 return self._ev_cache[key]
             # structure-only pass first: a query that does not fit fails here, before any table is contracted
@@ -809,6 +887,114 @@ class VECompiler:
         self._ev_cache[key] = plan
         return plan
 
+    def _evidence_child(self) -> "VECompiler":
+        """The evidence-mode compiler (log space, no range control, no support pruning) over the same tables."""
+        if self._ev_child is None:
+            self._ev_child = VECompiler(self.t, table_budget_cells=self.table_budget, merge_budget_cells=self.merge_budget,
+                                        check_support=False, row_temp_floats=self.row_temp_floats, log_space=True,
+                                        rescale=False, profile_compile=self.profile_compile,
+                                        row_unit_layout=self.row_unit_layout, mpe_argmax_budget_bytes=self.mpe_argmax_budget)
+        return self._ev_child
+
+    def _evidence_ids(self, evidence_names: Sequence[str]) -> List[int]:
+        t = self.t
+        for e in evidence_names:
+            if e not in t.index:
+                raise ValueError(f"{e} is not a node of the network")
+        E = [t.index[e] for e in evidence_names]
+        if len(set(E)) != len(E):
+            raise ValueError("an evidence variable is listed twice")
+        return E
+
+    def _drop_stale_plans(self):
+        version = getattr(self.t, "cond_version", 0)
+        if self._ev_cache_version != version:          # re-fitted tables: every cached plan is stale
+            self._ev_cache = {}
+            self._mpe_cache = {}
+            self._ev_cache_version = version
+
+    # ---------------------------------------------------------------- MPE mode: argmax_h P(h, e)
+    def compile_mpe(self, evidence_names: Sequence[str], dry: bool = False):
+        """Compile the most probable explanation for the evidence set ``evidence_names``: per row, the jointly most
+        probable value of EVERY other node, ``argmax_h P(h, e)``, and ``log max_h P(h, e)``.
+
+        The elimination of ``compile_evidence`` with max in place of log-sum-exp, over every CPT of the network (barren
+        descendants are not summed out here: their values are part of the answer).  CPTs whose scope lies inside ``E`` go to
+        the observed-families kernel.  Every hidden variable is eliminated by ``cbn_factor_contract_max``, which also
+        records the argmax table of the step; what is left are tables over evidence subsets, so the value of a row is
+        exactly what an ``EvidencePlan`` computes from them.  The traceback (``cbn_mpe_run``) decodes the hidden values
+        in reverse elimination order.  There is no per-row executor for MPE: a step beyond the table budget, argmax tables
+        beyond ``mpe_argmax_budget_bytes`` or a row of more than ``N.MPE_MAX_SLOTS`` codes raise ``PlanTooLarge`` in the
+        structure-only pass, before any table is contracted.
+
+        ``dry=True`` works on ``DryTables`` and returns the ``MPESplit`` only (no device work)."""
+        if not self.log_space or self.rescale:
+            return self._evidence_child().compile_mpe(evidence_names, dry=dry)
+        t = self.t
+        cards = t.cards
+        E = self._evidence_ids(evidence_names)
+        key = tuple(E)
+        if not dry:
+            self._drop_stale_plans()
+            if key in self._mpe_cache:
+                return self._mpe_cache[key]
+            self.compile_mpe(evidence_names, dry=True)      # the limits fail here, before any table is contracted
+            self._events = []
+        Eset = set(E)
+        self._ev_set = Eset
+        order_key = {v: i for i, v in enumerate(E)}
+
+        def sort_scope(scope) -> List[int]:
+            return sorted(set(scope), key=lambda v: (0 if v in Eset else 1, order_key.get(v, v)))
+
+        stats = PlanStats()
+        stats.n_relevant = len(t.names)
+        observed: List[int] = []
+        factors: List[Factor] = []
+        for v in range(len(t.names)):
+            scope = t.family_vars(t.names[v])
+            if all(u in Eset for u in scope):
+                observed.append(v)
+                continue
+            tensor = None if dry else t.table_view(t.log_cond, t.names[v]).reshape(-1)
+            factors.append(Factor(list(scope), tensor))
+        hidden = [v for v in range(len(t.names)) if v not in Eset]
+        stats.n_hidden = len(hidden)
+        stats.relevant_evidence = list(E)
+        elim: list = []
+        finals: List[Factor] = []
+        if factors:
+            finals = self._eliminate(factors, hidden, sort_scope, stats, dry, None, decode=elim)
+        argmax_bytes = sum(max(_prod(cards[u] for u in sc), 1) for _, sc, _ in elim)
+        if dry:
+            if argmax_bytes > self.mpe_argmax_budget:
+                raise PlanTooLarge(f"the argmax tables of this explanation need {argmax_bytes} bytes "
+                                   f"(budget {self.mpe_argmax_budget})")
+            widest = max((len(sc) for _, sc, _ in elim), default=0)
+            if widest > N.MAX_CONTRACT_DIMS:
+                raise PlanTooLarge(f"an argmax table with {widest} axes exceeds {N.MAX_CONTRACT_DIMS}")
+            ev_read = {u for _, sc, _ in elim for u in sc if u in Eset}
+            if len(ev_read) + len(hidden) > N.MPE_MAX_SLOTS:
+                raise PlanTooLarge(f"{len(ev_read)} evidence columns and {len(hidden)} hidden variables exceed the "
+                                   f"{N.MPE_MAX_SLOTS} codes the traceback keeps per row")
+        ve_plan = None
+        if finals:
+            finals = self._merge_finals(finals, sort_scope, stats, dry, None)
+            stats.final_tables = [(tuple(f.scope), f.size(cards)) for f in finals]
+            if not dry:
+                ve_plan = QueryPlan(t, None, E, 1, finals, True, stats, log_space=True)
+        decode = [(v, tuple(sc), am) for v, sc, am in reversed(elim)]
+        split = MPESplit(evidence=list(E), hidden=hidden, observed_families=observed,
+                         decode=[(v, sc) for v, sc, _ in decode], argmax_bytes=argmax_bytes, stats=stats)
+        if dry:
+            return split
+        stats.contraction_gpu_ms = self._drain_events()
+        value = EvidencePlan(t, E, observed, ve_plan,
+                             EvidenceSplit(evidence=list(E), observed_families=observed, ve_stats=stats if factors else None))
+        plan = MPEPlan(t, split, decode, value)
+        self._mpe_cache[key] = plan
+        return plan
+
     def _drain_events(self) -> float:
         if not self._events:
             return 0.0
@@ -818,9 +1004,12 @@ class VECompiler:
         return ms
 
     def _eliminate(self, factors: List[Factor], hidden: List[int], sort_scope, stats: PlanStats, dry: bool, T: int,
-                   partial: bool = False):
+                   partial: bool = False, decode: Optional[list] = None):
         """Evidence-symbolic elimination.  With ``partial`` the loop stops when the cheapest step exceeds the table
-        budget and returns ``(factors, remaining_hidden)`` for the per-row executor instead of raising."""
+        budget and returns ``(factors, remaining_hidden)`` for the per-row executor instead of raising.
+
+        With a ``decode`` list the elimination is max-sum (log space): every step maximises over its variable and appends
+        ``(variable, output scope, argmax table)`` to the list (the table is None in a dry run)."""
         cards = self.t.cards
         live: Dict[int, Factor] = dict(enumerate(factors))
         next_key = len(factors)
@@ -839,7 +1028,9 @@ class VECompiler:
             if best_cost > self.table_budget:
                 raise PlanTooLarge(
                     f"eliminating the cheapest hidden variable needs a table of {best_cost} cells "
-                    f"(budget {self.table_budget}); this query needs the per-row executor")
+                    f"(budget {self.table_budget}); " +
+                    ("the most probable explanation has no per-row executor" if decode is not None else
+                     "this query needs the per-row executor"))
             keys = g.touching(v)
             touching = [live[k] for k in keys]
             # the kernel multiplies at most MAX_CONTRACT_INPUTS factors at once: pre-multiply the smallest ones
@@ -863,7 +1054,12 @@ class VECompiler:
             stats.n_steps += 1
             stats.max_table_cells = max(stats.max_table_cells, best_cost)
             stats.contraction_madds += best_cost * cards[v] * len(touching)
-            res = self._contract(touching, out_scope, v, dry)
+            if decode is not None:
+                am = None if dry else torch.empty(max(best_cost, 1), dtype=torch.uint8, device=self.t.device)
+                res = self._contract(touching, out_scope, v, dry, argmax=am)
+                decode.append((v, out_scope, am))
+            else:
+                res = self._contract(touching, out_scope, v, dry)
             for k in keys:
                 del live[k]
             live[next_key] = res

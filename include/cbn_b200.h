@@ -201,6 +201,12 @@ typedef struct cbn_contract {
                              normalize_last the output is the LINEAR normalised distribution (softmax of the slice) */
 } cbn_contract;
 CBN_API int cbn_factor_contract(cbn_ctx* ctx, const cbn_contract* desc, cbn_stream stream);
+/* One max-sum step of a most-probable-explanation elimination, on the same descriptor:
+ *     out[o]        = max_{s < sum_card} sum_k in_k[ o . stride_k + s * sum_stride_k ]
+ *     argmax_out[o] = the smallest s attaining that maximum (strict > on the fp32 values as computed)
+ * An all -inf reduction gives -inf and index 0.  Requires log_space = 1, normalize_last = 0, sum_card <= 255 and a
+ * non-NULL argmax_out (device uint8 [n_out]); anything else is CBN_ERR_INVALID. */
+CBN_API int cbn_factor_contract_max(cbn_ctx* ctx, const cbn_contract* desc, uint8_t* argmax_out, cbn_stream stream);
 /* Range control of the compile-time elimination (the linear-space counterpart of working in log space): `table` holds
  * n_slices contiguous slices of slice_size cells -- one slice per configuration of the factor's evidence axes, which are
  * its slowest axes -- and every slice is divided by its own maximum (all-zero slices stay zero).  A factor that depends on
@@ -357,6 +363,43 @@ CBN_API int cbn_loglik_run(cbn_ctx* ctx, const cbn_loglik_plan* plan, const uint
                            float* out, int32_t accumulate, cbn_stream stream);
 /* introspection for the bench: table lookups per row after merging (<= number of families) */
 CBN_API int cbn_loglik_plan_tables(const cbn_loglik_plan* plan);
+
+/* ---- most probable explanation: the traceback ---------------------------------------------------------------------
+ * After a max-sum elimination (cbn_factor_contract_max) of every hidden variable with the evidence kept symbolic, the
+ * jointly most probable hidden values of a row are read back from the argmax tables in reverse elimination order.  A row
+ * keeps one code per SLOT: slots 0 .. n_evidence-1 are the evidence columns of ev_codes, slot n_evidence + h is hidden
+ * variable h.  Step k (in decode order) writes
+ *     code[slot_k] = argmax_k[ sum_j code[ctx_slot_k_j] * ctx_stride_k_j ]
+ * where every context slot is evidence or was written by an earlier step.  Nothing in the reference computes this.
+ *
+ * cbn_mpe_plan_create: checks that every context slot is evidence or written earlier, that every hidden slot is written
+ * exactly once (n_steps == n_hidden), that cardinalities lie in [1, 255] and that the largest index of every table is
+ * below its n_cells (CBN_ERR_INVALID otherwise).  The kernel keeps a row's codes in shared memory: the evidence columns
+ * some table reads plus the hidden variables may be at most CBN_MPE_MAX_SLOTS (CBN_ERR_UNSUPPORTED beyond).  Small argmax
+ * tables are copied into the plan (staged in shared memory at run time); larger ones are read where they are, so the
+ * caller keeps them alive as long as the plan.  Uploads run on `stream`, and the function returns when it has drained.
+ * cbn_mpe_run: hidden_codes: device uint8, hidden variable h at hidden_codes + h * out_ld (out_ld >= n_rows, a multiple
+ * of 16, 16-byte aligned base; ev_codes likewise), so the hidden codes stack with the evidence into complete rows.
+ * log_value: device float [n_rows], the row's log max_h P(h, e) (EvidencePlan of the same elimination).  A row whose
+ * log_value is -inf or NaN, or whose evidence code is not below its cardinality, gets CBN_UNSEEN in every hidden column.
+ * Indices are clamped: no table is read out of range.  Launched without programmatic dependent launch, so log_value may
+ * come from the kernel right before it on the stream. */
+#define CBN_MPE_MAX_SLOTS 512
+typedef struct cbn_mpe_plan cbn_mpe_plan;
+typedef struct cbn_mpe_step {
+  int32_t slot;                              /* slot this step writes: n_evidence + h for hidden variable h */
+  int32_t card;                              /* that variable's cardinality (<= 255) */
+  const uint8_t* argmax;                     /* device */
+  int64_t n_cells;
+  int32_t n_ctx;                             /* axes the table is indexed by */
+  int32_t ctx_slot[CBN_MAX_CONTRACT_DIMS];   /* evidence slots, or hidden slots written by an EARLIER step */
+  int32_t ctx_stride[CBN_MAX_CONTRACT_DIMS];
+} cbn_mpe_step;
+CBN_API int cbn_mpe_plan_create(cbn_ctx* ctx, int32_t n_evidence, const int32_t* ev_cards, int32_t n_hidden,
+                                const cbn_mpe_step* steps, int32_t n_steps, cbn_stream stream, cbn_mpe_plan** out);
+CBN_API void cbn_mpe_plan_destroy(cbn_mpe_plan* plan);
+CBN_API int cbn_mpe_run(cbn_ctx* ctx, const cbn_mpe_plan* plan, const uint8_t* ev_codes, int64_t ld, int64_t n_rows,
+                        const float* log_value, uint8_t* hidden_codes, int64_t out_ld, cbn_stream stream);
 
 /* ---- ancestral sampling (synthetic workloads; BruteForce._sample's network analogue,
  * brute_force.py:246-265).  Counter-based: sample i of variable v depends only on
