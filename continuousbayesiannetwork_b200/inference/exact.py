@@ -15,7 +15,6 @@ class ExactInference(BaseInference):
         super(ExactInference, self).__init__(config=config, **kwargs)
         self.normalization = "row"
         self.compiler: Optional[VECompiler] = None
-        self._fused: Dict[tuple, FusedPlan] = {}
         self._setup_model(config, **kwargs)
 
     def _setup_model(self, config: Dict, **kwargs):
@@ -33,7 +32,6 @@ class ExactInference(BaseInference):
         """Attach the fitted network tables (called by BayesianNetwork after every fit)."""
         self.tables = tables
         self.compiler = VECompiler(tables, **self._budget)
-        self._fused: Dict[tuple, FusedPlan] = {}
 
     def plan(self, target_node: str, evidence_names: Sequence[str], do: Sequence[str] = ()) -> QueryPlan:
         assert self.compiler is not None, "inference engine is not bound to a fitted network"
@@ -43,6 +41,26 @@ class ExactInference(BaseInference):
         """One launch for several targets that share the evidence list (same target cardinality)."""
         return FusedPlan([self.plan(t, evidence_names) for t in targets])
 
+    def _columns(self, evidence: Dict[str, torch.Tensor], names: Sequence[str], n_empty: int = 1,
+                 mismatch: str = "n_queries must be equal for all features."):
+        """``evidence[n]`` for ``names`` (tensors [n_rows] or [n_rows, 1] of category VALUES) as contiguous float32 device
+        columns, and their common number of rows (``n_empty`` when there is no column)."""
+        t = self.tables
+        for n in names:
+            if n not in t.index:
+                raise ValueError(f"{n} is not a node of the network")
+        cols = [torch.as_tensor(evidence[n]).to(t.device, torch.float32, non_blocking=True).reshape(-1).contiguous()
+                for n in names]
+        nq = int(cols[0].numel()) if cols else n_empty
+        if any(int(c.numel()) != nq for c in cols):
+            raise ValueError(mismatch)
+        return cols, nq
+
+    def _codes(self, evidence: Dict[str, torch.Tensor], names: Sequence[str], **kw):
+        """``_columns`` encoded on the device: (uint8 code matrix, row e = ``names[e]``; number of rows)."""
+        cols, nq = self._columns(evidence, names, **kw)
+        return self.tables.encode_evidence([self.tables.index[n] for n in names], cols, nq), nq
+
     def infer_many(self, targets: Sequence[str], evidence: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
         """Posteriors of SEVERAL targets under the same evidence: the evidence columns are uploaded and encoded once,
         and targets of equal cardinality are answered by one fused launch (``cbn_ve_plan_fuse``).  Not part of the
@@ -51,17 +69,10 @@ class ExactInference(BaseInference):
         t = self.tables
         evidence = evidence or {}
         names = [n for n in evidence.keys() if n not in targets]
-        for n in list(names) + list(targets):
+        for n in targets:
             if n not in t.index:
                 raise ValueError(f"{n} is not a node of the network")
-        nq = int(evidence[names[0]].shape[0]) if names else 1
-        ld = (max(nq, 1) + 15) // 16 * 16
-        codes = torch.empty((max(len(names), 1), ld), dtype=torch.uint8, device=t.device)
-        for e, n in enumerate(names):
-            c = evidence[n]
-            if c.shape[0] != nq:
-                raise ValueError("n_queries must be equal for all features.")
-            t.encode(c.to(t.device, torch.float32, non_blocking=True).reshape(-1), t.index[n], codes[e])
+        codes, nq = self._codes(evidence, names)
         out: Dict[str, torch.Tensor] = {}
         by_card: Dict[int, list] = {}
         for tg in targets:
@@ -72,10 +83,7 @@ class ExactInference(BaseInference):
             for i in range(0, len(group), 8 if fusable else 1):
                 chunk = group[i: i + 8]
                 if fusable and len(chunk) > 1:
-                    key = ("fused", tuple(chunk), tuple(names))
-                    fused = self._fused.get(key)
-                    if fused is None:
-                        fused = self._fused[key] = FusedPlan(plans[i: i + 8])
+                    fused = self.compiler.cached(("fused", tuple(chunk), tuple(names)), lambda: FusedPlan(plans[i: i + 8]))
                     for tg, o in zip(chunk, fused.run_codes(codes, nq)):
                         out[tg] = o
                 else:
@@ -91,22 +99,9 @@ class ExactInference(BaseInference):
         [n_rows, 1] of category VALUES, the same observed set for every row; every other node is summed out exactly.
         -inf for a value outside the fitted domain (NaN included) or evidence of probability zero; an empty dict gives an
         empty result.  Not part of the reference's surface."""
-        t = self.tables
-        evidence = evidence or {}
-        names = list(evidence.keys())
-        for n in names:
-            if n not in t.index:
-                raise ValueError(f"{n} is not a node of the network")
-        cols = [torch.as_tensor(evidence[n]).reshape(-1) for n in names]
-        nq = int(cols[0].numel()) if cols else 0
-        if any(int(c.numel()) != nq for c in cols):
-            raise ValueError("all evidence columns must have the same number of rows")
-        plan = self.evidence_plan(names)
-        ld = (max(nq, 1) + 15) // 16 * 16
-        codes = torch.empty((max(len(names), 1), ld), dtype=torch.uint8, device=t.device)
-        for e, (n, c) in enumerate(zip(names, cols)):
-            t.encode(c.to(t.device, torch.float32, non_blocking=True), t.index[n], codes[e])
-        return plan.run_codes(codes, nq)
+        names = list(evidence or {})
+        codes, nq = self._codes(evidence, names, n_empty=0, mismatch="all evidence columns must have the same number of rows")
+        return self.evidence_plan(names).run_codes(codes, nq)
 
     def mpe_plan(self, evidence_names: Sequence[str]) -> MPEPlan:
         assert self.compiler is not None, "inference engine is not bound to a fitted network"
@@ -120,20 +115,9 @@ class ExactInference(BaseInference):
         of probability zero).  No evidence gives one row, the explanation of the prior.  Not part of the reference's
         surface."""
         t = self.tables
-        evidence = evidence or {}
-        names = list(evidence.keys())
-        for n in names:
-            if n not in t.index:
-                raise ValueError(f"{n} is not a node of the network")
-        cols = [torch.as_tensor(evidence[n]).reshape(-1) for n in names]
-        nq = int(cols[0].numel()) if cols else 1
-        if any(int(c.numel()) != nq for c in cols):
-            raise ValueError("all evidence columns must have the same number of rows")
+        names = list(evidence or {})
+        codes, nq = self._codes(evidence, names, mismatch="all evidence columns must have the same number of rows")
         plan = self.mpe_plan(names)
-        ld = (max(nq, 1) + 15) // 16 * 16
-        codes = torch.empty((max(len(names), 1), ld), dtype=torch.uint8, device=t.device)
-        for e, (n, c) in enumerate(zip(names, cols)):
-            t.encode(c.to(t.device, torch.float32, non_blocking=True), t.index[n], codes[e])
         hidden, log_prob = plan.run_codes(codes, nq)
         assignment = {}
         for h, v in enumerate(plan.hidden):
@@ -146,22 +130,12 @@ class ExactInference(BaseInference):
     def infer_map(self, target_node: str, evidence: Dict[str, torch.Tensor]) -> Optional[torch.Tensor]:
         """MAP value of the target per row through the fused kernel (``cbn_ve_run_f32_map``); ``None`` when the plan is
         not a single-target gather plan with at most 8 target values (the caller then takes posterior + argmax)."""
-        t = self.tables
         evidence = evidence or {}
         names = [n for n in evidence.keys() if n != target_node]
-        for n in names:
-            if n not in t.index:
-                raise ValueError(f"evidence variable {n} is not a node of the network")
+        cols, nq = self._columns(evidence, names)
         plan = self.plan(target_node, names)
         if not isinstance(plan, QueryPlan) or plan.card_t > N.GATHER_MAX_CT or len(names) > N.MAX_EVIDENCE_PTRS:
             return None
-        nq = int(evidence[names[0]].shape[0]) if names else 1
-        cols = []
-        for n in names:
-            c = evidence[n]
-            if c.shape[0] != nq:
-                raise ValueError("n_queries must be equal for all features.")
-            cols.append(c.to(t.device, torch.float32, non_blocking=True).reshape(-1).contiguous())
         return plan.run_f32_map(cols, nq)
 
     def _infer(self, target_node: str, evidence: Dict[str, torch.Tensor], do=None, **kwargs) -> torch.Tensor:
@@ -172,21 +146,8 @@ class ExactInference(BaseInference):
         t = self.tables
         evidence = evidence or {}
         names = [n for n in evidence.keys() if n != target_node]
-        for n in names:
-            if n not in t.index:
-                raise ValueError(f"evidence variable {n} is not a node of the network")
-        plan = self.plan(target_node, names, do=do or ())
-        if names:
-            nq = int(evidence[names[0]].shape[0])
-            cols = []
-            for n in names:
-                c = evidence[n]
-                if c.shape[0] != nq:
-                    raise ValueError("n_queries must be equal for all features.")
-                cols.append(c.to(t.device, torch.float32, non_blocking=True).reshape(-1).contiguous())
-        else:
-            nq, cols = 1, []
-        out = plan.run_f32(cols, nq)
+        cols, nq = self._columns(evidence, names)
+        out = self.plan(target_node, names, do=do or ()).run_f32(cols, nq)
         norm = kwargs.get("normalization", self.normalization)
         if norm == "global_max":
             m = torch.zeros(1, dtype=torch.float32, device=t.device)

@@ -233,9 +233,18 @@ class DiscreteTables:
                                        self.cards[var], out.data_ptr(), unseen.data_ptr() if unseen is not None else None,
                                        N.stream_ptr(self.device)), self.ctx.handle)
 
-    def new_code_matrix(self, n: int) -> torch.Tensor:
+    def new_code_matrix(self, n: int, n_vars: Optional[int] = None) -> torch.Tensor:
+        """uint8 [n_vars (default: every variable), ld] for ``n`` samples; ld is a multiple of 16."""
         ld = _round_up(max(n, 1), 16)
-        return torch.empty((len(self.names), ld), dtype=torch.uint8, device=self.device)
+        return torch.empty((len(self.names) if n_vars is None else n_vars, ld), dtype=torch.uint8, device=self.device)
+
+    def encode_evidence(self, variables: Sequence[int], cols: Sequence[torch.Tensor], n: int) -> torch.Tensor:
+        """Evidence columns of category VALUES -> uint8 code matrix [max(len(variables), 1), ld] whose row e holds the
+        codes of ``cols[e]`` for variable ``variables[e]`` (an unseen value, NaN included, becomes CBN_UNSEEN)."""
+        codes = self.new_code_matrix(n, max(len(variables), 1))
+        for e, (v, col) in enumerate(zip(variables, cols)):
+            self.encode(col, v, codes[e])
+        return codes
 
     def _domain_matrix(self):
         """All domains as one device matrix [n_vars, 256] + cardinalities (built once per ``set_domains``)."""

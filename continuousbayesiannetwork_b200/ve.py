@@ -27,7 +27,8 @@ reverse elimination order.
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass, field
+import math
+from dataclasses import dataclass, field, replace
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
@@ -39,23 +40,33 @@ class PlanTooLarge(NotImplementedError):
     pass
 
 
-def _prod(it) -> int:
-    p = 1
-    for x in it:
-        p *= int(x)
-    return p
+def _cells(scope, cards) -> int:
+    """Cells of a table over ``scope``."""
+    return math.prod(cards[v] for v in scope)
+
+
+def _strides(scope, cards) -> Dict[int, int]:
+    """Variable -> stride of its axis in a row-major table over ``scope`` (last variable fastest)."""
+    st, s = {}, 1
+    for v in reversed(scope):
+        st[v] = s
+        s *= cards[v]
+    return st
+
+
+def _ld(ev_codes: torch.Tensor) -> int:
+    """Leading dimension of an evidence code matrix (0 for a single row vector)."""
+    return ev_codes.stride(0) if ev_codes.dim() == 2 else 0
+
+
+def _int32s(values):
+    return (C.c_int32 * max(len(values), 1))(*values)
 
 
 @dataclass
 class Factor:
     scope: List[int]                     # variable ids; tensor is row-major over this list
     tensor: Optional[torch.Tensor]       # float32 device tensor (None in dry-run)
-
-    def size(self, cards) -> int:
-        s = 1
-        for v in self.scope:
-            s *= cards[v]
-        return s
 
 
 @dataclass
@@ -74,85 +85,106 @@ class PlanStats:
     relevant_evidence: List[int] = field(default_factory=list)
 
 
-class QueryPlan:
-    """A compiled (target, evidence-set) query.  Owns the final tables and the native plan."""
+class _NativePlan:
+    """Owner of one native plan: ``handle`` is released by the C function ``_destroy`` when the owner is collected."""
+    _destroy = "cbn_ve_plan_destroy"
+    handle = None
 
-    def __init__(self, tables_owner, target: int, evidence: List[int], card_t: int, finals: List[Factor],
-                 normalize: bool, stats: PlanStats, log_space: bool = False):
+    def __init__(self, tables_owner):
         self.owner = tables_owner
         self.ctx = tables_owner.ctx
         self.device = tables_owner.device
-        self.target = target
-        self.evidence = list(evidence)
-        self.card_t = card_t
-        self.finals = finals
-        self.normalize = normalize
-        self.log_space = bool(log_space)           # the final tables hold logarithms (several tables, LSE epilogue per row)
-        self.stats = stats
-        self.handle = None
-        cards = tables_owner.cards
-        slot = {v: i for i, v in enumerate(self.evidence)}
-        arr = (N.GatherTable * len(finals))()
-        for k, f in enumerate(finals):
-            has_t = bool(f.scope) and f.scope[-1] == target
-            ev_scope = f.scope[:-1] if has_t else f.scope
-            g = arr[k]
-            g.data = f.tensor.data_ptr()
-            g.n_cells = f.tensor.numel()
-            g.n_ev = len(ev_scope)
-            g.has_target = 1 if has_t else 0
-            stride = card_t if has_t else 1
-            for j in range(len(ev_scope) - 1, -1, -1):
-                g.ev_slot[j] = slot[ev_scope[j]]
-                g.ev_stride[j] = stride
-                stride *= cards[ev_scope[j]]
-        ev_cards = (C.c_int32 * max(len(self.evidence), 1))(*[cards[v] for v in self.evidence])
-        h = C.c_void_p()
-        N.check(N.lib().cbn_ve_plan_create_gather(self.ctx.handle, len(self.evidence), ev_cards, card_t, arr, len(finals),
-                                                  (N.GATHER_NORMALIZE if normalize else 0) | (N.GATHER_LOG_SPACE if log_space else 0),
-                                                  N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
-        self.handle = h
 
     def __del__(self):
         try:
             if self.handle is not None:
-                N.lib().cbn_ve_plan_destroy(self.handle)
+                getattr(N.lib(), self._destroy)(self.handle)
                 self.handle = None
         except Exception:
             pass
 
+
+class _VEPlan(_NativePlan):
+    """What gather plans and per-row plans share: a ``cbn_ve_plan`` that answers ``target`` (None: ``log P(e)``) from the
+    codes of ``evidence`` (row e of a code matrix = evidence variable e of the plan)."""
+
+    def __init__(self, tables_owner, target: Optional[int], evidence: List[int], card_t: int, stats: PlanStats,
+                 log_space: bool):
+        super().__init__(tables_owner)
+        self.target = target
+        self.evidence = list(evidence)
+        self.card_t = card_t
+        self.stats = stats
+        self.log_space = bool(log_space)           # the tables hold logarithms
+
     # bytes the kernel must move per row (SURVEY.md section 8d): relevant evidence codes in, posterior out
     def algorithmic_bytes_per_row(self) -> int:
         return len(self.stats.relevant_evidence) + 4 * self.card_t
+
+    def set_static_evidence(self, on: bool = True):
+        """Declare that the evidence of this plan's runs is never written by the kernel preceding the run on the same
+        stream (resident batches replayed from a CUDA graph): evidence loads may then overlap the previous launch.  The
+        per-row kernels do not use it."""
+        N.check(N.lib().cbn_ve_plan_set_static_evidence(self.handle, 1 if on else 0), self.ctx.handle)
 
     def run_codes(self, ev_codes: torch.Tensor, n_rows: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """ev_codes: uint8 [len(evidence), ld] on the device (row e = evidence variable e of the plan)."""
         assert ev_codes.dtype == torch.uint8 and ev_codes.is_cuda
         if out is None:
             out = torch.empty((n_rows, self.card_t), dtype=torch.float32, device=self.device)
-        ld = ev_codes.stride(0) if ev_codes.dim() == 2 else 0
-        N.check(N.lib().cbn_ve_run_codes(self.ctx.handle, self.handle, ev_codes.data_ptr(), ld, int(n_rows),
+        N.check(N.lib().cbn_ve_run_codes(self.ctx.handle, self.handle, ev_codes.data_ptr(), _ld(ev_codes), int(n_rows),
                                          out.data_ptr(), N.stream_ptr(self.device)), self.ctx.handle)
         return out
 
-    def set_static_evidence(self, on: bool = True):
-        """Declare that the evidence of this plan's runs is never written by the kernel preceding the run on the same
-        stream (resident batches replayed from a CUDA graph): evidence loads may then overlap the previous launch."""
-        N.check(N.lib().cbn_ve_plan_set_static_evidence(self.handle, 1 if on else 0), self.ctx.handle)
+    def run_codes_log_evidence(self, ev_codes: torch.Tensor, n_rows: int, out: torch.Tensor) -> torch.Tensor:
+        """Float32 [n_rows]: the log of the sum over the plan's tables for each row (``log P(e_row)`` for a plan of
+        ``VECompiler.compile_evidence``)."""
+        N.check(N.lib().cbn_ve_run_codes_log_evidence(self.ctx.handle, self.handle, ev_codes.data_ptr(), _ld(ev_codes),
+                                                      int(n_rows), out.data_ptr(), N.stream_ptr(self.device)),
+                self.ctx.handle)
+        return out
 
-    def _encode_evidence(self, ev_cols: Sequence[torch.Tensor], n_rows: int) -> torch.Tensor:
-        ld = (max(n_rows, 1) + 15) // 16 * 16
-        codes = torch.empty((max(len(self.evidence), 1), ld), dtype=torch.uint8, device=self.device)
-        for e, (v, col) in enumerate(zip(self.evidence, ev_cols)):
-            self.owner.encode(col, v, codes[e])
-        return codes
+    def run_f32(self, ev_cols: Sequence[torch.Tensor], n_rows: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Float evidence columns: encoded on the device first (unseen values -> CBN_UNSEEN -> zero rows)."""
+        return self.run_codes(self.owner.encode_evidence(self.evidence, ev_cols, n_rows), n_rows, out)
+
+
+class QueryPlan(_VEPlan):
+    """A compiled (target, evidence-set) query.  Owns the final tables and the native plan."""
+
+    def __init__(self, tables_owner, target: int, evidence: List[int], card_t: int, finals: List[Factor],
+                 normalize: bool, stats: PlanStats, log_space: bool = False):
+        super().__init__(tables_owner, target, evidence, card_t, stats, log_space)
+        self.finals = finals
+        self.normalize = normalize
+        cards = tables_owner.cards
+        slot = {v: i for i, v in enumerate(self.evidence)}
+        arr = (N.GatherTable * len(finals))()
+        for k, f in enumerate(finals):
+            has_t = bool(f.scope) and f.scope[-1] == target
+            ev_scope = f.scope[:-1] if has_t else f.scope
+            stride = _strides(f.scope, cards)
+            g = arr[k]
+            g.data = f.tensor.data_ptr()
+            g.n_cells = f.tensor.numel()
+            g.n_ev = len(ev_scope)
+            g.has_target = 1 if has_t else 0
+            for j, v in enumerate(ev_scope):
+                g.ev_slot[j] = slot[v]
+                g.ev_stride[j] = stride[v]
+        h = C.c_void_p()
+        N.check(N.lib().cbn_ve_plan_create_gather(self.ctx.handle, len(self.evidence), _int32s([cards[v] for v in self.evidence]),
+                                                  card_t, arr, len(finals),
+                                                  (N.GATHER_NORMALIZE if normalize else 0) | (N.GATHER_LOG_SPACE if log_space else 0),
+                                                  N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
+        self.handle = h
 
     def run_f32(self, ev_cols: Sequence[torch.Tensor], n_rows: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """ev_cols[e]: float32 device column of evidence variable e (the reference's [nq,1] tensors)."""
         if self.card_t > N.GATHER_MAX_CT or len(self.evidence) > N.MAX_EVIDENCE_PTRS:
             # wide targets / very many evidence columns: the float kernel keeps the posterior in registers and takes its
             # column pointers as kernel arguments; encode on the device and use the code kernels (any cardinality)
-            return self.run_codes(self._encode_evidence(ev_cols, n_rows), n_rows, out)
+            return super().run_f32(ev_cols, n_rows, out)
         if out is None:
             out = torch.empty((n_rows, self.card_t), dtype=torch.float32, device=self.device)
         cols = N.ptr_array([c.data_ptr() for c in ev_cols])
@@ -166,8 +198,7 @@ class QueryPlan:
     def run_codes_map(self, ev_codes: torch.Tensor, n_rows: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         if out is None:
             out = torch.empty(n_rows, dtype=torch.float32, device=self.device)
-        ld = ev_codes.stride(0) if ev_codes.dim() == 2 else 0
-        N.check(N.lib().cbn_ve_run_codes_map(self.ctx.handle, self.handle, ev_codes.data_ptr(), ld, int(n_rows),
+        N.check(N.lib().cbn_ve_run_codes_map(self.ctx.handle, self.handle, ev_codes.data_ptr(), _ld(ev_codes), int(n_rows),
                                              self.owner.domains[self.target].data_ptr(), out.data_ptr(), N.stream_ptr(self.device)),
                 self.ctx.handle)
         return out
@@ -190,29 +221,20 @@ class QueryPlan:
         return out_host
 
 
-class FusedPlan:
+class FusedPlan(_NativePlan):
     """Several targets over the same evidence list answered by ONE launch: the evidence codes are read once
     and every target's posterior is written (``cbn_ve_plan_fuse`` / ``cbn_ve_run_codes_multi``)."""
 
     def __init__(self, plans: Sequence[QueryPlan]):
         assert len(plans) >= 1
+        super().__init__(plans[0].owner)
         self.plans = list(plans)            # keep the tables alive
-        self.ctx = plans[0].ctx
-        self.device = plans[0].device
         self.card_t = plans[0].card_t
         arr = N.ptr_array([p.handle.value for p in plans])
         h = C.c_void_p()
         N.check(N.lib().cbn_ve_plan_fuse(self.ctx.handle, arr, len(plans), N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
         self.handle = h
         self.n_out = N.lib().cbn_ve_plan_outputs(h)
-
-    def __del__(self):
-        try:
-            if self.handle is not None:
-                N.lib().cbn_ve_plan_destroy(self.handle)
-                self.handle = None
-        except Exception:
-            pass
 
     def set_static_evidence(self, on: bool = True):
         N.check(N.lib().cbn_ve_plan_set_static_evidence(self.handle, 1 if on else 0), self.ctx.handle)
@@ -228,22 +250,20 @@ class FusedPlan:
             outs = [torch.empty((n_rows, self.card_t), dtype=torch.float32, device=self.device) for _ in range(self.n_out)]
         assert len(outs) == self.n_out
         ptrs = N.ptr_array([o.data_ptr() for o in outs])
-        ld = ev_codes.stride(0) if ev_codes.dim() == 2 else 0
-        N.check(N.lib().cbn_ve_run_codes_multi(self.ctx.handle, self.handle, ev_codes.data_ptr(), ld, int(n_rows), ptrs,
-                                               N.stream_ptr(self.device)), self.ctx.handle)
+        N.check(N.lib().cbn_ve_run_codes_multi(self.ctx.handle, self.handle, ev_codes.data_ptr(), _ld(ev_codes), int(n_rows),
+                                               ptrs, N.stream_ptr(self.device)), self.ctx.handle)
         return list(outs)
 
-
-def _fused_run_codes_host(self, ev_codes_host: torch.Tensor, n_rows: int, outs_host: Sequence[torch.Tensor], compact: bool = False):
-    """Host buffers in, host buffers out, one fused launch per chunk (copies inside; synchronous).  ``compact``: the
-    outputs are float32 [n_rows, card_t - 1] (``CBN_HOST_OUT_DROP_LAST``; ``expand_compact`` restores the full rows)."""
-    assert not ev_codes_host.is_cuda and len(outs_host) == self.n_out and all(not o.is_cuda for o in outs_host)
-    width = self.card_t - 1 if compact else self.card_t
-    assert all(o.is_contiguous() and o.shape[-1] == width and o.shape[0] >= n_rows for o in outs_host)
-    ptrs = N.ptr_array([o.data_ptr() for o in outs_host])
-    N.check(N.lib().cbn_ve_run_codes_host_multi_ex(self.ctx.handle, self.handle, ev_codes_host.data_ptr(), ev_codes_host.stride(0),
-                                                   int(n_rows), ptrs, N.HOST_OUT_DROP_LAST if compact else 0), self.ctx.handle)
-    return list(outs_host)
+    def run_codes_host(self, ev_codes_host: torch.Tensor, n_rows: int, outs_host: Sequence[torch.Tensor], compact: bool = False):
+        """Host buffers in, host buffers out, one fused launch per chunk (copies inside; synchronous).  ``compact``: the
+        outputs are float32 [n_rows, card_t - 1] (``CBN_HOST_OUT_DROP_LAST``; ``expand_compact`` restores the full rows)."""
+        assert not ev_codes_host.is_cuda and len(outs_host) == self.n_out and all(not o.is_cuda for o in outs_host)
+        width = self.card_t - 1 if compact else self.card_t
+        assert all(o.is_contiguous() and o.shape[-1] == width and o.shape[0] >= n_rows for o in outs_host)
+        ptrs = N.ptr_array([o.data_ptr() for o in outs_host])
+        N.check(N.lib().cbn_ve_run_codes_host_multi_ex(self.ctx.handle, self.handle, ev_codes_host.data_ptr(), ev_codes_host.stride(0),
+                                                       int(n_rows), ptrs, N.HOST_OUT_DROP_LAST if compact else 0), self.ctx.handle)
+        return list(outs_host)
 
 
 def expand_compact(compact: torch.Tensor) -> torch.Tensor:
@@ -255,39 +275,23 @@ def expand_compact(compact: torch.Tensor) -> torch.Tensor:
     return full
 
 
-FusedPlan.run_codes_host = _fused_run_codes_host
-
-
-class RowPlan:
+class RowPlan(_VEPlan):
     """A query whose evidence boundary is too large to tabulate: static tables for what could be eliminated at
     compile time + a per-row schedule of product / sum-out steps (``cbn_ve_plan_create_rows``)."""
 
     def __init__(self, tables_owner, target: int, evidence: List[int], card_t: int, inputs: List[Factor],
                  steps: List[dict], offsets, stats: PlanStats, log_space: bool):
-        self.owner = tables_owner
-        self.ctx = tables_owner.ctx
-        self.device = tables_owner.device
-        self.target = target
-        self.evidence = list(evidence)
-        self.card_t = card_t
+        super().__init__(tables_owner, target, evidence, card_t, stats, log_space)
         self.inputs = inputs            # keep the tables alive
         self.offsets = offsets          # host int32 array (numpy): copied into the plan at creation
-        self.stats = stats
-        self.log_space = log_space
-        self.handle = None
         cards = tables_owner.cards
         slot = {v: i for i, v in enumerate(self.evidence)}
-        Eset = set(self.evidence)
         ins = (N.RowInput * len(inputs))()
         for k, f in enumerate(inputs):
+            stride = _strides(f.scope, cards)
+            ev_axes = [(slot[v], stride[v]) for v in reversed(f.scope) if v in slot]
             ins[k].data = f.tensor.data_ptr()
             ins[k].n_cells = f.tensor.numel()
-            stride, j = 1, 0
-            ev_axes = []
-            for v in reversed(f.scope):
-                if v in Eset:
-                    ev_axes.append((slot[v], stride))
-                stride *= cards[v]
             ins[k].n_ev = len(ev_axes)
             for j, (sl, st) in enumerate(ev_axes):
                 ins[k].ev_slot[j] = sl
@@ -301,40 +305,11 @@ class RowPlan:
                 sts[j].in_id[k] = i
                 sts[j].sum_stride[k] = ss
             sts[j].offsets = offsets.ctypes.data + 4 * st["offsets_at"]
-        ev_cards = (C.c_int32 * max(len(self.evidence), 1))(*[cards[v] for v in self.evidence])
         h = C.c_void_p()
-        N.check(N.lib().cbn_ve_plan_create_rows(self.ctx.handle, len(self.evidence), ev_cards, card_t, ins, len(inputs), sts,
-                                                len(steps), N.ROWS_LOG_SPACE if log_space else 0, N.stream_ptr(self.device),
-                                                C.byref(h)), self.ctx.handle)
+        N.check(N.lib().cbn_ve_plan_create_rows(self.ctx.handle, len(self.evidence), _int32s([cards[v] for v in self.evidence]),
+                                                card_t, ins, len(inputs), sts, len(steps), N.ROWS_LOG_SPACE if log_space else 0,
+                                                N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
         self.handle = h
-
-    def __del__(self):
-        try:
-            if self.handle is not None:
-                N.lib().cbn_ve_plan_destroy(self.handle)
-                self.handle = None
-        except Exception:
-            pass
-
-    def algorithmic_bytes_per_row(self) -> int:
-        return len(self.stats.relevant_evidence) + 4 * self.card_t
-
-    def run_codes(self, ev_codes: torch.Tensor, n_rows: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        assert ev_codes.dtype == torch.uint8 and ev_codes.is_cuda
-        if out is None:
-            out = torch.empty((n_rows, self.card_t), dtype=torch.float32, device=self.device)
-        ld = ev_codes.stride(0) if ev_codes.dim() == 2 else 0
-        N.check(N.lib().cbn_ve_run_codes(self.ctx.handle, self.handle, ev_codes.data_ptr(), ld, int(n_rows),
-                                         out.data_ptr(), N.stream_ptr(self.device)), self.ctx.handle)
-        return out
-
-    def run_f32(self, ev_cols: Sequence[torch.Tensor], n_rows: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Float evidence columns: encoded on the device first (unseen values -> CBN_UNSEEN -> zero rows)."""
-        ld = (max(n_rows, 1) + 15) // 16 * 16
-        codes = torch.empty((max(len(self.evidence), 1), ld), dtype=torch.uint8, device=self.device)
-        for e, (v, col) in enumerate(zip(self.evidence, ev_cols)):
-            self.owner.encode(col, v, codes[e])
-        return self.run_codes(codes, n_rows, out)
 
 
 @dataclass
@@ -347,14 +322,13 @@ class EvidenceSplit:
     per_row: bool = False
 
 
-class LogLikPlan:
+class LogLikPlan(_NativePlan):
     """Owner of a ``cbn_loglik_plan``: ``out[row] (+)= sum_f log cond_f[index_f(row)]`` over families whose variables are
     all columns of the code matrix handed to ``run`` (``columns[v]``: the column of network variable v)."""
+    _destroy = "cbn_loglik_plan_destroy"
 
     def __init__(self, tables_owner, families: Sequence[int], columns: Dict[int, int], n_cols: int):
-        self.ctx = tables_owner.ctx
-        self.device = tables_owner.device
-        self.handle = None
+        super().__init__(tables_owner)
         t = tables_owner
         fams = (N.Family * max(len(families), 1))()
         for i, v in enumerate(families):
@@ -366,14 +340,6 @@ class LogLikPlan:
                                                N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
         self.handle = h
         self.lookups_per_row = N.lib().cbn_loglik_plan_tables(h)
-
-    def __del__(self):
-        try:
-            if self.handle is not None:
-                N.lib().cbn_loglik_plan_destroy(self.handle)
-                self.handle = None
-        except Exception:
-            pass
 
     def run(self, codes: torch.Tensor, n_rows: int, out: torch.Tensor, accumulate: bool = False) -> torch.Tensor:
         assert codes.dtype == torch.uint8 and codes.is_cuda and out.dtype == torch.float32
@@ -412,15 +378,10 @@ class EvidencePlan:
             out = torch.empty(n_rows, dtype=torch.float32, device=self.device)
         if n_rows == 0:
             return out
-        accumulate = False
         if self.ve_plan is not None:
-            ld = ev_codes.stride(0) if ev_codes.dim() == 2 else 0
-            N.check(N.lib().cbn_ve_run_codes_log_evidence(self.ctx.handle, self.ve_plan.handle, ev_codes.data_ptr(), ld,
-                                                          int(n_rows), out.data_ptr(), N.stream_ptr(self.device)),
-                    self.ctx.handle)
-            accumulate = True
+            self.ve_plan.run_codes_log_evidence(ev_codes, n_rows, out)
         if self.loglik is not None:
-            self.loglik.run(ev_codes, n_rows, out, accumulate=accumulate)
+            self.loglik.run(ev_codes, n_rows, out, accumulate=self.ve_plan is not None)
         elif self.ve_plan is None:          # no evidence: log 1
             out.zero_()
         return out
@@ -437,20 +398,18 @@ class MPESplit:
     stats: PlanStats
 
 
-class MPEPlan:
+class MPEPlan(_NativePlan):
     """A compiled most probable explanation: the argmax tables of the max-sum elimination, the native traceback plan
     (``cbn_mpe_plan_create``) and the ``EvidencePlan`` that computes each row's value ``log max_h P(h, e)``."""
+    _destroy = "cbn_mpe_plan_destroy"
 
     def __init__(self, tables_owner, split: MPESplit, decode, value: EvidencePlan):
-        self.owner = tables_owner
-        self.ctx = tables_owner.ctx
-        self.device = tables_owner.device
+        super().__init__(tables_owner)
         self.split = split
         self.evidence = list(split.evidence)
         self.hidden = list(split.hidden)
         self.value = value
         self.argmax = [am for _, _, am in decode]           # referenced by the native plan: kept alive with it
-        self.handle = None
         cards = tables_owner.cards
         n_ev = len(self.evidence)
         slot = {v: i for i, v in enumerate(self.evidence)}
@@ -465,24 +424,14 @@ class MPEPlan:
             st.argmax = am.data_ptr()
             st.n_cells = am.numel()
             st.n_ctx = len(scope)
-            stride = 1
-            for j in range(len(scope) - 1, -1, -1):
-                st.ctx_slot[j] = slot[scope[j]]
-                st.ctx_stride[j] = stride
-                stride *= cards[scope[j]]
-        ev_cards = (C.c_int32 * max(n_ev, 1))(*[cards[v] for v in self.evidence])
+            stride = _strides(scope, cards)
+            for j, u in enumerate(scope):
+                st.ctx_slot[j] = slot[u]
+                st.ctx_stride[j] = stride[u]
         h = C.c_void_p()
-        N.check(N.lib().cbn_mpe_plan_create(self.ctx.handle, n_ev, ev_cards, len(self.hidden), steps, len(decode),
-                                            N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
+        N.check(N.lib().cbn_mpe_plan_create(self.ctx.handle, n_ev, _int32s([cards[v] for v in self.evidence]), len(self.hidden),
+                                            steps, len(decode), N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
         self.handle = h
-
-    def __del__(self):
-        try:
-            if self.handle is not None:
-                N.lib().cbn_mpe_plan_destroy(self.handle)
-                self.handle = None
-        except Exception:
-            pass
 
     def set_static_evidence(self, on: bool = True):
         self.value.set_static_evidence(on)
@@ -495,12 +444,10 @@ class MPEPlan:
         assert ev_codes.dtype == torch.uint8 and ev_codes.is_cuda
         value = self.value.run_codes(ev_codes, n_rows, value_out)
         if hidden_out is None:
-            ld = (max(n_rows, 1) + 15) // 16 * 16
-            hidden_out = torch.empty((len(self.hidden), ld), dtype=torch.uint8, device=self.device)
+            hidden_out = self.owner.new_code_matrix(n_rows, len(self.hidden))
         if self.handle is not None and n_rows > 0:
-            ld = ev_codes.stride(0) if ev_codes.dim() == 2 else 0
-            N.check(N.lib().cbn_mpe_run(self.ctx.handle, self.handle, ev_codes.data_ptr(), ld, int(n_rows), value.data_ptr(),
-                                        hidden_out.data_ptr(), hidden_out.stride(0), N.stream_ptr(self.device)),
+            N.check(N.lib().cbn_mpe_run(self.ctx.handle, self.handle, ev_codes.data_ptr(), _ld(ev_codes), int(n_rows),
+                                        value.data_ptr(), hidden_out.data_ptr(), hidden_out.stride(0), N.stream_ptr(self.device)),
                     self.ctx.handle)
         return hidden_out, value
 
@@ -569,6 +516,37 @@ class _Greedy:
         self.add(new_key, new_scope)
 
 
+@dataclass
+class _Pass:
+    """One pass of a compile: the arithmetic of its contractions and the state that lives only as long as the pass.
+
+    ``log_space``: the factors hold logarithms (log-sum-exp or max-sum contractions).  ``rescale``: range control of
+    linear-space elimination -- after every contraction each evidence slice of the result is divided by its maximum
+    (``cbn_factor_rescale``), a factor of the evidence configuration only, which cancels in the final normalisation, so
+    products of many small likelihoods stay inside the fp32 range.  ``dry``: structure only, no device work."""
+    E: List[int]                                        # evidence ids, in plan order
+    T: Optional[int]                                    # the target (None: log P(e) and MPE)
+    dry: bool
+    log_space: bool
+    rescale: bool
+    stats: PlanStats = field(default_factory=PlanStats)
+    events: list = field(default_factory=list)          # CUDA events around every contraction (profile_compile)
+
+    def __post_init__(self):
+        self.ev = set(self.E)
+        self._order = {v: i for i, v in enumerate(self.E)}
+
+    def sort_scope(self, scope) -> List[int]:
+        # evidence axes (plan order) first, then hidden, target last (fastest)
+        return sorted(set(scope), key=lambda v: (2 if v == self.T else (0 if v in self.ev else 1), self._order.get(v, v)))
+
+    def device_ms(self) -> float:
+        if not self.events:
+            return 0.0
+        self.events[-1][1].synchronize()
+        return sum(a.elapsed_time(b) for a, b in self.events)
+
+
 class VECompiler:
     """Lower (target, evidence set) to a gather plan over a fitted ``DiscreteTables``."""
 
@@ -576,27 +554,29 @@ class VECompiler:
                  check_support: bool = True, row_temp_floats: int = 5000, log_space: bool = False, rescale: bool = True,
                  profile_compile: bool = False, row_unit_layout: bool = True, mpe_argmax_budget_bytes: int = 1 << 30):
         self.t = tables
-        # range control of the compile-time elimination: after every contraction each evidence slice of the result is
-        # divided by its maximum (cbn_factor_rescale) -- a factor of the evidence configuration only, which cancels in the
-        # final normalisation -- so products of many small likelihoods stay inside the fp32 range
+        self.log_space = bool(log_space)                 # arithmetic of posterior compiles (see _Pass)
         self.rescale = bool(rescale)
         self.profile_compile = bool(profile_compile)      # CUDA events around every contraction -> PlanStats.contraction_gpu_ms
-        self._ev_set: set = set()
-        self._events: list = []
         self.table_budget = int(table_budget_cells)
         self.merge_budget = int(merge_budget_cells)
         self.check_support = check_support
         self.row_temp_floats = int(row_temp_floats)     # per-row temporaries of the per-row executor (shared memory)
         self.row_unit_layout = bool(row_unit_layout)    # lay every per-row factor out with its consumer's summed variable innermost
-        self.log_space = bool(log_space)
-        self._cache: Dict[tuple, QueryPlan] = {}
+        self.mpe_argmax_budget = int(mpe_argmax_budget_bytes)    # argmax tables of one MPE plan, in bytes
+        self._plans: Dict[tuple, object] = {}           # (mode, key) -> plan
+        self._plans_version = None
         self._has_zero: Dict[int, bool] = {}
         self.last_row_schedule: Optional[dict] = None
-        self._ev_child: Optional["VECompiler"] = None       # the evidence-mode compiler (log space, no range control)
-        self._ev_cache: Dict[tuple, "EvidencePlan"] = {}
-        self._ev_cache_version = None
-        self.mpe_argmax_budget = int(mpe_argmax_budget_bytes)    # argmax tables of one MPE plan, in bytes
-        self._mpe_cache: Dict[tuple, "MPEPlan"] = {}
+
+    def cached(self, key: tuple, build):
+        """The plan stored under ``key``, built by ``build()`` when missing.  Every plan and the zero-entry memo derive from
+        the CPTs: all are dropped together when the tables' ``cond_version`` changes."""
+        version = getattr(self.t, "cond_version", 0)
+        if self._plans_version != version:
+            self._plans, self._has_zero, self._plans_version = {}, {}, version
+        if key not in self._plans:
+            self._plans[key] = build()
+        return self._plans[key]
 
     # ---------------------------------------------------------------- graph helpers
     def _parents(self, v: int) -> List[int]:
@@ -620,13 +600,23 @@ class VECompiler:
             self._has_zero[v] = bool((view == 0).any().item())
         return self._has_zero[v]
 
+    def _evidence_ids(self, evidence_names: Sequence[str]) -> List[int]:
+        t = self.t
+        for e in evidence_names:
+            if e not in t.index:
+                raise ValueError(f"{e} is not a node of the network")
+        E = [t.index[e] for e in evidence_names]
+        if len(set(E)) != len(E):
+            raise ValueError("an evidence variable is listed twice")
+        return E
+
     # ---------------------------------------------------------------- device contraction
-    def _contract(self, inputs: List[Factor], out_scope: List[int], sum_var: Optional[int], dry: bool,
+    def _contract(self, inputs: List[Factor], out_scope: List[int], sum_var: Optional[int], cx: _Pass,
                   normalize_last: bool = False, argmax: Optional[torch.Tensor] = None) -> Factor:
         """``argmax``: uint8 device buffer of the output's size -- maximise over ``sum_var`` instead of summing
         (``cbn_factor_contract_max``, log space) and record the maximising value of every output cell there."""
         cards = self.t.cards
-        if dry:
+        if cx.dry:
             return Factor(out_scope, None)
         if len(out_scope) > N.MAX_CONTRACT_DIMS:
             raise PlanTooLarge(f"factor with {len(out_scope)} axes exceeds {N.MAX_CONTRACT_DIMS}")
@@ -637,22 +627,16 @@ class VECompiler:
         d.sum_card = cards[sum_var] if sum_var is not None else 1
         d.n_in = len(inputs)
         for k, f in enumerate(inputs):
-            strides = {}
-            s = 1
-            for v in reversed(f.scope):
-                strides[v] = s
-                s *= cards[v]
+            strides = _strides(f.scope, cards)
             d.inp[k] = f.tensor.data_ptr()
             for a, v in enumerate(out_scope):
                 d.in_stride[k][a] = strides.get(v, 0)
             d.sum_stride[k] = strides.get(sum_var, 0) if sum_var is not None else 0
-        n_out = 1
-        for v in out_scope:
-            n_out *= cards[v]
+        n_out = _cells(out_scope, cards)
         out = torch.empty(max(n_out, 1), dtype=torch.float32, device=self.t.device)
         d.out = out.data_ptr()
         d.normalize_last = 1 if normalize_last else 0
-        d.log_space = 1 if self.log_space else 0
+        d.log_space = 1 if cx.log_space else 0
         if self.profile_compile:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
@@ -661,29 +645,87 @@ class VECompiler:
                     self.t.ctx.handle)
         else:
             N.check(N.lib().cbn_factor_contract(self.t.ctx.handle, C.byref(d), N.stream_ptr(self.t.device)), self.t.ctx.handle)
-        if self.rescale and not normalize_last:
+        if cx.rescale and not normalize_last:
             # evidence axes are the slowest axes of every factor (sort_scope): one contiguous slice per evidence configuration
             lead = 0
-            while lead < len(out_scope) and out_scope[lead] in self._ev_set:
+            while lead < len(out_scope) and out_scope[lead] in cx.ev:
                 lead += 1
-            n_slices = 1
-            for v in out_scope[:lead]:
-                n_slices *= cards[v]
+            n_slices = _cells(out_scope[:lead], cards)
             slice_size = max(n_out, 1) // max(n_slices, 1)
-            if all(v not in self._ev_set for v in out_scope[lead:]):
+            if all(v not in cx.ev for v in out_scope[lead:]):
                 N.check(N.lib().cbn_factor_rescale(self.t.ctx.handle, out.data_ptr(), n_slices, slice_size,
-                                                   1 if self.log_space else 0, N.stream_ptr(self.t.device)), self.t.ctx.handle)
+                                                   1 if cx.log_space else 0, N.stream_ptr(self.t.device)), self.t.ctx.handle)
         if self.profile_compile:
             e1.record()
-            self._events.append((e0, e1))
+            cx.events.append((e0, e1))
         return Factor(out_scope, out)
 
-    # ---------------------------------------------------------------- compile
+    # ---------------------------------------------------------------- compile front end
+    def _compile(self, mode: str, key: tuple, E: List[int], T: Optional[int], dry: bool, build,
+                 log_space: bool = True, rescale: bool = False):
+        """Run ``build(pass)`` -- the part of the compile that is the mode's own -- as a structure-only pass (``dry``), or
+        return the cached plan of ``(mode, key)``.  A plan is compiled after a structure-only pass: a query that does not
+        fit fails there, before any table is contracted.  The default arithmetic is that of ``log P(e)`` and MPE: log space
+        without range control."""
+        if dry:
+            return build(_Pass(E, T, True, log_space, rescale))
+
+        def compile_plan():
+            build(_Pass(E, T, True, log_space, rescale))
+            cx = _Pass(E, T, False, log_space, rescale)
+            plan = build(cx)
+            cx.stats.contraction_gpu_ms = cx.device_ms()
+            return plan
+
+        return self.cached((mode, key), compile_plan)
+
+    def _factors(self, cx: _Pass, owners, split_observed: bool):
+        """The CPTs of ``owners`` as factors (their logarithms in log space) and, with ``split_observed``, apart from them
+        the owners whose whole family is evidence: constants of the row, summed by the observed-families kernel."""
+        t = self.t
+        src = None if cx.dry else (t.log_cond if cx.log_space else t.cond)
+        factors, observed = [], []
+        for v in owners:
+            scope = t.family_vars(t.names[v])
+            if split_observed and all(u in cx.ev for u in scope):
+                observed.append(v)
+            else:
+                factors.append(Factor(list(scope), None if src is None else t.table_view(src, t.names[v]).reshape(-1)))
+        return factors, observed
+
+    def _tail(self, cx: _Pass, finals: List[Factor], left: List[int]):
+        """The plan over what the compile-time elimination leaves: a per-row plan when hidden variables are ``left``, else a
+        gather over the merged final tables.  Fills the statistics of either; returns None in a dry pass."""
+        cards, stats = self.t.cards, cx.stats
+        if left:
+            # the boundary is too large to tabulate: the rest of the hidden variables is eliminated per row
+            stats.per_row_hidden = len(left)
+            stats.final_tables = [(tuple(f.scope), _cells(f.scope, cards)) for f in finals]
+            stats.per_row_slice_cells = sum(_cells(f.scope, cards) // _cells([v for v in f.scope if v in cx.ev], cards)
+                                            for f in finals)
+            return self._row_plan(cx, finals, left)
+        finals = self._merge_finals(cx, finals)
+        stats.final_tables = [(tuple(f.scope), _cells(f.scope, cards)) for f in finals]
+        if cx.dry:
+            return None
+        T, normalize, log_tables = cx.T, True, cx.log_space
+        if T is not None:
+            with_t = [f for f in finals if f.scope and f.scope[-1] == T]
+            if not with_t:
+                # target independent of everything kept (cannot happen: P(T|pa) always mentions T)
+                raise RuntimeError("internal: no final factor mentions the target")
+            if len(finals) == 1:
+                # a single pre-normalised target table needs no arithmetic per row (in log space the normalising
+                # contraction returns the LINEAR distribution: the plan is an ordinary gather)
+                finals = [self._contract(finals, finals[0].scope, None, cx, normalize_last=True)]
+                normalize, log_tables = False, False
+        return QueryPlan(self.t, T, cx.E, cards[T] if T is not None else 1, finals, normalize, stats, log_space=log_tables)
+
+    # ---------------------------------------------------------------- posterior: P(T | e)
     def compile(self, target: str, evidence: Sequence[str], do: Sequence[str] = (), dry: bool = False):
         """``do``: evidence variables that are set by intervention (graph surgery: their own CPT is dropped
         and their parents are cut off) -- the reference's ``infer(do=...)`` is a TODO (bayesian_network.py:229-232)."""
         t = self.t
-        cards = t.cards
         T = t.index[target]
         E = [t.index[e] for e in evidence if e != target]      # evidence on the target itself is not forwarded
         D = set()                                               # (bayesian_network.py:190-196)
@@ -693,34 +735,14 @@ class VECompiler:
             if d == target:
                 raise ValueError("cannot intervene on the target node")
             D.add(t.index[d])
-        key = (T, tuple(E), tuple(sorted(D)))
-        if not dry and key in self._cache:
-            return self._cache[key]
-        if not dry:
-            # structure-only pass first: a query that does not fit fails here, before any table is contracted
-            self.compile(target, evidence, do=do, dry=True)
-        Eset = set(E)
-        self._ev_set = Eset
-        if not dry:
-            self._events = []
-        order_key = {v: i for i, v in enumerate(E)}
-        stats = PlanStats()
+        return self._compile("posterior", (T, tuple(E), tuple(sorted(D))), E, T, dry, lambda cx: self._posterior(cx, D),
+                             log_space=self.log_space, rescale=self.rescale)
 
-        def sort_scope(scope) -> List[int]:
-            # evidence axes (plan order) first, then hidden, target last (fastest)
-            return sorted(set(scope), key=lambda v: (2 if v == T else (0 if v in Eset else 1), order_key.get(v, v)))
-
-        relevant = self._ancestors([T] + E, cut=D)
+    def _posterior(self, cx: _Pass, D: set):
+        T, Eset, stats = cx.T, cx.ev, cx.stats
+        relevant = self._ancestors([T] + cx.E, cut=D)
         stats.n_relevant = len(relevant)
-        factors: List[Factor] = []
-        for v in sorted(relevant):
-            if v in D:
-                continue
-            scope = t.family_vars(t.names[v])
-            tensor = None if dry else t.table_view(t.cond, t.names[v]).reshape(-1)
-            if tensor is not None and self.log_space:
-                tensor = torch.log(tensor)          # log 0 = -inf: a zero-probability entry stays one through sums and LSE
-            factors.append(Factor(list(scope), tensor))
+        factors, _ = self._factors(cx, sorted(relevant - D), split_observed=False)
         hidden = [v for v in relevant if v not in Eset and v != T]
         stats.n_hidden = len(hidden)
 
@@ -744,14 +766,14 @@ class VECompiler:
         rel_ev = set()
         for f in main:
             rel_ev |= {v for v in f.scope if v in Eset}
-        stats.relevant_evidence = [v for v in E if v in rel_ev]
+        stats.relevant_evidence = [v for v in cx.E if v in rel_ev]
 
-        finals, left = self._eliminate(main, [v for v in hidden if find(v) == comp_t], sort_scope, stats, dry, T, partial=True)
+        finals, left = self._eliminate(cx, main, [v for v in hidden if find(v) == comp_t], partial=True)
 
         # support of the dropped part: a row whose (irrelevant) evidence has probability zero is all zeros in
         # the oracle's convention; only factors that can be zero matter
         if self.check_support and rest:
-            if dry:
+            if cx.dry:
                 stats.support_unchecked = True
             else:
                 groups: Dict[int, List[Factor]] = {}
@@ -763,52 +785,23 @@ class VECompiler:
                 for f in consts:
                     v = f.scope[-1]
                     if self._cond_has_zero(v):
-                        finals.append(self._contract([f], sort_scope(f.scope), None, dry))
+                        finals.append(self._contract([f], cx.sort_scope(f.scope), None, cx))
                 for root, fs in groups.items():
                     owners = [f.scope[-1] for f in fs]
                     if not any(self._cond_has_zero(v) for v in owners):
                         continue
                     try:
-                        sub = PlanStats()
-                        res = self._eliminate(fs, [v for v in hidden if find(v) == root], sort_scope, sub, dry, T)
-                        stats.contraction_madds += sub.contraction_madds
+                        sub = replace(cx, stats=PlanStats())        # the same pass; only its multiply-adds are counted
+                        res = self._eliminate(sub, fs, [v for v in hidden if find(v) == root])
+                        stats.contraction_madds += sub.stats.contraction_madds
                         for r in res:
-                            if bool((r.tensor == (float("-inf") if self.log_space else 0)).any().item()):
+                            if bool((r.tensor == (float("-inf") if cx.log_space else 0)).any().item()):
                                 finals.append(r)
                     except PlanTooLarge:
                         stats.support_unchecked = True
 
-        if left:
-            # the boundary is too large to tabulate: the rest of the hidden variables is eliminated per row
-            stats.per_row_hidden = len(left)
-            stats.final_tables = [(tuple(f.scope), f.size(cards)) for f in finals]
-            stats.per_row_slice_cells = sum(int(f.size(cards) // max(1, _prod(cards[v] for v in f.scope if v in Eset))) for f in finals)
-            plan = self._row_plan(T, E, finals, left, stats, dry)
-            if dry:
-                return stats
-            stats.contraction_gpu_ms = self._drain_events()
-            self._cache[key] = plan
-            return plan
-        finals = self._merge_finals(finals, sort_scope, stats, dry, T)
-        stats.final_tables = [(tuple(f.scope), f.size(cards)) for f in finals]
-        if dry:
-            return stats
-        # a single pre-normalised target table needs no arithmetic per row
-        normalize = True
-        with_t = [f for f in finals if f.scope and f.scope[-1] == T]
-        log_tables = self.log_space
-        if len(finals) == 1 and len(with_t) == 1:
-            # (in log space the normalising contraction returns the LINEAR distribution: the plan is an ordinary gather)
-            finals = [self._contract(finals, finals[0].scope, None, dry, normalize_last=True)]
-            normalize = False
-            log_tables = False
-        if not with_t:
-            # target independent of everything kept (cannot happen: P(T|pa) always mentions T)
-            raise RuntimeError("internal: no final factor mentions the target")
-        stats.contraction_gpu_ms = self._drain_events()
-        plan = QueryPlan(t, T, E, cards[T], finals, normalize, stats, log_space=log_tables)
-        self._cache[key] = plan
-        return plan
+        plan = self._tail(cx, finals, left)
+        return stats if cx.dry else plan
 
     # ---------------------------------------------------------------- evidence mode: log P(e)
     def compile_evidence(self, evidence_names: Sequence[str], dry: bool = False):
@@ -821,97 +814,29 @@ class VECompiler:
         gathered by ``cbn_ve_run_codes_log_evidence``.  When the elimination exceeds the table budget the remaining
         hidden variables go to the per-row executor, as for posteriors.
 
-        The elimination runs in log space WITHOUT range control: log-sum-exp contractions have no range problem in fp32,
-        and dropping the per-slice rescaling is what keeps the normaliser.  The network's posterior plans keep their own
-        configuration and cache; evidence plans are cached separately, keyed by the evidence tuple, and dropped when the
-        tables are re-fitted.
+        The elimination runs in log space WITHOUT range control, whatever the posterior configuration: log-sum-exp
+        contractions have no range problem in fp32, and dropping the per-slice rescaling is what keeps the normaliser.
+        Plans are cached, keyed by the evidence tuple, and dropped when the tables are re-fitted.
 
         ``dry=True`` works on ``DryTables`` and returns the ``EvidenceSplit`` only (no device work)."""
-        if not self.log_space or self.rescale:
-            return self._evidence_child().compile_evidence(evidence_names, dry=dry)
-        t = self.t
-        cards = t.cards
         E = self._evidence_ids(evidence_names)
-        key = tuple(E)
-        if not dry:
-            self._drop_stale_plans()
-            if key in self._ev_cache:
-                return self._ev_cache[key]
-            # structure-only pass first: a query that does not fit fails here, before any table is contracted
-            self.compile_evidence(evidence_names, dry=True)
-            self._events = []
-        Eset = set(E)
-        self._ev_set = Eset
-        order_key = {v: i for i, v in enumerate(E)}
+        return self._compile("evidence", tuple(E), E, None, dry, self._evidence)
 
-        def sort_scope(scope) -> List[int]:
-            # evidence axes (plan order) first, then hidden
-            return sorted(set(scope), key=lambda v: (0 if v in Eset else 1, order_key.get(v, v)))
-
-        stats = PlanStats()
-        relevant = self._ancestors(E)
+    def _evidence(self, cx: _Pass):
+        stats = cx.stats
+        relevant = sorted(self._ancestors(cx.E))
         stats.n_relevant = len(relevant)
-        observed: List[int] = []
-        factors: List[Factor] = []
-        for v in sorted(relevant):
-            scope = t.family_vars(t.names[v])
-            if all(u in Eset for u in scope):
-                observed.append(v)
-                continue
-            tensor = None if dry else t.table_view(t.log_cond, t.names[v]).reshape(-1)
-            factors.append(Factor(list(scope), tensor))
-        hidden = [v for v in sorted(relevant) if v not in Eset]
+        factors, observed = self._factors(cx, relevant, split_observed=True)
+        hidden = [v for v in relevant if v not in cx.ev]
         stats.n_hidden = len(hidden)
-        stats.relevant_evidence = list(E)
-        ve_plan, per_row = None, False
+        stats.relevant_evidence = list(cx.E)
+        ve_plan, left = None, []
         if factors:
-            finals, left = self._eliminate(factors, hidden, sort_scope, stats, dry, None, partial=True)
-            if left:
-                per_row = True
-                stats.per_row_hidden = len(left)
-                stats.final_tables = [(tuple(f.scope), f.size(cards)) for f in finals]
-                stats.per_row_slice_cells = sum(int(f.size(cards) // max(1, _prod(cards[v] for v in f.scope if v in Eset)))
-                                                for f in finals)
-                ve_plan = self._row_plan(None, E, finals, left, stats, dry)
-            else:
-                finals = self._merge_finals(finals, sort_scope, stats, dry, None)
-                stats.final_tables = [(tuple(f.scope), f.size(cards)) for f in finals]
-                if not dry:
-                    ve_plan = QueryPlan(t, None, E, 1, finals, True, stats, log_space=True)
-        split = EvidenceSplit(evidence=list(E), observed_families=observed, ve_stats=stats if factors else None,
-                              per_row=per_row)
-        if dry:
-            return split
-        stats.contraction_gpu_ms = self._drain_events()
-        plan = EvidencePlan(t, E, observed, ve_plan, split)
-        self._ev_cache[key] = plan
-        return plan
-
-    def _evidence_child(self) -> "VECompiler":
-        """The evidence-mode compiler (log space, no range control, no support pruning) over the same tables."""
-        if self._ev_child is None:
-            self._ev_child = VECompiler(self.t, table_budget_cells=self.table_budget, merge_budget_cells=self.merge_budget,
-                                        check_support=False, row_temp_floats=self.row_temp_floats, log_space=True,
-                                        rescale=False, profile_compile=self.profile_compile,
-                                        row_unit_layout=self.row_unit_layout, mpe_argmax_budget_bytes=self.mpe_argmax_budget)
-        return self._ev_child
-
-    def _evidence_ids(self, evidence_names: Sequence[str]) -> List[int]:
-        t = self.t
-        for e in evidence_names:
-            if e not in t.index:
-                raise ValueError(f"{e} is not a node of the network")
-        E = [t.index[e] for e in evidence_names]
-        if len(set(E)) != len(E):
-            raise ValueError("an evidence variable is listed twice")
-        return E
-
-    def _drop_stale_plans(self):
-        version = getattr(self.t, "cond_version", 0)
-        if self._ev_cache_version != version:          # re-fitted tables: every cached plan is stale
-            self._ev_cache = {}
-            self._mpe_cache = {}
-            self._ev_cache_version = version
+            finals, left = self._eliminate(cx, factors, hidden, partial=True)
+            ve_plan = self._tail(cx, finals, left)
+        split = EvidenceSplit(evidence=list(cx.E), observed_families=observed, ve_stats=stats if factors else None,
+                              per_row=bool(left))
+        return split if cx.dry else EvidencePlan(self.t, cx.E, observed, ve_plan, split)
 
     # ---------------------------------------------------------------- MPE mode: argmax_h P(h, e)
     def compile_mpe(self, evidence_names: Sequence[str], dry: bool = False):
@@ -928,99 +853,53 @@ class VECompiler:
         structure-only pass, before any table is contracted.
 
         ``dry=True`` works on ``DryTables`` and returns the ``MPESplit`` only (no device work)."""
-        if not self.log_space or self.rescale:
-            return self._evidence_child().compile_mpe(evidence_names, dry=dry)
-        t = self.t
-        cards = t.cards
         E = self._evidence_ids(evidence_names)
-        key = tuple(E)
-        if not dry:
-            self._drop_stale_plans()
-            if key in self._mpe_cache:
-                return self._mpe_cache[key]
-            self.compile_mpe(evidence_names, dry=True)      # the limits fail here, before any table is contracted
-            self._events = []
-        Eset = set(E)
-        self._ev_set = Eset
-        order_key = {v: i for i, v in enumerate(E)}
+        return self._compile("mpe", tuple(E), E, None, dry, self._mpe)
 
-        def sort_scope(scope) -> List[int]:
-            return sorted(set(scope), key=lambda v: (0 if v in Eset else 1, order_key.get(v, v)))
-
-        stats = PlanStats()
+    def _mpe(self, cx: _Pass):
+        t, cards, stats = self.t, self.t.cards, cx.stats
+        every = range(len(t.names))
         stats.n_relevant = len(t.names)
-        observed: List[int] = []
-        factors: List[Factor] = []
-        for v in range(len(t.names)):
-            scope = t.family_vars(t.names[v])
-            if all(u in Eset for u in scope):
-                observed.append(v)
-                continue
-            tensor = None if dry else t.table_view(t.log_cond, t.names[v]).reshape(-1)
-            factors.append(Factor(list(scope), tensor))
-        hidden = [v for v in range(len(t.names)) if v not in Eset]
+        factors, observed = self._factors(cx, every, split_observed=True)
+        hidden = [v for v in every if v not in cx.ev]
         stats.n_hidden = len(hidden)
-        stats.relevant_evidence = list(E)
+        stats.relevant_evidence = list(cx.E)
         elim: list = []
-        finals: List[Factor] = []
-        if factors:
-            finals = self._eliminate(factors, hidden, sort_scope, stats, dry, None, decode=elim)
-        argmax_bytes = sum(max(_prod(cards[u] for u in sc), 1) for _, sc, _ in elim)
-        if dry:
+        finals = self._eliminate(cx, factors, hidden, decode=elim) if factors else []
+        argmax_bytes = sum(max(_cells(sc, cards), 1) for _, sc, _ in elim)
+        if cx.dry:
             if argmax_bytes > self.mpe_argmax_budget:
                 raise PlanTooLarge(f"the argmax tables of this explanation need {argmax_bytes} bytes "
                                    f"(budget {self.mpe_argmax_budget})")
             widest = max((len(sc) for _, sc, _ in elim), default=0)
             if widest > N.MAX_CONTRACT_DIMS:
                 raise PlanTooLarge(f"an argmax table with {widest} axes exceeds {N.MAX_CONTRACT_DIMS}")
-            ev_read = {u for _, sc, _ in elim for u in sc if u in Eset}
+            ev_read = {u for _, sc, _ in elim for u in sc if u in cx.ev}
             if len(ev_read) + len(hidden) > N.MPE_MAX_SLOTS:
                 raise PlanTooLarge(f"{len(ev_read)} evidence columns and {len(hidden)} hidden variables exceed the "
                                    f"{N.MPE_MAX_SLOTS} codes the traceback keeps per row")
-        ve_plan = None
-        if finals:
-            finals = self._merge_finals(finals, sort_scope, stats, dry, None)
-            stats.final_tables = [(tuple(f.scope), f.size(cards)) for f in finals]
-            if not dry:
-                ve_plan = QueryPlan(t, None, E, 1, finals, True, stats, log_space=True)
+        ve_plan = self._tail(cx, finals, []) if finals else None
         decode = [(v, tuple(sc), am) for v, sc, am in reversed(elim)]
-        split = MPESplit(evidence=list(E), hidden=hidden, observed_families=observed,
+        split = MPESplit(evidence=list(cx.E), hidden=hidden, observed_families=observed,
                          decode=[(v, sc) for v, sc, _ in decode], argmax_bytes=argmax_bytes, stats=stats)
-        if dry:
+        if cx.dry:
             return split
-        stats.contraction_gpu_ms = self._drain_events()
-        value = EvidencePlan(t, E, observed, ve_plan,
-                             EvidenceSplit(evidence=list(E), observed_families=observed, ve_stats=stats if factors else None))
-        plan = MPEPlan(t, split, decode, value)
-        self._mpe_cache[key] = plan
-        return plan
+        value = EvidencePlan(t, cx.E, observed, ve_plan,
+                             EvidenceSplit(evidence=list(cx.E), observed_families=observed, ve_stats=stats if factors else None))
+        return MPEPlan(t, split, decode, value)
 
-    def _drain_events(self) -> float:
-        if not self._events:
-            return 0.0
-        self._events[-1][1].synchronize()
-        ms = sum(a.elapsed_time(b) for a, b in self._events)
-        self._events = []
-        return ms
-
-    def _eliminate(self, factors: List[Factor], hidden: List[int], sort_scope, stats: PlanStats, dry: bool, T: int,
-                   partial: bool = False, decode: Optional[list] = None):
+    # ---------------------------------------------------------------- elimination
+    def _eliminate(self, cx: _Pass, factors: List[Factor], hidden: List[int], partial: bool = False,
+                   decode: Optional[list] = None):
         """Evidence-symbolic elimination.  With ``partial`` the loop stops when the cheapest step exceeds the table
         budget and returns ``(factors, remaining_hidden)`` for the per-row executor instead of raising.
 
         With a ``decode`` list the elimination is max-sum (log space): every step maximises over its variable and appends
         ``(variable, output scope, argmax table)`` to the list (the table is None in a dry run)."""
-        cards = self.t.cards
+        cards, stats = self.t.cards, cx.stats
         live: Dict[int, Factor] = dict(enumerate(factors))
         next_key = len(factors)
         g = _Greedy(cards, {k: f.scope for k, f in live.items()}, hidden)
-
-        def cells(scope):
-            s = 1
-            for v in scope:
-                s *= cards[v]
-            return s
-
         while g.hidden:
             v, best_cost, best_scope = g.best()
             if best_cost > self.table_budget and partial:
@@ -1035,14 +914,14 @@ class VECompiler:
             touching = [live[k] for k in keys]
             # the kernel multiplies at most MAX_CONTRACT_INPUTS factors at once: pre-multiply the smallest ones
             while len(touching) > N.MAX_CONTRACT_INPUTS:
-                order = sorted(range(len(touching)), key=lambda i: touching[i].size(cards))
+                order = sorted(range(len(touching)), key=lambda i: _cells(touching[i].scope, cards))
                 ia, ib = order[0], order[1]
                 a, b = touching[ia], touching[ib]
-                sc = sort_scope(a.scope + b.scope)
-                if cells(sc) > self.table_budget:
+                sc = cx.sort_scope(a.scope + b.scope)
+                if _cells(sc, cards) > self.table_budget:
                     raise PlanTooLarge("pre-multiplication exceeds the table budget")
-                stats.contraction_madds += 2 * cells(sc)
-                prod = self._contract([a, b], sc, None, dry)
+                stats.contraction_madds += 2 * _cells(sc, cards)
+                prod = self._contract([a, b], sc, None, cx)
                 g.replace([keys[ia], keys[ib]], next_key, sc)
                 for k in (keys[ia], keys[ib]):
                     del live[k]
@@ -1050,16 +929,16 @@ class VECompiler:
                 keys = [k for i, k in enumerate(keys) if i not in (ia, ib)] + [next_key]
                 touching = [f for i, f in enumerate(touching) if i not in (ia, ib)] + [prod]
                 next_key += 1
-            out_scope = sort_scope(best_scope)
+            out_scope = cx.sort_scope(best_scope)
             stats.n_steps += 1
             stats.max_table_cells = max(stats.max_table_cells, best_cost)
             stats.contraction_madds += best_cost * cards[v] * len(touching)
             if decode is not None:
-                am = None if dry else torch.empty(max(best_cost, 1), dtype=torch.uint8, device=self.t.device)
-                res = self._contract(touching, out_scope, v, dry, argmax=am)
+                am = None if cx.dry else torch.empty(max(best_cost, 1), dtype=torch.uint8, device=self.t.device)
+                res = self._contract(touching, out_scope, v, cx, argmax=am)
                 decode.append((v, out_scope, am))
             else:
-                res = self._contract(touching, out_scope, v, dry)
+                res = self._contract(touching, out_scope, v, cx)
             for k in keys:
                 del live[k]
             live[next_key] = res
@@ -1069,7 +948,7 @@ class VECompiler:
         return (out, []) if partial else out
 
     # ---------------------------------------------------------------- per-row schedule
-    def _row_plan(self, T: int, E: List[int], statics: List[Factor], hidden: List[int], stats: PlanStats, dry: bool):
+    def _row_plan(self, cx: _Pass, statics: List[Factor], hidden: List[int]):
         """Schedule the elimination of ``hidden`` per row: evidence axes of the static tables are sliced by the
         row's codes, so only hidden axes (and the target) count towards the size of a temporary.
 
@@ -1080,13 +959,9 @@ class VECompiler:
         permuted once, here, at compile time."""
         import numpy as np
 
-        cards = self.t.cards
-        Eset = set(E)
+        cards, T, E, Eset, stats = self.t.cards, cx.T, cx.E, cx.ev, cx.stats
         n_in = len(statics)
         MAXIN = N.MAX_CONTRACT_INPUTS
-
-        def size_of(scope):
-            return _prod(cards[v] for v in scope)
 
         # pass 1: (input keys, output key, output scope, summed variable or None)
         live = {k: [v for v in f.scope if v not in Eset] for k, f in enumerate(statics)}
@@ -1097,7 +972,7 @@ class VECompiler:
             v, _, sc = g.best()
             keys = list(g.touching(v))
             while len(keys) > MAXIN:                           # pre-multiply the two smallest
-                order = sorted(range(len(keys)), key=lambda i: size_of(live[keys[i]]))
+                order = sorted(range(len(keys)), key=lambda i: _cells(live[keys[i]], cards))
                 ka, kb = keys[order[0]], keys[order[1]]
                 psc = sorted(set(live[ka]) | set(live[kb]))
                 ops.append(([ka, kb], next_key, psc, None))
@@ -1137,13 +1012,6 @@ class VECompiler:
                 sc.append(v)
             return sc
 
-        def strides_of(scope):
-            st, s = {}, 1
-            for v in reversed(scope):
-                st[v] = s
-                s *= cards[v]
-            return st
-
         laid = []                                              # the static tables as the executor reads them
         fac = {}                                               # key -> (input id, free scope, strides over the free axes)
         for k, f in enumerate(statics):
@@ -1158,14 +1026,14 @@ class VECompiler:
             elif f.tensor is not None and f.tensor.data_ptr() % 16:
                 f = Factor(list(f.scope), f.tensor.clone())    # a view into a packed buffer: realign for vector loads
             laid.append(f)
-            st = strides_of(f.scope)
+            st = _strides(f.scope, cards)
             fac[k] = (k, [v for v in f.scope if v not in Eset], {v: st[v] for v in f.scope if v not in Eset})
         steps, off_chunks, off_at, temp_total = [], [], 0, 0
         for keys, out_key, out_scope, sum_var in ops:
             inputs = [fac[k] for k in keys]
             out_scope = lay_out(out_scope, out_key)
             out_shape = [cards[v] for v in out_scope]
-            out_size = _prod(out_shape)
+            out_size = math.prod(out_shape)
             if temp_total + (out_size + 3) // 4 * 4 > self.row_temp_floats:
                 raise PlanTooLarge(
                     f"per-row elimination needs more than {temp_total + out_size} floats of temporaries per row "
@@ -1186,36 +1054,29 @@ class VECompiler:
             temp_total += (out_size + 3) // 4 * 4
             stats.contraction_madds += out_size * sum_card * len(inputs)
             stats.per_row_madds += out_size * sum_card * len(inputs)
-            fac[out_key] = (n_in + len(steps) - 1, list(out_scope), strides_of(out_scope))
+            fac[out_key] = (n_in + len(steps) - 1, list(out_scope), _strides(out_scope, cards))
         offsets = np.ascontiguousarray(np.concatenate(off_chunks), dtype=np.int32)
         # the schedule as plain host data (what cbn_ve_plan_create_rows receives): kept for inspection and for the
         # CPU-side interpreter of tests/test_host_logic.py
         self.last_row_schedule = {"target": T, "evidence": list(E), "static_scopes": [list(f.scope) for f in laid],
                                   "static_source_scopes": [list(f.scope) for f in statics],
                                   "steps": steps, "offsets": offsets}
-        if dry:
+        if cx.dry:
             return None
-        return RowPlan(self.t, T, E, cards[T] if T is not None else 1, laid, steps, offsets, stats, self.log_space)
+        return RowPlan(self.t, T, E, cards[T] if T is not None else 1, laid, steps, offsets, stats, cx.log_space)
 
-    def _merge_finals(self, finals: List[Factor], sort_scope, stats: PlanStats, dry: bool, T: int) -> List[Factor]:
+    def _merge_finals(self, cx: _Pass, finals: List[Factor]) -> List[Factor]:
         """Multiply final tables together while the product stays within the merge budget: fewer gathers
         per row, and a single table can be normalised at compile time."""
-        cards = self.t.cards
+        sort_scope = cx.sort_scope
         finals = [Factor(sort_scope(f.scope), f.tensor) if f.scope == sort_scope(f.scope) else
-                  self._contract([f], sort_scope(f.scope), None, dry) for f in finals]
-
-        def cells(scope):
-            s = 1
-            for v in scope:
-                s *= cards[v]
-            return s
-
+                  self._contract([f], sort_scope(f.scope), None, cx) for f in finals]
         while len(finals) > 1:
             best = None
             for i in range(len(finals)):
                 for j in range(i + 1, len(finals)):
                     sc = sort_scope(finals[i].scope + finals[j].scope)
-                    c = cells(sc)
+                    c = _cells(sc, self.t.cards)
                     if best is None or c < best[0]:
                         best = (c, i, j, sc)
             c, i, j, sc = best
@@ -1225,9 +1086,9 @@ class VECompiler:
                 raise PlanTooLarge("cannot reduce the number of final tables within the budget")
             a, b = finals[i], finals[j]
             finals = [f for k, f in enumerate(finals) if k not in (i, j)]
-            stats.contraction_madds += 2 * c
-            stats.max_table_cells = max(stats.max_table_cells, c)
-            finals.append(self._contract([a, b], sc, None, dry))
+            cx.stats.contraction_madds += 2 * c
+            cx.stats.max_table_cells = max(cx.stats.max_table_cells, c)
+            finals.append(self._contract([a, b], sc, None, cx))
         return finals
 
 

@@ -86,13 +86,13 @@ def test_evidence_split_alarm_headline_set():
     assert [c for _, c in st.final_tables] == [839808]
 
 
-def test_evidence_split_per_row_when_the_budget_is_small():
+def test_evidence_per_row_schedule_when_the_budget_is_small():
     spec = synth.alarm()
     comp = VECompiler(DryTables(spec.names, spec.cards, spec.parents_by_name()), table_budget_cells=1 << 10)
     split = comp.compile_evidence(synth.ALARM_EVIDENCE, dry=True)
     assert split.per_row and split.ve_stats.per_row_hidden > 0
     # the per-row schedule ends in one cell (no target)
-    sched = comp._ev_child.last_row_schedule
+    sched = comp.last_row_schedule
     assert sched["target"] is None and sched["steps"][-1]["out_size"] == 1
 
 

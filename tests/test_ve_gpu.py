@@ -63,6 +63,50 @@ def test_asia_all_evidence_configurations():
         _check(spec, infer, target, names, ev)
 
 
+def test_new_cpts_reach_every_plan():
+    """New CPTs installed on bound tables (``set_cond_tables``, no re-fit and no re-bind) replace every plan built from
+    the old ones: posterior plans, fused posteriors, log P(e) and MPE all answer from the new tables."""
+    import sys
+
+    from continuousbayesiannetwork_b200 import synth
+    from continuousbayesiannetwork_b200.engine import install_cpts
+
+    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+    import loglik_oracle as LO
+    import mpe_oracle as MO
+
+    spec = synth.asia()
+    tables, infer = install_cpts(spec, DEV)
+    ev_names = ["asia", "smoke", "xray", "dysp"]
+    ids = [spec.names.index(e) for e in ev_names]
+    ev = np.array([[(i >> k) & 1 for k in range(4)] for i in range(16)])
+    cols = {n: torch.tensor(ev[:, e], dtype=torch.float32, device=DEV) for e, n in enumerate(ev_names)}
+    rng = np.random.default_rng(11)
+    new = synth.NetSpec(spec.names, spec.cards, spec.parents,
+                        [rng.dirichlet(np.ones(c.shape[-1]), size=c.shape[:-1]).astype(np.float32).astype(np.float64)
+                         for c in spec.cpts])
+    for s in (spec, new):
+        if s is new:
+            tables.set_cond_tables(new.cpts)
+        net = _net(s)
+        many = infer.infer_many(["lung", "bronc"], cols)           # two targets of two values: one fused launch
+        for tg in ("lung", "bronc"):
+            want = O.enumerate_posterior(net, s.names.index(tg), ids, ev)
+            np.testing.assert_allclose(infer.plan(tg, ev_names).run_codes(_codes_matrix(ev), 16).cpu().numpy(), want,
+                                       rtol=RTOL, atol=1e-30)
+            np.testing.assert_allclose(many[tg].cpu().numpy(), want, rtol=RTOL, atol=1e-30)
+        np.testing.assert_allclose(infer.log_evidence(cols).cpu().numpy(), LO.enumerate_log_evidence(net, ids, ev),
+                                   rtol=1e-5, atol=1e-5)
+        assignment, log_prob = infer.most_probable_explanation(cols)
+        best, _, _ = MO.enumerate_mpe(net, ids, ev)
+        np.testing.assert_allclose(log_prob.cpu().numpy(), best, rtol=1e-5, atol=1e-5)
+        full = np.zeros((16, s.n), dtype=np.int64)
+        full[:, ids] = ev
+        for name, vals in assignment.items():
+            full[:, s.names.index(name)] = vals.cpu().numpy().astype(np.int64)
+        np.testing.assert_allclose(MO.log_joint(net, full), best, rtol=1e-5, atol=1e-5)
+
+
 def test_alarm_and_random_dags():
     from continuousbayesiannetwork_b200 import synth
     from continuousbayesiannetwork_b200.engine import install_cpts
@@ -277,17 +321,17 @@ def test_config5_layered_dag_shallow_patterns():
     assert done >= 12 and kinds == {True, False}
 
 
-def test_contraction_kernel_on_large_outputs():
+def test_contraction_and_rescale_kernels_on_large_outputs():
     """``cbn_factor_contract`` against torch.einsum on outputs of 2^28+ cells with 10 axes of mixed cardinalities: the
     index decoding (multiply + shift per axis) must stay exact where the running remainder is close to 2^31."""
     from continuousbayesiannetwork_b200.tables import DiscreteTables
-    from continuousbayesiannetwork_b200.ve import Factor, VECompiler
+    from continuousbayesiannetwork_b200.ve import Factor, VECompiler, _Pass
 
     cards = [7, 3, 8, 5, 2, 6, 4, 255, 9, 3, 2]                     # variables 0..10; variable 10 is summed out
     names = [f"v{i}" for i in range(len(cards))]
     t = DiscreteTables(names, {}, device=DEV)
     t.set_cards(cards)
-    c = VECompiler(t, rescale=False)                                # the raw kernel; the rescaled variant is checked below
+    c = VECompiler(t)
     g = torch.Generator(device=DEV); g.manual_seed(4)
     a_scope, b_scope = [0, 2, 4, 7, 10], [1, 3, 5, 6, 8, 9, 10]
     A = torch.rand([cards[v] for v in a_scope], device=DEV, generator=g)
@@ -295,16 +339,16 @@ def test_contraction_kernel_on_large_outputs():
     out_scope = [7, 0, 1, 2, 3, 4, 5, 6, 8, 9]                      # 277,603,200 cells (1.1 GB of float32)
     n_out = int(np.prod([cards[v] for v in out_scope]))
     assert 1 << 28 < n_out < 1 << 31
-    got = c._contract([Factor(a_scope, A.reshape(-1)), Factor(b_scope, B.reshape(-1))], out_scope, 10, dry=False).tensor
+    got = c._contract([Factor(a_scope, A.reshape(-1)), Factor(b_scope, B.reshape(-1))], out_scope, 10,   # the raw kernel
+                      _Pass([], None, dry=False, log_space=False, rescale=False)).tensor
     letters = "abcdefghijk"
     expr = "".join(letters[v] for v in a_scope) + "," + "".join(letters[v] for v in b_scope) + "->" + "".join(letters[v] for v in out_scope)
     want = torch.einsum(expr, A, B).reshape(-1)
     assert got.numel() == n_out
     # range control: with variable 7 (the slowest output axis) declared an evidence axis, every one of its 255 slices is
     # divided by its own maximum (cbn_factor_rescale) -- bit-equal to the division done by torch
-    cr = VECompiler(t)
-    cr._ev_set = {7}
-    scaled = cr._contract([Factor(a_scope, A.reshape(-1)), Factor(b_scope, B.reshape(-1))], out_scope, 10, dry=False).tensor
+    scaled = c._contract([Factor(a_scope, A.reshape(-1)), Factor(b_scope, B.reshape(-1))], out_scope, 10,
+                         _Pass([7], None, dry=False, log_space=False, rescale=True)).tensor
     w2 = want.view(255, -1)
     torch.testing.assert_close(scaled.view(255, -1), w2 * (1.0 / w2.max(dim=1, keepdim=True).values), rtol=1e-6, atol=0)
     del scaled, w2
