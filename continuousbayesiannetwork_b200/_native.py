@@ -98,6 +98,19 @@ class MpeStep(C.Structure):
     ]
 
 
+class PsampleStep(C.Structure):
+    _fields_ = [
+        ("slot", C.c_int32),
+        ("card", C.c_int32),
+        ("cdf", C.c_void_p),
+        ("n_cells", C.c_int64),
+        ("n_ctx", C.c_int32),
+        ("ctx_slot", C.c_int32 * MAX_CONTRACT_DIMS),
+        ("ctx_stride", C.c_int32 * MAX_CONTRACT_DIMS),
+        ("var", C.c_int32),
+    ]
+
+
 MPE_MAX_SLOTS = 512
 ROWS_LOG_SPACE = 1
 GATHER_NORMALIZE, GATHER_LOG_SPACE = 1, 2
@@ -158,6 +171,12 @@ SIGNATURES = {
                                       C.POINTER(_P)]),
     "cbn_mpe_plan_destroy": (None, [_P]),
     "cbn_mpe_run": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, _P, C.c_int64, _P]),
+    "cbn_factor_contract_cdf": (C.c_int, [_P, C.POINTER(Contract), _P, _P]),
+    "cbn_psample_plan_create": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(PsampleStep), C.c_int32,
+                                          _P, C.POINTER(_P)]),
+    "cbn_psample_plan_destroy": (None, [_P]),
+    "cbn_psample_run": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, C.c_uint64, C.c_int64, C.c_int32, _P, C.c_int64,
+                                  _P]),
     "cbn_ve_run_codes_host": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P]),
     "cbn_ve_run_codes_host_multi": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P)]),
     "cbn_ve_run_codes_host_multi_ex": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P), C.c_int32]),

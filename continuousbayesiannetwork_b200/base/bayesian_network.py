@@ -251,6 +251,29 @@ class BayesianNetwork:
             raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not compute explanations")
         return mpe(cols)
 
+    def sample_posterior(self, data, n_draws: int = 1, seed: int = 0,
+                         first_row: int = 0) -> Tuple[Dict[str, torch.Tensor], torch.Tensor]:
+        """Exact joint draws of every node NOT in ``data`` from its posterior given each row, ``h ~ P(h | e)``: for
+        multiple imputation, uncertainty over hidden causes, or Monte Carlo estimates of joint queries.
+
+        :param data: a DataFrame or a dict name -> values holding domain VALUES, as ``most_probable_explanation`` takes
+                     them; the observed set is the set of columns passed, the same for every row.  A column that is not a
+                     node raises ``ValueError``.
+        :param n_draws: draws per row.
+        :param seed, first_row: draw d of row i depends only on ``(seed, first_row + i, d)``, so a batch split over calls
+                     (pass each part's offset as ``first_row``) or a smaller ``n_draws`` gives the same bits.
+        :return: ``(draws, log_evidence)``.  ``draws`` maps every other node to float32 [n_draws, n_rows] domain values on
+                 the device; ``log_evidence`` is float32 [n_rows], ``log P(e)`` (natural log).  A row with a value outside
+                 the fitted domain (NaN included) or evidence of probability zero gives ``log_evidence = -inf`` and NaN in
+                 every draw (never a NaN ``log_evidence``).  With no columns the result is one row of draws from the prior;
+                 with every node observed ``draws`` is empty and ``log_evidence`` equals ``log_likelihood``.
+        """
+        cols, _ = self._observed_columns(data)
+        sample = getattr(self.inference_obj, "sample_posterior", None)
+        if sample is None:
+            raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not sample posteriors")
+        return sample(cols, n_draws=n_draws, seed=seed, first_row=first_row)
+
     def _observed_columns(self, data) -> Tuple[Dict[str, torch.Tensor], int]:
         """``_columns`` for a subset of the nodes: (name -> float32 device column, number of rows)."""
         dev = self.device

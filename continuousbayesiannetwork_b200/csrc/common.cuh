@@ -145,6 +145,14 @@ __device__ __forceinline__ int domain_code(const float* __restrict__ dom, int ca
   return (lo < card && dom[lo] == x) ? lo : CBN_UNSEEN;
 }
 
+// the counter hash of the samplers (cbn_sample_forward, cbn_psample_run): splitmix64's increment and finaliser
+__device__ __forceinline__ uint64_t splitmix64(uint64_t z) {
+  z += 0x9E3779B97F4A7C15ull;
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  return z ^ (z >> 31);
+}
+
 // ---- mbarrier + 1-D bulk async copy (TMA engine) ----------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {

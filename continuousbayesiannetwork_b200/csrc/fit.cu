@@ -641,12 +641,6 @@ extern "C" int cbn_get_prob_f32(cbn_ctx* ctx, const float* table, const cbn_fami
 
 // =========================================================================== ancestral sampling
 namespace {
-__device__ __forceinline__ uint64_t splitmix64(uint64_t z) {
-  z += 0x9E3779B97F4A7C15ull;
-  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  return z ^ (z >> 31);
-}
 
 struct SampleFam {
   int var;

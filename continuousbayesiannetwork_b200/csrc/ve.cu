@@ -25,12 +25,19 @@ __device__ __forceinline__ float lse_pair(float a, float b) {
   return (hi == NEG_INF) ? NEG_INF : hi + log1pf(expf(lo - hi));
 }
 
-// LOG: the tables hold logarithms -- products are sums, the sum over the eliminated variable is a log-sum-exp.
-// MAX (requires LOG): max-sum instead -- the reduction keeps the largest term and its index s (strict >, so the smallest s
-// attaining the maximum), written to amax[o]; an all -inf reduction gives -inf and index 0.
-template <bool FAST, bool LOG, bool MAX = false>
+// The reduction over the eliminated variable s.
+// RED_SUM: sum (LOG: the tables hold logarithms -- products are sums, the sum is a log-sum-exp).
+// RED_MAX (requires LOG): max-sum -- the reduction keeps the largest term and its index s (strict >, so the smallest s
+// attaining the maximum), written to aux[o] (uint8); an all -inf reduction gives -inf and index 0.
+// RED_CDF (requires LOG): the log-sum-exp of RED_SUM, bit for bit, plus the conditional of s given the cell as cumulative
+// thresholds, aux[o * (sum_card - 1) + x] = sum_{s <= x} exp(term_s - out[o]) (float, a second pass over s that
+// recomputes the terms); every threshold from the last s with a finite term onwards is exactly 1, so a value of
+// probability zero has an empty interval wherever it sits, and an all -inf cell is all ones.
+enum Red { RED_SUM, RED_MAX, RED_CDF };
+
+template <bool FAST, bool LOG, Red RED = RED_SUM>
 __global__ void __launch_bounds__(256) contract_kernel(const __grid_constant__ cbn_contract d, const __grid_constant__ ContractMagic mg,
-                                                       long long n_out, uint8_t* __restrict__ amax) {
+                                                       long long n_out, void* __restrict__ aux) {
   for (long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x; o < n_out;
        o += (long long)gridDim.x * blockDim.x) {
     long long base[CBN_MAX_CONTRACT_INPUTS];
@@ -56,9 +63,7 @@ __global__ void __launch_bounds__(256) contract_kernel(const __grid_constant__ c
           if (k < d.n_in) base[k] += (long long)c * d.in_stride[k][a];
       }
     }
-    float acc = LOG ? __int_as_float(0xff800000) : 0.0f;
-    int arg = 0;
-    for (int s = 0; s < d.sum_card; ++s) {
+    auto term = [&](int s) {
       float prod = LOG ? 0.0f : 1.0f;
 #pragma unroll
       for (int k = 0; k < CBN_MAX_CONTRACT_INPUTS; ++k)
@@ -66,14 +71,29 @@ __global__ void __launch_bounds__(256) contract_kernel(const __grid_constant__ c
           const float x = __ldg(d.in[k] + base[k] + (long long)s * d.sum_stride[k]);
           prod = LOG ? prod + x : prod * x;
         }
-      if constexpr (MAX) {
+      return prod;
+    };
+    float acc = LOG ? __int_as_float(0xff800000) : 0.0f;
+    int arg = RED == RED_CDF ? -1 : 0;
+    for (int s = 0; s < d.sum_card; ++s) {
+      const float prod = term(s);
+      if constexpr (RED == RED_MAX) {
         if (prod > acc) { acc = prod; arg = s; }
       } else {
         acc = LOG ? lse_pair(acc, prod) : acc + prod;
+        if constexpr (RED == RED_CDF) arg = prod > __int_as_float(0xff800000) ? s : arg;
       }
     }
     d.out[o] = acc;
-    if constexpr (MAX) amax[o] = (uint8_t)arg;
+    if constexpr (RED == RED_MAX) static_cast<uint8_t*>(aux)[o] = (uint8_t)arg;
+    if constexpr (RED == RED_CDF) {
+      float* c = static_cast<float*>(aux) + o * (d.sum_card - 1);
+      float run = 0.0f;
+      for (int s = 0; s < d.sum_card - 1; ++s) {
+        run += expf(term(s) - acc);
+        c[s] = s >= arg ? 1.0f : run;
+      }
+    }
   }
 }
 
@@ -81,9 +101,9 @@ __global__ void __launch_bounds__(256) contract_kernel(const __grid_constant__ c
 // (LO <= 1024 cells).  The per-input offsets of every o_lo are decoded ONCE per CTA into shared memory, o_hi is decoded
 // once per (CTA, o_hi) instead of once per cell, and a cell costs n_in shared-memory reads plus its table loads -- the
 // plain kernel spends most of its time on the multiply-shift decode of up to 13 axes per cell.
-template <bool LOG, int NIN, bool MAX = false>
+template <bool LOG, int NIN, Red RED = RED_SUM>
 __global__ void __launch_bounds__(256) contract_tiled_kernel(const __grid_constant__ cbn_contract d, const __grid_constant__ ContractMagic mg,
-                                                             long long n_hi, int lo_cells, int n_lo_dims, uint8_t* __restrict__ amax) {
+                                                             long long n_hi, int lo_cells, int n_lo_dims, void* __restrict__ aux) {
   extern __shared__ int lo_off[];          // [NIN][lo_cells]
   const int n_hi_dims = d.n_out_dims - n_lo_dims;
   for (int ol = threadIdx.x; ol < lo_cells; ol += blockDim.x) {
@@ -125,7 +145,7 @@ __global__ void __launch_bounds__(256) contract_tiled_kernel(const __grid_consta
 #pragma unroll
       for (int k = 0; k < NIN; ++k) p[k] = src[k] + hb[k] + lo_off[k * lo_cells + ol];
       float acc = LOG ? __int_as_float(0xff800000) : 0.0f;
-      int arg = 0;
+      int arg = RED == RED_CDF ? -1 : 0;
       for (int sv = 0; sv < sum_card; ++sv) {
         float prod = LOG ? 0.0f : 1.0f;
 #pragma unroll
@@ -134,14 +154,31 @@ __global__ void __launch_bounds__(256) contract_tiled_kernel(const __grid_consta
           p[k] += ss[k];
           prod = LOG ? prod + x : prod * x;
         }
-        if constexpr (MAX) {
+        if constexpr (RED == RED_MAX) {
           if (prod > acc) { acc = prod; arg = sv; }
         } else {
           acc = LOG ? lse_pair(acc, prod) : acc + prod;
+          if constexpr (RED == RED_CDF) arg = prod > __int_as_float(0xff800000) ? sv : arg;
         }
       }
       out[ol] = acc;
-      if constexpr (MAX) amax[oh * lo_cells + ol] = (uint8_t)arg;
+      if constexpr (RED == RED_MAX) static_cast<uint8_t*>(aux)[oh * lo_cells + ol] = (uint8_t)arg;
+      if constexpr (RED == RED_CDF) {
+        float* c = static_cast<float*>(aux) + (oh * lo_cells + ol) * (sum_card - 1);
+#pragma unroll
+        for (int k = 0; k < NIN; ++k) p[k] = src[k] + hb[k] + lo_off[k * lo_cells + ol];
+        float run = 0.0f;
+        for (int sv = 0; sv < sum_card - 1; ++sv) {
+          float prod = 0.0f;
+#pragma unroll
+          for (int k = 0; k < NIN; ++k) {
+            prod += __ldg(p[k]);
+            p[k] += ss[k];
+          }
+          run += expf(prod - acc);
+          c[sv] = sv >= arg ? 1.0f : run;
+        }
+      }
     }
   }
 }
@@ -240,9 +277,10 @@ int check_contract(cbn_ctx* ctx, const cbn_contract* desc, const char* fn, long 
   return CBN_OK;
 }
 
-// MAX: the max-sum reduction of cbn_factor_contract_max (log space, no normalisation: checked by the caller)
-template <bool MAX>
-int launch_contract(cbn_ctx* ctx, const cbn_contract* desc, long long n_out, uint8_t* amax, cudaStream_t s) {
+// RED_MAX / RED_CDF: the reductions of cbn_factor_contract_max / cbn_factor_contract_cdf (log space, no normalisation:
+// checked by the caller); aux is their argmax / threshold buffer
+template <Red RED>
+int launch_contract(cbn_ctx* ctx, const cbn_contract* desc, long long n_out, void* aux, cudaStream_t s) {
   int blocks = (int)std::min<long long>((n_out + 255) / 256, (long long)ctx->sm_count * 16);
   bool fast = n_out < (1ll << 31);
   ContractMagic mg{};
@@ -271,8 +309,8 @@ int launch_contract(cbn_ctx* ctx, const cbn_contract* desc, long long n_out, uin
       tiled = true;
       const int tb = (int)std::min<long long>(n_hi, (long long)ctx->sm_count * 8);
       const size_t sm = size_t(desc->n_in) * size_t(lo) * sizeof(int);
-      if constexpr (MAX) {
-#define CBN_TILED(K) contract_tiled_kernel<true, K, true><<<tb, 256, sm, s>>>(*desc, mg, n_hi, (int)lo, nlo, amax)
+      if constexpr (RED != RED_SUM) {
+#define CBN_TILED(K) contract_tiled_kernel<true, K, RED><<<tb, 256, sm, s>>>(*desc, mg, n_hi, (int)lo, nlo, aux)
         switch (desc->n_in) {
           case 1: CBN_TILED(1); break;
           case 2: CBN_TILED(2); break;
@@ -293,9 +331,9 @@ int launch_contract(cbn_ctx* ctx, const cbn_contract* desc, long long n_out, uin
     }
   }
   if (!tiled) {
-    if constexpr (MAX) {
-      if (fast) contract_kernel<true, true, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out, amax);
-      else contract_kernel<false, true, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out, amax);
+    if constexpr (RED != RED_SUM) {
+      if (fast) contract_kernel<true, true, RED><<<blocks, 256, 0, s>>>(*desc, mg, n_out, aux);
+      else contract_kernel<false, true, RED><<<blocks, 256, 0, s>>>(*desc, mg, n_out, aux);
     } else {
       if (fast) { if (lg) contract_kernel<true, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out, nullptr); else contract_kernel<true, false><<<blocks, 256, 0, s>>>(*desc, mg, n_out, nullptr); }
       else { if (lg) contract_kernel<false, true><<<blocks, 256, 0, s>>>(*desc, mg, n_out, nullptr); else contract_kernel<false, false><<<blocks, 256, 0, s>>>(*desc, mg, n_out, nullptr); }
@@ -303,6 +341,20 @@ int launch_contract(cbn_ctx* ctx, const cbn_contract* desc, long long n_out, uin
   }
   CBN_CHECK_LAUNCH(ctx);
   return CBN_OK;
+}
+
+// cbn_factor_contract_max / cbn_factor_contract_cdf: the checks they share, then the launch
+template <Red RED>
+int contract_with_table(cbn_ctx* ctx, const cbn_contract* desc, void* table, cbn_stream stream, const char* fn) {
+  if (!ctx) return cbn_fail(nullptr, CBN_ERR_INVALID, "%s: ctx is NULL", fn);
+  long long n_out = 0;
+  int rc = check_contract(ctx, desc, fn, &n_out);
+  if (rc) return rc;
+  if (!table || desc->log_space != 1 || desc->normalize_last != 0 || desc->sum_card > 255)
+    return cbn_fail(ctx, CBN_ERR_INVALID, "%s: needs log_space = 1, normalize_last = 0, sum_card <= 255 and %s buffer", fn,
+                    RED == RED_MAX ? "an argmax" : "a threshold");
+  DeviceGuard g(ctx->device);
+  return launch_contract<RED>(ctx, desc, n_out, table, (cudaStream_t)stream);
 }
 }  // namespace
 
@@ -313,7 +365,7 @@ extern "C" int cbn_factor_contract(cbn_ctx* ctx, const cbn_contract* desc, cbn_s
   if (rc) return rc;
   DeviceGuard g(ctx->device);
   cudaStream_t s = (cudaStream_t)stream;
-  rc = launch_contract<false>(ctx, desc, n_out, nullptr, s);
+  rc = launch_contract<RED_SUM>(ctx, desc, n_out, nullptr, s);
   if (rc) return rc;
   const bool lg = desc->log_space != 0;
   if (desc->normalize_last && desc->n_out_dims > 0) {
@@ -328,15 +380,11 @@ extern "C" int cbn_factor_contract(cbn_ctx* ctx, const cbn_contract* desc, cbn_s
 }
 
 extern "C" int cbn_factor_contract_max(cbn_ctx* ctx, const cbn_contract* desc, uint8_t* argmax_out, cbn_stream stream) {
-  if (!ctx) return cbn_fail(nullptr, CBN_ERR_INVALID, "cbn_factor_contract_max: ctx is NULL");
-  long long n_out = 0;
-  int rc = check_contract(ctx, desc, "cbn_factor_contract_max", &n_out);
-  if (rc) return rc;
-  if (!argmax_out || desc->log_space != 1 || desc->normalize_last != 0 || desc->sum_card > 255)
-    return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_factor_contract_max: needs log_space = 1, normalize_last = 0, sum_card <= 255 "
-                    "and an argmax buffer");
-  DeviceGuard g(ctx->device);
-  return launch_contract<true>(ctx, desc, n_out, argmax_out, (cudaStream_t)stream);
+  return contract_with_table<RED_MAX>(ctx, desc, argmax_out, stream, "cbn_factor_contract_max");
+}
+
+extern "C" int cbn_factor_contract_cdf(cbn_ctx* ctx, const cbn_contract* desc, float* cdf_out, cbn_stream stream) {
+  return contract_with_table<RED_CDF>(ctx, desc, cdf_out, stream, "cbn_factor_contract_cdf");
 }
 
 // =========================================================================== gather plan

@@ -7,7 +7,7 @@ import torch
 
 from .. import _native as N
 from ..base.inference import BaseInference
-from ..ve import EvidencePlan, FusedPlan, MPEPlan, QueryPlan, RowPlan, VECompiler
+from ..ve import EvidencePlan, FusedPlan, MPEPlan, PosteriorSamplePlan, QueryPlan, RowPlan, VECompiler
 
 
 class ExactInference(BaseInference):
@@ -22,7 +22,7 @@ class ExactInference(BaseInference):
         if self.normalization not in ("row", "global_max"):
             raise ValueError(f"normalization must be 'row' or 'global_max', got {self.normalization!r}")
         self._budget = {k: int(config[k]) for k in ("table_budget_cells", "merge_budget_cells", "row_temp_floats",
-                                                    "mpe_argmax_budget_bytes")
+                                                    "mpe_argmax_budget_bytes", "sample_table_budget_bytes")
                         if config and k in config}
         for k in ("log_space", "rescale", "profile_compile", "row_unit_layout"):
             if config and k in config:
@@ -119,13 +119,36 @@ class ExactInference(BaseInference):
         codes, nq = self._codes(evidence, names, mismatch="all evidence columns must have the same number of rows")
         plan = self.mpe_plan(names)
         hidden, log_prob = plan.run_codes(codes, nq)
-        assignment = {}
-        for h, v in enumerate(plan.hidden):
-            c = hidden[h, :nq].long()
-            dead = c >= t.cards[v]
-            vals = t.domains[v][c.clamp(max=t.cards[v] - 1)]
-            assignment[t.names[v]] = torch.where(dead, torch.full_like(vals, float("nan")), vals)
-        return assignment, log_prob
+        return {t.names[v]: self._values(v, hidden[h, :nq]) for h, v in enumerate(plan.hidden)}, log_prob
+
+    def _values(self, v: int, codes: torch.Tensor) -> torch.Tensor:
+        """Codes of variable ``v`` as float32 domain values, NaN where the code is CBN_UNSEEN."""
+        t = self.tables
+        c = codes.long()
+        vals = t.domains[v][c.clamp(max=t.cards[v] - 1)]
+        return torch.where(c >= t.cards[v], torch.full_like(vals, float("nan")), vals)
+
+    def posterior_sampler(self, evidence_names: Sequence[str]) -> PosteriorSamplePlan:
+        assert self.compiler is not None, "inference engine is not bound to a fitted network"
+        return self.compiler.compile_posterior_sampler(list(evidence_names))
+
+    def sample_posterior(self, evidence: Dict[str, torch.Tensor], n_draws: int = 1, seed: int = 0, first_row: int = 0):
+        """Exact draws from ``P(h | e)`` per row: ``(draws, log_evidence)``.  ``evidence``: name -> tensor [n_rows] or
+        [n_rows, 1] of category VALUES, the same observed set for every row.  ``draws`` maps every other node to float32
+        [n_draws, n_rows] domain values, each draw a joint sample of all of them (NaN where ``log_evidence`` is -inf);
+        ``log_evidence`` is float32 [n_rows] ``log P(e)`` (natural log; -inf for a value outside the fitted domain, NaN
+        included, or evidence of probability zero).  Draw d of row i depends only on ``(seed, first_row + i, d)``: split
+        a batch over calls with ``first_row`` and the draws are the same bits.  No evidence gives one row of draws from the
+        prior.  Not part of the reference's surface."""
+        if n_draws < 0 or first_row < 0:
+            raise ValueError("n_draws and first_row must not be negative")
+        t = self.tables
+        names = list(evidence or {})
+        codes, nq = self._codes(evidence, names, mismatch="all evidence columns must have the same number of rows")
+        plan = self.posterior_sampler(names)
+        hidden, log_evidence = plan.run_codes(codes, nq, n_draws=n_draws, seed=seed, first_row=first_row)
+        nh = len(plan.hidden)          # row d * nh + h of the code matrix: draw d of plan.hidden[h]
+        return {t.names[v]: self._values(v, hidden[h::nh][:n_draws, :nq]) for h, v in enumerate(plan.hidden)}, log_evidence
 
     def infer_map(self, target_node: str, evidence: Dict[str, torch.Tensor]) -> Optional[torch.Tensor]:
         """MAP value of the target per row through the fused kernel (``cbn_ve_run_f32_map``); ``None`` when the plan is

@@ -189,3 +189,15 @@ def sample_forward_numpy(spec: NetSpec, seed: int, first: int, n: int) -> np.nda
             x = (u[:, None] >= rows[:, : spec.cards[v] - 1]).sum(axis=1)
             codes[v] = x.astype(np.uint8)
     return codes
+
+
+def posterior_uniforms(seed: int, rows: np.ndarray, draw: int, var: int) -> np.ndarray:
+    """numpy restatement of ``cbn_psample_run``'s uniforms (bit-identical float32): the uniform of draw ``draw`` of
+    network variable ``var`` in each global row index of ``rows`` (``first_row + i``).  The row base is that of
+    ``sample_forward_numpy``; the draw index is mixed in before the variable."""
+    with np.errstate(over="ignore"):
+        rows = np.asarray(rows, dtype=np.uint64)
+        base = splitmix64(np.uint64(seed) ^ (rows * np.uint64(0xD1B54A32D192ED03)))
+        base = splitmix64(base ^ (np.uint64(draw) * np.uint64(0x9E6C63D0676A9A99)))
+        h = splitmix64(base + np.uint64(var))
+    return ((h >> np.uint64(40)).astype(np.uint32)).astype(np.float32) * np.float32(1.0 / 16777216.0)

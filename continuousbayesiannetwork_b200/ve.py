@@ -22,7 +22,9 @@ compile time, the gather / per-row kernels per evidence row).
 
 The same elimination with ``max`` in place of the sum (``VECompiler.compile_mpe``) gives the most probable explanation:
 every step also records its argmax table, and a per-row traceback (``cbn_mpe_run``) reads the hidden values back in
-reverse elimination order.
+reverse elimination order.  With the sum kept and the conditional of every step recorded as cumulative thresholds
+(``VECompiler.compile_posterior_sampler``), the same traceback with a random draw per step (``cbn_psample_run``) samples
+the hidden values exactly from ``P(h | e)``.
 """
 from __future__ import annotations
 
@@ -388,53 +390,73 @@ class EvidencePlan:
 
 
 @dataclass
-class MPESplit:
-    """Structure of a most-probable-explanation plan (``VECompiler.compile_mpe``)."""
+class DecodeSplit:
+    """Structure of a traceback plan over every hidden variable: the most probable explanation
+    (``VECompiler.compile_mpe``, ``MPESplit``) or posterior sampling (``VECompiler.compile_posterior_sampler``)."""
     evidence: List[int]
     hidden: List[int]                                   # network ids; row h of the decoded code matrix is hidden[h]
     observed_families: List[int]                        # CPTs scored by the observed-families kernel
-    decode: List[Tuple[int, Tuple[int, ...]]]           # (variable, scope of its argmax table) in decode order
-    argmax_bytes: int
+    decode: List[Tuple[int, Tuple[int, ...]]]           # (variable, scope of its table) in decode order
+    table_bytes: int                                    # argmax (uint8) or threshold (float) tables of every step
     stats: PlanStats
 
 
-class MPEPlan(_NativePlan):
-    """A compiled most probable explanation: the argmax tables of the max-sum elimination, the native traceback plan
-    (``cbn_mpe_plan_create``) and the ``EvidencePlan`` that computes each row's value ``log max_h P(h, e)``."""
-    _destroy = "cbn_mpe_plan_destroy"
+class MPESplit(DecodeSplit):
+    @property
+    def argmax_bytes(self) -> int:
+        return self.table_bytes
 
-    def __init__(self, tables_owner, split: MPESplit, decode, value: EvidencePlan):
+
+class _TracebackPlan(_NativePlan):
+    """What MPE and posterior-sampling plans share: the tables of the elimination (read by the native plan, so they are
+    kept alive with it), the native plan with one step per hidden variable in decode order (``_create``, steps of type
+    ``_step`` whose table pointer is the field ``_table``), and the ``EvidencePlan`` over the final tables, which gives
+    each row's value."""
+    _create = _step = _table = None
+
+    def __init__(self, tables_owner, split: DecodeSplit, decode, value: EvidencePlan):
         super().__init__(tables_owner)
         self.split = split
         self.evidence = list(split.evidence)
         self.hidden = list(split.hidden)
         self.value = value
-        self.argmax = [am for _, _, am in decode]           # referenced by the native plan: kept alive with it
+        self.tables = [tb for _, _, tb in decode]
         cards = tables_owner.cards
         n_ev = len(self.evidence)
         slot = {v: i for i, v in enumerate(self.evidence)}
         slot.update({v: n_ev + h for h, v in enumerate(self.hidden)})
         if not self.hidden:
             return
-        steps = (N.MpeStep * len(decode))()
-        for k, (v, scope, am) in enumerate(decode):
+        steps = (self._step * len(decode))()
+        for k, (v, scope, tb) in enumerate(decode):
             st = steps[k]
             st.slot = slot[v]
             st.card = cards[v]
-            st.argmax = am.data_ptr()
-            st.n_cells = am.numel()
+            setattr(st, self._table, tb.data_ptr())
+            st.n_cells = _cells(scope, cards)
             st.n_ctx = len(scope)
             stride = _strides(scope, cards)
             for j, u in enumerate(scope):
                 st.ctx_slot[j] = slot[u]
                 st.ctx_stride[j] = stride[u]
+            self._step_var(st, v)
         h = C.c_void_p()
-        N.check(N.lib().cbn_mpe_plan_create(self.ctx.handle, n_ev, _int32s([cards[v] for v in self.evidence]), len(self.hidden),
-                                            steps, len(decode), N.stream_ptr(self.device), C.byref(h)), self.ctx.handle)
+        N.check(getattr(N.lib(), self._create)(self.ctx.handle, n_ev, _int32s([cards[v] for v in self.evidence]),
+                                               len(self.hidden), steps, len(decode), N.stream_ptr(self.device), C.byref(h)),
+                self.ctx.handle)
         self.handle = h
+
+    def _step_var(self, step, v: int):
+        pass
 
     def set_static_evidence(self, on: bool = True):
         self.value.set_static_evidence(on)
+
+
+class MPEPlan(_TracebackPlan):
+    """A compiled most probable explanation: the argmax tables of the max-sum elimination, the native traceback plan
+    (``cbn_mpe_plan_create``) and the ``EvidencePlan`` that computes each row's value ``log max_h P(h, e)``."""
+    _destroy, _create, _step, _table = "cbn_mpe_plan_destroy", "cbn_mpe_plan_create", N.MpeStep, "argmax"
 
     def run_codes(self, ev_codes: torch.Tensor, n_rows: int, hidden_out: Optional[torch.Tensor] = None,
                   value_out: Optional[torch.Tensor] = None):
@@ -448,6 +470,32 @@ class MPEPlan(_NativePlan):
         if self.handle is not None and n_rows > 0:
             N.check(N.lib().cbn_mpe_run(self.ctx.handle, self.handle, ev_codes.data_ptr(), _ld(ev_codes), int(n_rows),
                                         value.data_ptr(), hidden_out.data_ptr(), hidden_out.stride(0), N.stream_ptr(self.device)),
+                    self.ctx.handle)
+        return hidden_out, value
+
+
+class PosteriorSamplePlan(_TracebackPlan):
+    """A compiled posterior sampler: the threshold tables of the sum-product elimination, the native backward-sampling
+    plan (``cbn_psample_plan_create``) and the ``EvidencePlan`` that computes each row's ``log P(e)``."""
+    _destroy, _create, _step, _table = "cbn_psample_plan_destroy", "cbn_psample_plan_create", N.PsampleStep, "cdf"
+
+    def _step_var(self, step, v: int):
+        step.var = v
+
+    def run_codes(self, ev_codes: torch.Tensor, n_rows: int, n_draws: int = 1, seed: int = 0, first_row: int = 0,
+                  hidden_out: Optional[torch.Tensor] = None, value_out: Optional[torch.Tensor] = None):
+        """ev_codes: uint8 [len(evidence), ld] on the device (row e = evidence variable e of the plan, ld a multiple of
+        16).  Returns ``(hidden_codes, log_evidence)``: uint8 [n_draws * len(hidden), ld'], row ``d * len(hidden) + h``
+        holding draw d of network variable ``hidden[h]`` (CBN_UNSEEN in every row whose ``log P(e)`` is -inf), and float32
+        [n_rows] ``log P(e_row)``.  Draw d of row i depends only on ``(seed, first_row + i, d)``."""
+        assert ev_codes.dtype == torch.uint8 and ev_codes.is_cuda
+        value = self.value.run_codes(ev_codes, n_rows, value_out)
+        if hidden_out is None:
+            hidden_out = self.owner.new_code_matrix(n_rows, max(int(n_draws) * len(self.hidden), 1))
+        if self.handle is not None and n_rows > 0:
+            N.check(N.lib().cbn_psample_run(self.ctx.handle, self.handle, ev_codes.data_ptr(), _ld(ev_codes), int(n_rows),
+                                            value.data_ptr(), int(seed) & ((1 << 64) - 1), int(first_row), int(n_draws),
+                                            hidden_out.data_ptr(), hidden_out.stride(0), N.stream_ptr(self.device)),
                     self.ctx.handle)
         return hidden_out, value
 
@@ -523,12 +571,15 @@ class _Pass:
     ``log_space``: the factors hold logarithms (log-sum-exp or max-sum contractions).  ``rescale``: range control of
     linear-space elimination -- after every contraction each evidence slice of the result is divided by its maximum
     (``cbn_factor_rescale``), a factor of the evidence configuration only, which cancels in the final normalisation, so
-    products of many small likelihoods stay inside the fp32 range.  ``dry``: structure only, no device work."""
+    products of many small likelihoods stay inside the fp32 range.  ``dry``: structure only, no device work.
+    ``reduce``: the reduction of the elimination steps that record a table for a traceback -- ``"max"`` (max-sum, argmax
+    tables: MPE) or ``"cdf"`` (log-sum-exp, cumulative conditionals: posterior sampling); ``"sum"`` records none."""
     E: List[int]                                        # evidence ids, in plan order
     T: Optional[int]                                    # the target (None: log P(e) and MPE)
     dry: bool
     log_space: bool
     rescale: bool
+    reduce: str = "sum"
     stats: PlanStats = field(default_factory=PlanStats)
     events: list = field(default_factory=list)          # CUDA events around every contraction (profile_compile)
 
@@ -552,7 +603,8 @@ class VECompiler:
 
     def __init__(self, tables, table_budget_cells: int = 1 << 28, merge_budget_cells: int = 1 << 24,
                  check_support: bool = True, row_temp_floats: int = 5000, log_space: bool = False, rescale: bool = True,
-                 profile_compile: bool = False, row_unit_layout: bool = True, mpe_argmax_budget_bytes: int = 1 << 30):
+                 profile_compile: bool = False, row_unit_layout: bool = True, mpe_argmax_budget_bytes: int = 1 << 30,
+                 sample_table_budget_bytes: int = 1 << 30):
         self.t = tables
         self.log_space = bool(log_space)                 # arithmetic of posterior compiles (see _Pass)
         self.rescale = bool(rescale)
@@ -563,6 +615,7 @@ class VECompiler:
         self.row_temp_floats = int(row_temp_floats)     # per-row temporaries of the per-row executor (shared memory)
         self.row_unit_layout = bool(row_unit_layout)    # lay every per-row factor out with its consumer's summed variable innermost
         self.mpe_argmax_budget = int(mpe_argmax_budget_bytes)    # argmax tables of one MPE plan, in bytes
+        self.sample_table_budget = int(sample_table_budget_bytes)    # threshold tables of one posterior sampler, in bytes
         self._plans: Dict[tuple, object] = {}           # (mode, key) -> plan
         self._plans_version = None
         self._has_zero: Dict[int, bool] = {}
@@ -612,9 +665,11 @@ class VECompiler:
 
     # ---------------------------------------------------------------- device contraction
     def _contract(self, inputs: List[Factor], out_scope: List[int], sum_var: Optional[int], cx: _Pass,
-                  normalize_last: bool = False, argmax: Optional[torch.Tensor] = None) -> Factor:
-        """``argmax``: uint8 device buffer of the output's size -- maximise over ``sum_var`` instead of summing
-        (``cbn_factor_contract_max``, log space) and record the maximising value of every output cell there."""
+                  normalize_last: bool = False, table: Optional[torch.Tensor] = None) -> Factor:
+        """``table``: the traceback table of this step, reduced by ``cx.reduce`` (log space) -- ``"max"``: maximise over
+        ``sum_var`` instead of summing and record the maximising value of every output cell (uint8 [cells],
+        ``cbn_factor_contract_max``); ``"cdf"``: sum as usual and record the conditional of ``sum_var`` given every output
+        cell as cumulative thresholds (float32 [cells, card - 1], ``cbn_factor_contract_cdf``)."""
         cards = self.t.cards
         if cx.dry:
             return Factor(out_scope, None)
@@ -640,9 +695,9 @@ class VECompiler:
         if self.profile_compile:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-        if argmax is not None:
-            N.check(N.lib().cbn_factor_contract_max(self.t.ctx.handle, C.byref(d), argmax.data_ptr(), N.stream_ptr(self.t.device)),
-                    self.t.ctx.handle)
+        if table is not None:
+            fn = N.lib().cbn_factor_contract_max if cx.reduce == "max" else N.lib().cbn_factor_contract_cdf
+            N.check(fn(self.t.ctx.handle, C.byref(d), table.data_ptr(), N.stream_ptr(self.t.device)), self.t.ctx.handle)
         else:
             N.check(N.lib().cbn_factor_contract(self.t.ctx.handle, C.byref(d), N.stream_ptr(self.t.device)), self.t.ctx.handle)
         if cx.rescale and not normalize_last:
@@ -662,17 +717,17 @@ class VECompiler:
 
     # ---------------------------------------------------------------- compile front end
     def _compile(self, mode: str, key: tuple, E: List[int], T: Optional[int], dry: bool, build,
-                 log_space: bool = True, rescale: bool = False):
+                 log_space: bool = True, rescale: bool = False, reduce: str = "sum"):
         """Run ``build(pass)`` -- the part of the compile that is the mode's own -- as a structure-only pass (``dry``), or
         return the cached plan of ``(mode, key)``.  A plan is compiled after a structure-only pass: a query that does not
         fit fails there, before any table is contracted.  The default arithmetic is that of ``log P(e)`` and MPE: log space
         without range control."""
         if dry:
-            return build(_Pass(E, T, True, log_space, rescale))
+            return build(_Pass(E, T, True, log_space, rescale, reduce))
 
         def compile_plan():
-            build(_Pass(E, T, True, log_space, rescale))
-            cx = _Pass(E, T, False, log_space, rescale)
+            build(_Pass(E, T, True, log_space, rescale, reduce))
+            cx = _Pass(E, T, False, log_space, rescale, reduce)
             plan = build(cx)
             cx.stats.contraction_gpu_ms = cx.device_ms()
             return plan
@@ -854,10 +909,31 @@ class VECompiler:
 
         ``dry=True`` works on ``DryTables`` and returns the ``MPESplit`` only (no device work)."""
         E = self._evidence_ids(evidence_names)
-        return self._compile("mpe", tuple(E), E, None, dry, self._mpe)
+        return self._compile("mpe", tuple(E), E, None, dry, self._traceback, reduce="max")
 
-    def _mpe(self, cx: _Pass):
+    # ---------------------------------------------------------------- posterior sampling: h ~ P(h | e)
+    def compile_posterior_sampler(self, evidence_names: Sequence[str], dry: bool = False):
+        """Compile exact sampling from ``P(h | e)`` for the evidence set ``evidence_names``: per row and draw, a value of
+        EVERY other node drawn jointly from its posterior, and the row's ``log P(e)``.
+
+        Forward filtering, backward sampling over the elimination of ``compile_mpe`` (same order, every CPT of the
+        network) with the sum kept: ``cbn_factor_contract_cdf`` eliminates each hidden variable ``v_k`` by log-sum-exp and
+        records ``P(v_k | ctx_k)`` -- its touching factors over their log-sum-exp -- as cumulative thresholds per context.
+        What is left are tables over evidence subsets, whose ``EvidencePlan`` gives ``log P(e)``.  The traceback
+        (``cbn_psample_run``) draws the variables in reverse elimination order, each from the thresholds of a context that
+        is evidence or was drawn before it, so the draws follow ``prod_k P(v_k | ctx_k) = P(h | e)``.  The limits are those
+        of MPE, with the threshold tables bounded by ``sample_table_budget_bytes``; all raise ``PlanTooLarge`` in the
+        structure-only pass.
+
+        ``dry=True`` works on ``DryTables`` and returns the ``DecodeSplit`` only (no device work)."""
+        E = self._evidence_ids(evidence_names)
+        return self._compile("psample", tuple(E), E, None, dry, self._traceback, reduce="cdf")
+
+    def _traceback(self, cx: _Pass):
+        """The part of ``compile_mpe`` and ``compile_posterior_sampler`` that is theirs: every hidden variable is eliminated
+        with its table recorded (``cx.reduce``), then the tables are handed to the traceback in decode order."""
         t, cards, stats = self.t, self.t.cards, cx.stats
+        sampling = cx.reduce == "cdf"
         every = range(len(t.names))
         stats.n_relevant = len(t.names)
         factors, observed = self._factors(cx, every, split_observed=True)
@@ -866,27 +942,33 @@ class VECompiler:
         stats.relevant_evidence = list(cx.E)
         elim: list = []
         finals = self._eliminate(cx, factors, hidden, decode=elim) if factors else []
-        argmax_bytes = sum(max(_cells(sc, cards), 1) for _, sc, _ in elim)
+        if sampling:
+            table_bytes = sum(4 * _cells(sc, cards) * (cards[v] - 1) for v, sc, _ in elim)
+            budget, what = self.sample_table_budget, "the threshold tables of this sampler"
+        else:
+            table_bytes = sum(max(_cells(sc, cards), 1) for _, sc, _ in elim)
+            budget, what = self.mpe_argmax_budget, "the argmax tables of this explanation"
         if cx.dry:
-            if argmax_bytes > self.mpe_argmax_budget:
-                raise PlanTooLarge(f"the argmax tables of this explanation need {argmax_bytes} bytes "
-                                   f"(budget {self.mpe_argmax_budget})")
+            if table_bytes > budget:
+                raise PlanTooLarge(f"{what} need {table_bytes} bytes (budget {budget})")
             widest = max((len(sc) for _, sc, _ in elim), default=0)
             if widest > N.MAX_CONTRACT_DIMS:
-                raise PlanTooLarge(f"an argmax table with {widest} axes exceeds {N.MAX_CONTRACT_DIMS}")
+                raise PlanTooLarge(f"{'a threshold' if sampling else 'an argmax'} table with {widest} axes exceeds "
+                                   f"{N.MAX_CONTRACT_DIMS}")
             ev_read = {u for _, sc, _ in elim for u in sc if u in cx.ev}
             if len(ev_read) + len(hidden) > N.MPE_MAX_SLOTS:
                 raise PlanTooLarge(f"{len(ev_read)} evidence columns and {len(hidden)} hidden variables exceed the "
                                    f"{N.MPE_MAX_SLOTS} codes the traceback keeps per row")
         ve_plan = self._tail(cx, finals, []) if finals else None
-        decode = [(v, tuple(sc), am) for v, sc, am in reversed(elim)]
-        split = MPESplit(evidence=list(cx.E), hidden=hidden, observed_families=observed,
-                         decode=[(v, sc) for v, sc, _ in decode], argmax_bytes=argmax_bytes, stats=stats)
+        decode = [(v, tuple(sc), tb) for v, sc, tb in reversed(elim)]
+        split = (DecodeSplit if sampling else MPESplit)(
+            evidence=list(cx.E), hidden=hidden, observed_families=observed, decode=[(v, sc) for v, sc, _ in decode],
+            table_bytes=table_bytes, stats=stats)
         if cx.dry:
             return split
         value = EvidencePlan(t, cx.E, observed, ve_plan,
                              EvidenceSplit(evidence=list(cx.E), observed_families=observed, ve_stats=stats if factors else None))
-        return MPEPlan(t, split, decode, value)
+        return (PosteriorSamplePlan if sampling else MPEPlan)(t, split, decode, value)
 
     # ---------------------------------------------------------------- elimination
     def _eliminate(self, cx: _Pass, factors: List[Factor], hidden: List[int], partial: bool = False,
@@ -894,8 +976,8 @@ class VECompiler:
         """Evidence-symbolic elimination.  With ``partial`` the loop stops when the cheapest step exceeds the table
         budget and returns ``(factors, remaining_hidden)`` for the per-row executor instead of raising.
 
-        With a ``decode`` list the elimination is max-sum (log space): every step maximises over its variable and appends
-        ``(variable, output scope, argmax table)`` to the list (the table is None in a dry run)."""
+        With a ``decode`` list every step records its traceback table, reduced by ``cx.reduce`` (see ``_contract``), and
+        appends ``(variable, output scope, table)`` to the list (the table is None in a dry run)."""
         cards, stats = self.t.cards, cx.stats
         live: Dict[int, Factor] = dict(enumerate(factors))
         next_key = len(factors)
@@ -908,8 +990,8 @@ class VECompiler:
                 raise PlanTooLarge(
                     f"eliminating the cheapest hidden variable needs a table of {best_cost} cells "
                     f"(budget {self.table_budget}); " +
-                    ("the most probable explanation has no per-row executor" if decode is not None else
-                     "this query needs the per-row executor"))
+                    (f"{'the most probable explanation' if cx.reduce == 'max' else 'posterior sampling'} has no per-row "
+                     "executor" if decode is not None else "this query needs the per-row executor"))
             keys = g.touching(v)
             touching = [live[k] for k in keys]
             # the kernel multiplies at most MAX_CONTRACT_INPUTS factors at once: pre-multiply the smallest ones
@@ -934,9 +1016,13 @@ class VECompiler:
             stats.max_table_cells = max(stats.max_table_cells, best_cost)
             stats.contraction_madds += best_cost * cards[v] * len(touching)
             if decode is not None:
-                am = None if cx.dry else torch.empty(max(best_cost, 1), dtype=torch.uint8, device=self.t.device)
-                res = self._contract(touching, out_scope, v, cx, argmax=am)
-                decode.append((v, out_scope, am))
+                tb = None
+                if not cx.dry and cx.reduce == "max":
+                    tb = torch.empty(max(best_cost, 1), dtype=torch.uint8, device=self.t.device)
+                elif not cx.dry:
+                    tb = torch.empty(max(best_cost * (cards[v] - 1), 1), dtype=torch.float32, device=self.t.device)
+                res = self._contract(touching, out_scope, v, cx, table=tb)
+                decode.append((v, out_scope, tb))
             else:
                 res = self._contract(touching, out_scope, v, cx)
             for k in keys:

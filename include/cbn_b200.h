@@ -207,6 +207,15 @@ CBN_API int cbn_factor_contract(cbn_ctx* ctx, const cbn_contract* desc, cbn_stre
  * An all -inf reduction gives -inf and index 0.  Requires log_space = 1, normalize_last = 0, sum_card <= 255 and a
  * non-NULL argmax_out (device uint8 [n_out]); anything else is CBN_ERR_INVALID. */
 CBN_API int cbn_factor_contract_max(cbn_ctx* ctx, const cbn_contract* desc, uint8_t* argmax_out, cbn_stream stream);
+/* One sum step of a posterior-sampling elimination, on the same descriptor: out[o] is bit for bit what cbn_factor_contract
+ * writes in log space, and the conditional of s given the output cell is recorded as cumulative thresholds
+ *     cdf_out[o * (sum_card - 1) + x] = sum_{s <= x} exp(term_s - out[o])      for x < sum_card - 1   (fp32 running sum)
+ * where term_s is the log product that out[o] sums.  Every threshold from the last s with a finite term onwards is exactly
+ * 1.0f, and a cell whose terms are all -inf is all 1.0f, so a value of probability zero has an empty interval and is never
+ * drawn by the rule x = #{t : u >= cdf[t]} for u in [0, 1).  sum_card = 1 writes no thresholds.  Requires log_space = 1,
+ * normalize_last = 0, sum_card <= 255 and a non-NULL cdf_out (device float [n_out * (sum_card - 1)]); anything else is
+ * CBN_ERR_INVALID. */
+CBN_API int cbn_factor_contract_cdf(cbn_ctx* ctx, const cbn_contract* desc, float* cdf_out, cbn_stream stream);
 /* Range control of the compile-time elimination (the linear-space counterpart of working in log space): `table` holds
  * n_slices contiguous slices of slice_size cells -- one slice per configuration of the factor's evidence axes, which are
  * its slowest axes -- and every slice is divided by its own maximum (all-zero slices stay zero).  A factor that depends on
@@ -400,6 +409,49 @@ CBN_API int cbn_mpe_plan_create(cbn_ctx* ctx, int32_t n_evidence, const int32_t*
 CBN_API void cbn_mpe_plan_destroy(cbn_mpe_plan* plan);
 CBN_API int cbn_mpe_run(cbn_ctx* ctx, const cbn_mpe_plan* plan, const uint8_t* ev_codes, int64_t ld, int64_t n_rows,
                         const float* log_value, uint8_t* hidden_codes, int64_t out_ld, cbn_stream stream);
+
+/* ---- posterior sampling: backward sampling through the thresholds of a sum-product elimination ----------------------
+ * After a log-space sum-product elimination (cbn_factor_contract_cdf) of every hidden variable with the evidence kept
+ * symbolic, exact draws from P(h | e) are taken in reverse elimination order: step k draws its variable from the
+ * conditional recorded for the context of the row,
+ *     c = cdf_k + (sum_j code[ctx_slot_k_j] * ctx_stride_k_j) * (card_k - 1),    code[slot_k] = #{t < card_k - 1 : u >= c[t]}
+ * with the slots of cbn_mpe_step (every context is evidence or was drawn by an earlier step).  The product of the
+ * conditionals is P(h | e) exactly.  Nothing in the reference computes this.
+ *
+ * The uniform of draw d of variable `var` (network id) in row first_row + i is a counter hash, a function of those four
+ * numbers only (not of n_draws, of the split of the rows over calls, or of the grid):
+ *     mix(z) = splitmix64 finaliser (cbn_sample_forward's hash)
+ *     h = mix(mix(mix(seed ^ (row * 0xD1B54A32D192ED03)) ^ (d * 0x9E6C63D0676A9A99)) + var)      (uint64 arithmetic)
+ *     u = (h >> 40) * 2^-24                                                                      (a 24-bit uniform)
+ * so for d = 0 the row base is that of cbn_sample_forward's sample `row`, and a prefix of the draws of a larger n_draws
+ * is bit-identical to a smaller n_draws.
+ *
+ * cbn_psample_plan_create: the checks, slot limit (CBN_MPE_MAX_SLOTS), staging and lifetime rules of
+ * cbn_mpe_plan_create; n_cells counts contexts (the table holds n_cells * (card - 1) floats; cdf may be NULL when
+ * card == 1).
+ * cbn_psample_run: draw d of hidden variable h at hidden_codes + (d * n_hidden + h) * out_ld (out_ld >= n_rows, a
+ * multiple of 16, 16-byte aligned base; ev_codes likewise), so every draw stacks with the evidence into complete rows.
+ * log_value: device float [n_rows], the row's log P(e) (EvidencePlan of the same elimination).  A row whose log_value is
+ * -inf or NaN, or whose evidence code is not below its cardinality, gets CBN_UNSEEN in every hidden column of every
+ * draw.  Indices are clamped.  Launched without programmatic dependent launch, so log_value may come from the kernel
+ * right before it on the stream. */
+typedef struct cbn_psample_plan cbn_psample_plan;
+typedef struct cbn_psample_step {
+  int32_t slot;                              /* slot this step writes: n_evidence + h for hidden variable h */
+  int32_t card;                              /* that variable's cardinality (<= 255) */
+  const float* cdf;                          /* device: n_cells rows of card - 1 thresholds */
+  int64_t n_cells;                           /* contexts */
+  int32_t n_ctx;                             /* axes the table is indexed by */
+  int32_t ctx_slot[CBN_MAX_CONTRACT_DIMS];   /* evidence slots, or hidden slots written by an EARLIER step */
+  int32_t ctx_stride[CBN_MAX_CONTRACT_DIMS];
+  int32_t var;                               /* network id of the variable: the counter of its uniforms */
+} cbn_psample_step;
+CBN_API int cbn_psample_plan_create(cbn_ctx* ctx, int32_t n_evidence, const int32_t* ev_cards, int32_t n_hidden,
+                                    const cbn_psample_step* steps, int32_t n_steps, cbn_stream stream, cbn_psample_plan** out);
+CBN_API void cbn_psample_plan_destroy(cbn_psample_plan* plan);
+CBN_API int cbn_psample_run(cbn_ctx* ctx, const cbn_psample_plan* plan, const uint8_t* ev_codes, int64_t ld, int64_t n_rows,
+                            const float* log_value, uint64_t seed, int64_t first_row, int32_t n_draws, uint8_t* hidden_codes,
+                            int64_t out_ld, cbn_stream stream);
 
 /* ---- ancestral sampling (synthetic workloads; BruteForce._sample's network analogue,
  * brute_force.py:246-265).  Counter-based: sample i of variable v depends only on

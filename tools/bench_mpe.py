@@ -92,7 +92,7 @@ def alarm_legs(peak):
     legs.append(_rate("alarm_traceback", n, ms, len(ev_read) + 4 + len(plan.hidden), peak, it, win,
                       dependent_lookups_per_row=len(plan.hidden), evidence_columns_read=len(ev_read),
                       argmax_bytes=plan.split.argmax_bytes,
-                      largest_argmax_table=max(int(a.numel()) for a in plan.argmax)))
+                      largest_argmax_table=max(int(a.numel()) for a in plan.tables)))
     # oracle: a seeded sample of rows of the last launches
     rows = np.sort(np.random.default_rng(71).choice(n, size=SAMPLE, replace=False))
     r = torch.from_numpy(rows).to(DEV)
