@@ -1143,7 +1143,7 @@ class VECompiler:
             fac[out_key] = (n_in + len(steps) - 1, list(out_scope), _strides(out_scope, cards))
         offsets = np.ascontiguousarray(np.concatenate(off_chunks), dtype=np.int32)
         # the schedule as plain host data (what cbn_ve_plan_create_rows receives): kept for inspection and for the
-        # CPU-side interpreter of tests/test_host_logic.py
+        # fp64 interpreter of tests/row_oracle.py
         self.last_row_schedule = {"target": T, "evidence": list(E), "static_scopes": [list(f.scope) for f in laid],
                                   "static_source_scopes": [list(f.scope) for f in statics],
                                   "steps": steps, "offsets": offsets}

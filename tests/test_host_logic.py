@@ -10,6 +10,9 @@ import pytest
 from continuousbayesiannetwork_b200 import sharding, synth
 from continuousbayesiannetwork_b200.ve import DryTables, PlanTooLarge, VECompiler
 
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import row_oracle as RO  # noqa: E402
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -154,42 +157,16 @@ def test_incremental_greedy_matches_full_rescan():
         assert not g.hidden
 
 
-def _interpret_row_schedule(sch, spec, rows):
-    """numpy interpreter of a per-row schedule (the host data ``cbn_ve_plan_create_rows`` receives), fed with the ground-truth
-    CPTs laid out as the schedule says; one posterior row per evidence row."""
-    ev_ids = sch["evidence"]
+def _cpt_statics(sch, spec):
+    """The static tables of a per-row schedule compiled with a table budget of one cell: the CPTs themselves, permuted to
+    the layout the schedule reads."""
     statics = []
     for scope, source in zip(sch["static_scopes"], sch["static_source_scopes"]):
-        node = source[-1]        # with a table budget of one cell the static tables are the CPTs themselves
+        node = source[-1]
         assert source == spec.parents[node] + [node] and sorted(scope) == sorted(source)
         cpt = np.asarray(spec.cpts[node], dtype=np.float64).reshape([spec.cards[v] for v in source])
-        statics.append((scope, np.ascontiguousarray(cpt.transpose([source.index(v) for v in scope])).reshape(-1)))
-    got = np.zeros((rows.shape[0], spec.cards[sch["target"]]))
-    offs_all = sch["offsets"]
-    for r, ev in enumerate(rows):
-        code_of = dict(zip(ev_ids, ev))
-        bases = []
-        for scope, _ in statics:                          # slice every static table by the row's evidence codes
-            b, stride = 0, 1
-            for v in reversed(scope):
-                if v in code_of:
-                    b += int(code_of[v]) * stride
-                stride *= spec.cards[v]
-            bases.append(b)
-        temps = []
-        for st in sch["steps"]:
-            n_in, out_size = len(st["in_id"]), st["out_size"]
-            offs = offs_all[st["offsets_at"]: st["offsets_at"] + n_in * out_size].reshape(n_in, out_size).astype(np.int64)
-            out = np.zeros(out_size)
-            for sv in range(st["sum_card"]):
-                prod = np.ones(out_size)
-                for k, i in enumerate(st["in_id"]):
-                    idx = offs[k] + sv * st["sum_stride"][k]
-                    prod = prod * (statics[i][1][bases[i] + idx] if i < len(statics) else temps[i - len(statics)][idx])
-                out += prod
-            temps.append(out)
-        got[r] = temps[-1] / temps[-1].sum()
-    return got
+        statics.append(np.ascontiguousarray(cpt.transpose([source.index(v) for v in scope])).reshape(-1))
+    return statics
 
 
 def test_row_schedule_interpreted_on_the_cpu_matches_the_oracle():
@@ -231,6 +208,6 @@ def test_row_schedule_interpreted_on_the_cpu_matches_the_oracle():
             assert all(i < len(sch["static_scopes"]) + j for j, st in enumerate(sch["steps"]) for i in st["in_id"])
             codes = synth.sample_forward_numpy(spec, 9, 0, 40)
             rows = codes[ev_ids].T
-            got = _interpret_row_schedule(sch, spec, rows)
+            got = RO.posterior(RO.interpret(sch, _cpt_statics(sch, spec), spec.cards, rows))
             want = O.ve_posterior(O.DiscreteNet(spec.cards, spec.parents, spec.cpts), sch["target"], ev_ids, rows, dtype=torch.float64)
             np.testing.assert_allclose(got, want, rtol=1e-9, atol=1e-15)
