@@ -111,7 +111,21 @@ class PsampleStep(C.Structure):
     ]
 
 
+class EssDest(C.Structure):
+    _fields_ = [
+        ("table_offset", C.c_int64),
+        ("n_cells", C.c_int64),
+        ("n_obs", C.c_int32),
+        ("obs_row", C.c_int32 * MAX_FAMILY_VARS),
+        ("obs_card", C.c_int32 * MAX_FAMILY_VARS),
+        ("obs_stride", C.c_int32 * MAX_FAMILY_VARS),
+        ("hidden_cell", C.c_void_p),
+    ]
+
+
 MPE_MAX_SLOTS = 512
+ESS_MAX_DESTS = 64
+ESS_MAX_CONFIGS = 65536
 ROWS_LOG_SPACE = 1
 GATHER_NORMALIZE, GATHER_LOG_SPACE = 1, 2
 HOST_OUT_DROP_LAST = 1
@@ -177,6 +191,10 @@ SIGNATURES = {
     "cbn_psample_plan_destroy": (None, [_P]),
     "cbn_psample_run": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, C.c_uint64, C.c_int64, C.c_int32, _P, C.c_int64,
                                   _P]),
+    "cbn_ess_plan_create": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32), C.POINTER(EssDest), C.c_int32, _P, C.POINTER(_P)]),
+    "cbn_ess_plan_destroy": (None, [_P]),
+    "cbn_ess_run": (C.c_int, [_P, _P, C.POINTER(_P), _P, C.c_int64, C.c_int64, _P, _P]),
+    "cbn_ess_plan_smem_dests": (C.c_int, [_P]),
     "cbn_ve_run_codes_host": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P]),
     "cbn_ve_run_codes_host_multi": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P)]),
     "cbn_ve_run_codes_host_multi_ex": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P), C.c_int32]),

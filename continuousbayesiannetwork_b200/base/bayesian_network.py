@@ -16,6 +16,8 @@ or undefined, SURVEY.md section 3.3):
   summed out exactly (held-out log-likelihood, anomaly scores, probability of evidence); the reference has no such query.
 * ``most_probable_explanation(data)`` gives, per row, the jointly most probable values of every node not in ``data`` and
   their log-probability ``log max_h P(h, e)`` (missing-value completion, diagnosis); the reference has no such query.
+* ``latent={"Z": k}`` / ``fit_em(data)`` fit networks with hidden nodes (no column in the data) by exact EM; the reference
+  can only fit complete data.
 """
 from __future__ import annotations
 
@@ -33,9 +35,14 @@ from ..utils import choose_inference_obj
 
 class BayesianNetwork:
     def __init__(self, dag: nx.DiGraph, data, parameters_learning_config: Dict, inference_config: Dict, **kwargs):
+        """``latent``: hidden nodes, which have no column in ``data``: name -> cardinality k (domain 0.0 .. k-1) or the list
+        of domain values.  With it the network is fitted by ``fit_em``, with the settings read from
+        ``parameters_learning_config`` keys ``em_max_iter`` (100), ``em_tol`` (1e-6), ``em_seed`` (0) and
+        ``em_pseudo_count`` (0); ``self.em_result`` holds the ``EMResult``."""
         if not nx.is_directed_acyclic_graph(dag):
             raise ValueError("The provided graph is not a directed acyclic graph (DAG).")
 
+        latent = kwargs.pop("latent", None)
         self.initial_dag = dag
         self.column_mapping = {node: i for i, node in enumerate(self.initial_dag.nodes)}
         self.device = kwargs.get("device", "cuda")
@@ -48,6 +55,11 @@ class BayesianNetwork:
         self.tables: DiscreteTables = None
         self.inference_obj = None
         self._kwargs = kwargs
+        self._latent_domains = self._parse_latent(latent)
+        cfg = parameters_learning_config or {}
+        self._em_settings = {"max_iter": int(cfg.get("em_max_iter", 100)), "tol": float(cfg.get("em_tol", 1e-6)),
+                             "seed": int(cfg.get("em_seed", 0)), "pseudo_count": float(cfg.get("em_pseudo_count", 0.0))}
+        self.em_result = None
 
         self._setup_inference(inference_config)
         self._setup_parameters_learning(data, parameters_learning_config, **kwargs)
@@ -59,7 +71,27 @@ class BayesianNetwork:
             node: Node(node, estimator_name, config, self.get_parents(self.initial_dag, node), **kwargs)
             for node in self.initial_dag.nodes
         }
-        self._train(data, self.initial_dag.nodes)
+        if self._latent_domains:
+            self.fit_em(data, **self._em_settings)
+        else:
+            self._train(data, self.initial_dag.nodes)
+
+    def _parse_latent(self, latent) -> Dict[str, torch.Tensor]:
+        """name -> sorted float32 domain of every declared latent node."""
+        out = {}
+        for name, spec in (latent or {}).items():
+            if name not in self.initial_dag.nodes:
+                raise ValueError(f"latent node {name!r} is not a node of the network")
+            if isinstance(spec, (int, np.integer)):
+                if not 1 <= int(spec) <= 255:
+                    raise ValueError(f"latent node {name!r} has cardinality {int(spec)}; the discrete path supports 1..255")
+                vals = np.arange(int(spec), dtype=np.float32)
+            else:
+                vals = np.unique(np.asarray(spec, dtype=np.float32).reshape(-1))
+                if np.isnan(vals).any() or vals.size != len(spec) or not 1 <= vals.size <= 255:
+                    raise ValueError(f"latent node {name!r}: the domain must be 1..255 distinct values, not NaN")
+            out[name] = torch.from_numpy(vals)
+        return out
 
     def _setup_inference(self, config: Dict):
         self.inference_obj_name = config["inference_obj"]
@@ -67,10 +99,16 @@ class BayesianNetwork:
 
     def save_model(self, path: str):
         """One file with every count table and domain (the reference's version calls a method that
-        does not exist, bayesian_network.py:78-80)."""
+        does not exist, bayesian_network.py:78-80).  An EM fit also stores its CPTs, expected counts, hidden nodes and
+        EM settings: its CPTs are not a function of the counts."""
         t = self.tables
-        torch.save({"names": t.names, "parents": t.parents, "domains": [d.cpu() for d in t.domains],
-                    "counts": t.counts.cpu(), "n_total": t.n_total}, path)
+        sd = {"names": t.names, "parents": t.parents, "domains": [d.cpu() for d in t.domains],
+              "counts": t.counts.cpu(), "n_total": t.n_total}
+        if t.hidden:
+            sd.update({"cond": t.cond.cpu(), "joint": t.joint.cpu(), "expected_counts": t.expected_counts.cpu(),
+                       "hidden": sorted(t.names[v] for v in t.hidden), "em_settings": dict(self._em_settings),
+                       "latent": {n: d.cpu() for n, d in self._latent_domains.items()}})
+        torch.save(sd, path)
 
     def load_model(self, path: str):
         sd = torch.load(path)
@@ -79,7 +117,17 @@ class BayesianNetwork:
         self.tables.set_domains(sd["domains"])
         self.tables.counts.copy_(sd["counts"].to(self.tables.device))
         self.tables.n_total = int(sd["n_total"])
-        self.tables.finalize()
+        if "cond" in sd:                 # an EM fit: the CPTs are stored, not derived from the counts
+            t = self.tables
+            t.set_cond(sd["cond"].to(t.device))
+            t.joint = sd["joint"].to(t.device)
+            t.expected_counts = sd["expected_counts"].to(t.device)
+            t.hidden = {t.index[n] for n in sd["hidden"]}
+            self._em_settings = dict(sd["em_settings"])
+            self._latent_domains = {n: d.clone() for n, d in sd["latent"].items()}
+        else:
+            self.tables.hidden, self.tables.expected_counts = set(), None
+            self.tables.finalize()
         self._attach_all()
 
     # ------------------------------------------------------------------ graph helpers
@@ -146,7 +194,14 @@ class BayesianNetwork:
     def update_knowledge(self, data, accumulate: bool = False):
         """Re-fit on ``data`` (the reference REPLACES the tables: brute_force.py:47).  With
         ``accumulate=True`` the new samples are added to the existing int64 count tables instead
-        (values outside the fitted domains raise ValueError)."""
+        (values outside the fitted domains raise ValueError).  A network with latent nodes is re-fitted by ``fit_em`` with
+        its stored settings; it cannot accumulate (its expected counts depend on the parameters)."""
+        if self._latent_domains or (self.tables is not None and self.tables.hidden):
+            if accumulate:
+                raise ValueError("a network with latent nodes cannot accumulate counts: its expected counts depend on the "
+                                 "parameters; update_knowledge(data) re-fits it by EM")
+            self.fit_em(data, **self._em_settings)
+            return
         if not accumulate:
             self._train(data)
             return
@@ -155,6 +210,81 @@ class BayesianNetwork:
         self.tables.count(codes, int(next(iter(cols.values())).numel()))
         self.tables.finalize()
         self._attach_all()
+
+    def fit_em(self, data, max_iter: int = 100, tol: float = 1e-6, seed: int = 0, init: str = "random",
+               pseudo_count: float = 0.0):
+        """Fit by expectation-maximisation: every node without a column in ``data`` is hidden in every row.
+
+        :param data: a DataFrame or a dict name -> values, as ``log_likelihood`` takes them; the observed domains are
+                     discovered from it, as the ordinary fit does (a re-fit, like ``update_knowledge``).  A hidden node
+                     keeps the domain the network has for it (from ``latent=`` or an earlier fit).  Every row observes
+                     the same nodes: NaN in a column raises ``ValueError`` (per-row missing values are not supported).
+        :param init: ``"random"``: every CPT with a hidden member starts from Dirichlet(1) rows drawn with ``seed``;
+                     ``"current"``: from the network's current CPTs (the data's domains must be the current ones).  Fully
+                     observed families always get their exact MLE.
+        :param pseudo_count: ``a`` of the M-step ``cond = (N + a) / sum_x (N + a)`` (N: expected counts).  With 0 the
+                     M-step is the ordinary fit's formula.
+        :return: ``EMResult`` (log-likelihood per iteration plus the final one, ``n_iter``, ``converged`` when the
+                 relative gain fell below ``tol``, ``n_dead_rows``).  The fitted CPTs are installed; ``tables.counts``
+                 holds the integer counts of the fully observed families and ``tables.expected_counts`` (float64) the
+                 expected counts of every family.
+        """
+        from .. import _native as N
+        from ..em import EM, MAX_ROWS
+
+        if getattr(self.inference_obj, "evidence_plan", None) is None:
+            raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not compute posteriors for EM")
+        if init not in ("random", "current"):
+            raise ValueError(f"init must be 'random' or 'current', got {init!r}")
+        if not pseudo_count >= 0:
+            raise ValueError("pseudo_count must not be negative")
+        cols, n_rows = self._observed_columns(data)
+        given = [n for n in cols if n in self._latent_domains]
+        if given:
+            raise ValueError(f"data has columns for the latent nodes {given}")
+        if not 0 < n_rows < MAX_ROWS:
+            raise ValueError(f"EM needs 1 .. 2^31 - 1 rows, got {n_rows}")
+        if cols and int(sum(torch.isnan(c).sum() for c in cols.values()).item()):
+            raise ValueError("an observed column holds NaN: per-row missing values are not supported (every row observes "
+                             "the same nodes; a node without a column is hidden in every row)")
+        names = list(self.initial_dag.nodes)
+        old = self.tables
+        hidden = [n for n in names if n not in cols]
+        domains = {}
+        for n in hidden:
+            if n in self._latent_domains:
+                domains[n] = self._latent_domains[n]
+            elif old is not None and old.domains[old.index[n]] is not None:
+                domains[n] = old.domains[old.index[n]]
+            else:
+                raise ValueError(f"node {n} has no column and no domain: declare it with latent=")
+        current = None
+        if init == "current":
+            if old is None or old.cond is None:
+                raise ValueError("init='current' needs a fitted network")
+            current = old.cond.clone()
+        t = DiscreteTables(names, {n: self.get_parents(self.initial_dag, n) for n in names}, device=self.device)
+        observed = [n for n in names if n in cols]
+        domains.update(zip(observed, t.discover_domains([cols[n] for n in observed])))
+        t.set_domains([domains[n] for n in names])
+        if current is not None and not all(torch.equal(a, b.to(a.device)) for a, b in zip(t.domains, old.domains)):
+            raise ValueError("init='current': the data's domains differ from the network's, so its CPTs do not apply")
+        codes = t.new_code_matrix(n_rows)
+        codes.fill_(N.UNSEEN)              # hidden rows: the count kernel skips every family with a hidden member
+        for n in observed:
+            t.encode(cols[n], t.index[n], codes[t.index[n]])
+        t.count(codes, n_rows)
+        t.hidden = {t.index[n] for n in hidden}
+        self.tables = t
+        self._attach_all()
+        em = EM(t, self.inference_obj, codes, n_rows, sorted(t.hidden))
+        em.initialise(init, seed, current)
+        result = em.fit(max_iter, tol, pseudo_count)
+        t.expected_counts = em.expected_counts()
+        self._em_settings = {"max_iter": int(max_iter), "tol": float(tol), "seed": int(seed), "pseudo_count": float(pseudo_count)}
+        self._attach_all()
+        self.em_result = result
+        return result
 
     # ------------------------------------------------------------------ queries
     def get_pdf(self, target_node: str, evidence: Dict, N_max: int = 1024) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:

@@ -54,6 +54,8 @@ class DiscreteTables:
         self._discovered = None
         self._counts_buf: Optional[torch.Tensor] = None
         self._reduced = False            # the tables hold GLOBAL counts (summed over the ranks of a sharded fit)
+        self.hidden: set = set()                     # variables fitted by EM: hidden in every row
+        self.expected_counts: Optional[torch.Tensor] = None   # float64 [total_cells]: EM's expected counts N (rows)
 
     # ------------------------------------------------------------------ layout
     def set_domains(self, domains: Sequence[torch.Tensor]):
@@ -333,6 +335,12 @@ class DiscreteTables:
             assert t.numel() == self.n_cells[i]
             self.cond[self.offsets[i]: self.offsets[i] + self.n_cells[i]] = t.to(self.device)
 
+    def set_cond(self, cond: torch.Tensor):
+        """Install a whole float32 [total_cells] conditional table (EM's M-step)."""
+        assert cond.dtype == torch.float32 and cond.numel() == self.total_cells
+        self.cond = cond
+        self._drop_log_cond()
+
     def fit_columns(self, cols: Dict[str, torch.Tensor]):
         """Full fit from float32 columns: domains, codes, counts, CPTs."""
         doms = self.discover_domains([cols[n].reshape(-1) for n in self.names])
@@ -350,6 +358,9 @@ class DiscreteTables:
         """The reference's sparse ``mle_tensor`` [M, P+2] of one family (brute_force.py:45-53)."""
         i = self.index[name]
         vs = self.family_vars(name)
+        if any(v in self.hidden for v in vs):
+            raise ValueError(f"the family of {name} has a hidden member: it was fitted by EM, not counted; its expected "
+                             "counts are in expected_counts")
         out = torch.empty((self.n_cells[i], len(vs) + 1), dtype=torch.float32, device=self.device)
         rows = torch.zeros(1, dtype=torch.int64, device=self.device)
         doms = N.ptr_array([self.domains[v].data_ptr() for v in vs])

@@ -453,6 +453,47 @@ CBN_API int cbn_psample_run(cbn_ctx* ctx, const cbn_psample_plan* plan, const ui
                             const float* log_value, uint64_t seed, int64_t first_row, int32_t n_draws, uint8_t* hidden_codes,
                             int64_t out_ld, cbn_stream stream);
 
+/* ---- expectation-maximisation: expected family counts in fixed point ------------------------------------------------
+ * The E-step of EM over a group of families that share their hidden members H = (h_1 .. h_m): for every row, the joint
+ * posterior P(H | e_row) = prod_j P(h_j | e_row, h_<j) weights the row's cell of every destination family.  Factor j is
+ * the output of a single-target posterior plan of h_j given (evidence, h_<j), run once per assignment of h_<j:
+ *     factors[j]: device float [prod_{i<j} card_i][n_rows][card_j]   (stacked cbn_ve_run_codes outputs)
+ * and for every joint configuration h (mixed radix, h_1 slowest, card_H = prod_j card_j configurations) with
+ *     w = fp32 product ((F_1 F_2) F_3) .. of the chain entries of h,
+ * cbn_ess_run adds rint(double(w) * 2^32) to acc[table_offset + o(row) + hidden_cell[h]] of every destination, where
+ * o(row) = sum_k code[obs_row_k][row] * obs_stride_k over the destination's observed members.  A row whose observed code
+ * is not below the member's cardinality adds nothing to that destination; w = 0 adds nothing.  acc is the uint64 table
+ * layout of cbn_count_run (it accumulates, and a count c of a fully observed family enters as c << 32): integer sums, so
+ * the result is the same bits for any grid, chunking or batch split.  n_rows < 2^31 keeps every cell below 2^64.
+ * Nothing in the reference computes this.
+ *
+ * cbn_ess_plan_create: checks cardinalities (1..255), 1..CBN_MAX_FAMILY_VARS hidden variables, at most
+ * CBN_ESS_MAX_CONFIGS joint configurations and CBN_ESS_MAX_DESTS destinations, and that every cell a row can reach lies
+ * inside its destination's n_cells (CBN_ERR_INVALID otherwise).  hidden_cell is copied.  Uploads run on `stream`, and the
+ * function returns when it has drained.
+ * cbn_ess_run: factors: HOST array of n_hidden device pointers; codes: uint8, row c at codes + c * ld (ld >= n_rows, a
+ * multiple of 16, 16-byte aligned base).  Launched without programmatic dependent launch, so the factors may come from
+ * the kernel right before it on the stream.
+ * cbn_ess_plan_smem_dests: destinations whose tables the kernel privatises in shared memory (a prefix of the list). */
+#define CBN_ESS_MAX_DESTS 64
+#define CBN_ESS_MAX_CONFIGS 65536
+typedef struct cbn_ess_plan cbn_ess_plan;
+typedef struct cbn_ess_dest {
+  int64_t table_offset;                      /* first cell of the family's table in acc */
+  int64_t n_cells;                           /* cells of that table */
+  int32_t n_obs;                             /* observed members */
+  int32_t obs_row[CBN_MAX_FAMILY_VARS];      /* their rows in the code matrix */
+  int32_t obs_card[CBN_MAX_FAMILY_VARS];     /* their cardinalities */
+  int32_t obs_stride[CBN_MAX_FAMILY_VARS];   /* their strides in the table */
+  const int32_t* hidden_cell;                /* HOST int32 [card_H]: cell offset of joint hidden configuration h */
+} cbn_ess_dest;
+CBN_API int cbn_ess_plan_create(cbn_ctx* ctx, int32_t n_hidden, const int32_t* hidden_card, const cbn_ess_dest* dests,
+                                int32_t n_dests, cbn_stream stream, cbn_ess_plan** out);
+CBN_API void cbn_ess_plan_destroy(cbn_ess_plan* plan);
+CBN_API int cbn_ess_run(cbn_ctx* ctx, const cbn_ess_plan* plan, const float* const* factors, const uint8_t* codes, int64_t ld,
+                        int64_t n_rows, unsigned long long* acc, cbn_stream stream);
+CBN_API int cbn_ess_plan_smem_dests(const cbn_ess_plan* plan);
+
 /* ---- ancestral sampling (synthetic workloads; BruteForce._sample's network analogue,
  * brute_force.py:246-265).  Counter-based: sample i of variable v depends only on
  * (seed, first_sample + i, v), so any sharding of the sample range yields the same data.
