@@ -27,6 +27,14 @@ struct cbn_ctx {
   cudaMemPool_t pool = nullptr;
 };
 
+// Staging of the host-buffer entry points (ve.cu, count.cu).  cbn_ensure_io creates the two internal streams and events
+// and grows the device and pinned input / output buffers of both to at least in_bytes / out_bytes.  cbn_h2d_columns copies
+// rows [r0, r0 + m) of n_cols host columns (leading dimension ld) into io_dev_in[b] (leading dimension chunk) on
+// io_stream[b]: one strided copy from pinned memory, else through io_pin_in[b].
+int cbn_ensure_io(cbn_ctx* ctx, size_t in_bytes, size_t out_bytes);
+int cbn_h2d_columns(cbn_ctx* ctx, int b, const uint8_t* host, int64_t ld, int64_t r0, int64_t m, int n_cols, int64_t chunk,
+                    bool pinned);
+
 // stream-ordered scratch allocation from the context's pool
 static inline cudaError_t cbn_scratch_alloc(cbn_ctx* ctx, void** ptr, size_t bytes, cudaStream_t s) {
   return ctx->pool ? cudaMallocFromPoolAsync(ptr, bytes, ctx->pool, s) : cudaMallocAsync(ptr, bytes, s);

@@ -819,27 +819,13 @@ extern "C" int cbn_count_run_host(cbn_ctx* ctx, const cbn_count_plan* plan, cons
   // ~32 MB per chunk (at least 64K samples, a multiple of the largest tile so only the last chunk has a tail)
   int64_t chunk = std::max<int64_t>(1 << 16, (int64_t(32) << 20) / std::max(n_cols, 1));
   chunk = std::min<int64_t>((chunk + 8191) & ~int64_t(8191), (n + 8191) & ~int64_t(8191));
-  for (int i = 0; i < 2; ++i) {
-    if (!ctx->io_stream[i]) CBN_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->io_stream[i], cudaStreamNonBlocking));
-  }
-  const size_t need = size_t(chunk) * n_cols;
-  if (need > ctx->io_in_bytes) {
-    for (int i = 0; i < 2; ++i) {
-      if (ctx->io_dev_in[i]) cudaFree(ctx->io_dev_in[i]);
-      if (ctx->io_pin_in[i]) cudaFreeHost(ctx->io_pin_in[i]);
-      ctx->io_dev_in[i] = nullptr; ctx->io_pin_in[i] = nullptr;
-      CBN_CUDA(ctx, cudaMalloc(&ctx->io_dev_in[i], need));
-      CBN_CUDA(ctx, cudaMallocHost(&ctx->io_pin_in[i], need));
-    }
-    ctx->io_in_bytes = need;
-  }
+  int rc = cbn_ensure_io(ctx, size_t(chunk) * n_cols, 0);
+  if (rc) return rc;
   cudaPointerAttributes attr{};
   const bool pinned = cudaPointerGetAttributes(&attr, codes_host) == cudaSuccess && attr.type == cudaMemoryTypeHost;
   cudaGetLastError();
   // the counts may still be in use by work queued on the caller's stream: the internal streams wait for an event
   // recorded there (no device-wide synchronisation)
-  for (int i = 0; i < 2; ++i)
-    if (!ctx->io_event[i]) CBN_CUDA(ctx, cudaEventCreateWithFlags(&ctx->io_event[i], cudaEventDisableTiming));
   CBN_CUDA(ctx, cudaEventRecord(ctx->io_event[0], (cudaStream_t)stream));
   for (int i = 0; i < 2; ++i) CBN_CUDA(ctx, cudaStreamWaitEvent(ctx->io_stream[i], ctx->io_event[0], 0));
   int b = 0;
@@ -847,14 +833,8 @@ extern "C" int cbn_count_run_host(cbn_ctx* ctx, const cbn_count_plan* plan, cons
     const int64_t m = std::min(chunk, n - s0);
     cudaStream_t s = ctx->io_stream[b];
     CBN_CUDA(ctx, cudaStreamSynchronize(s));       // the staging buffer's previous chunk has been counted
-    uint8_t* din = (uint8_t*)ctx->io_dev_in[b];
-    if (pinned) {
-      CBN_CUDA(ctx, cudaMemcpy2DAsync(din, size_t(chunk), codes_host + s0, size_t(ld), size_t(m), size_t(n_cols), cudaMemcpyHostToDevice, s));
-    } else {
-      for (int c = 0; c < n_cols; ++c) memcpy((uint8_t*)ctx->io_pin_in[b] + int64_t(c) * chunk, codes_host + int64_t(c) * ld + s0, m);
-      CBN_CUDA(ctx, cudaMemcpyAsync(din, ctx->io_pin_in[b], need, cudaMemcpyHostToDevice, s));
-    }
-    int rc = cbn_count_run(ctx, plan, din, chunk, m, counts, (cbn_stream)s);
+    rc = cbn_h2d_columns(ctx, b, codes_host, ld, s0, m, n_cols, chunk, pinned);
+    if (!rc) rc = cbn_count_run(ctx, plan, (const uint8_t*)ctx->io_dev_in[b], chunk, m, counts, (cbn_stream)s);
     if (rc) return rc;
   }
   for (int i = 0; i < 2; ++i) CBN_CUDA(ctx, cudaStreamSynchronize(ctx->io_stream[i]));

@@ -7,6 +7,7 @@
 
 #include <algorithm>
 #include <new>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -924,12 +925,13 @@ __global__ void __launch_bounds__(GATHER_TPB) gather_tiles_kernel(const unsigned
                                                                   int n_stages, int hints, const uint8_t* __restrict__ ev, int64_t ld,
                                                                   int64_t n_rows, int early_ev, const __grid_constant__ GatherOuts outs) {
   constexpr int GT_TILE_ROWS = 4 * GATHER_TPB * GT_QPT;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
+  // a name of its own: extern __shared__ arrays of one name share one alignment, that of the first declaration compiled
+  extern __shared__ __align__(128) unsigned char tile_smem[];
   __shared__ __align__(8) uint64_t full[GT_MAX_STAGES], empty[GT_MAX_STAGES];
   pdl_trigger();
-  stage_blob(blob, blob_bytes, smem_raw);
+  stage_blob(blob, blob_bytes, tile_smem);
   if (!early_ev) pdl_wait();     // the evidence may have been written by the previous kernel of the stream
-  GTable* st = reinterpret_cast<GTable*>(smem_raw);
+  GTable* st = reinterpret_cast<GTable*>(tile_smem);
   // descriptors address evidence slots; inside this kernel they address staged tile columns
   for (int i = threadIdx.x; i < n_tables * GATHER_MAX_TABLE_EV; i += blockDim.x) {
     GTable& T = st[i / GATHER_MAX_TABLE_EV];
@@ -945,8 +947,8 @@ __global__ void __launch_bounds__(GATHER_TPB) gather_tiles_kernel(const unsigned
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
-  const float* pool = reinterpret_cast<const float*>(smem_raw + desc_bytes);
-  unsigned char* stages = smem_raw + ((blob_bytes + 127) & ~127);
+  const float* pool = reinterpret_cast<const float*>(tile_smem + desc_bytes);
+  unsigned char* stages = tile_smem + ((blob_bytes + 127) & ~127);
   // L2 policy: the streams (codes in, posteriors out) are touched once, the tables are what should stay resident
   uint64_t pol_first, pol_last;
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol_first));
@@ -1297,63 +1299,77 @@ int gather_blocks(cbn_ctx* ctx, int64_t n_rows, int per_sm) {
   const int64_t nquads = (n_rows + 3) >> 2;
   return (int)balanced_grid((nquads + GATHER_TPB - 1) / GATHER_TPB, int64_t(ctx->sm_count) * per_sm);
 }
-template <int CT, bool LOGEV = false>
-int launch_codes(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, const GatherOuts& outs,
-                 cudaStream_t s) {
+// A kernel's dynamic shared-memory limit, set once per device.  The template parameter is the kernel itself, so every
+// instantiation keeps its own flags.
+template <auto K>
+int set_smem_limit(cbn_ctx* ctx, int bytes) {
   static bool attr_set[64] = {};
   if (!attr_set[ctx->device & 63]) {
-    CBN_CUDA(ctx, cudaFuncSetAttribute(gather_codes_kernel<CT, LOGEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+    CBN_CUDA(ctx, cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
     attr_set[ctx->device & 63] = true;
   }
-  // one wave: as many CTAs as fit (register / shared-memory bound), the rest of the rows by the grid-stride loop
-  const int slot = LOGEV ? 2 : 0;
-  if (p->occ[slot] == 0 || p->occ_smem[slot] != p->blob_bytes) {   // resident CTAs per SM for this plan (queried once)
+  return CBN_OK;
+}
+// ... and its resident CTAs per SM at `smem` bytes, queried once per plan and footprint (slot: see cbn_ve_plan::occ)
+template <auto K>
+int resident_ctas(cbn_ctx* ctx, const cbn_ve_plan* p, int slot, int smem_limit, size_t smem, int* per_sm) {
+  int rc = set_smem_limit<K>(ctx, smem_limit);
+  if (rc) return rc;
+  if (p->occ[slot] == 0 || p->occ_smem[slot] != smem) {
     int occ = 1;
-    CBN_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gather_codes_kernel<CT, LOGEV>, GATHER_TPB, p->blob_bytes));
-    p->occ[slot] = std::max(occ, 1); p->occ_smem[slot] = p->blob_bytes;
+    CBN_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, K, GATHER_TPB, smem));
+    p->occ[slot] = std::max(occ, 1); p->occ_smem[slot] = smem;
   }
-  const int per_sm = p->occ[slot];
+  *per_sm = p->occ[slot];
+  return CBN_OK;
+}
+
+// card_t 1..GATHER_MAX_CT (checked by the caller) as a compile-time constant: f(std::integral_constant<int, CT>{})
+template <int CT = 1, typename F>
+int with_card_t(int ct, F&& f) {
+  if constexpr (CT < GATHER_MAX_CT)
+    if (ct != CT) return with_card_t<CT + 1>(ct, f);
+  return f(std::integral_constant<int, CT>{});
+}
+// the (card_t, targets) pairs that cbn_ve_plan_fuse interleaves: f(integral_constant CT, integral_constant NOUT)
+template <typename F>
+int with_interleaved(cbn_ctx* ctx, int ct, int n_out, F&& f) {
+  using C2 = std::integral_constant<int, 2>;
+  switch (ct * 10 + n_out) {
+    case 22: return f(C2{}, C2{});
+    case 23: return f(C2{}, std::integral_constant<int, 3>{});
+    case 24: return f(C2{}, std::integral_constant<int, 4>{});
+    case 32: return f(std::integral_constant<int, 3>{}, C2{});
+    case 42: return f(std::integral_constant<int, 4>{}, C2{});
+    default: return cbn_fail(ctx, CBN_ERR_UNSUPPORTED, "internal: interleaved plan %d x %d", ct, n_out);
+  }
+}
+
+// direct launches: one wave of as many CTAs as fit (register / shared-memory bound), the rest of the rows by the
+// grid-stride loop
+template <int CT, bool LOGEV>
+int launch_codes(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, const GatherOuts& outs,
+                 cudaStream_t s) {
+  int per_sm = 1;
+  int rc = resident_ctas<gather_codes_kernel<CT, LOGEV>>(ctx, p, LOGEV ? 2 : 0, 100 * 1024, p->blob_bytes, &per_sm);
+  if (rc) return rc;
   CBN_CUDA(ctx, launch_pdl(gather_codes_kernel<CT, LOGEV>, gather_blocks(ctx, n_rows, per_sm), GATHER_TPB, p->blob_bytes, s,
                            p->d_blob, (int)p->blob_bytes, (int)p->desc_bytes, p->n_tables, ev, ld, n_rows, p->static_evidence, outs));
   return CBN_OK;
 }
-template <int CT>
-int launch_f32(cbn_ctx* ctx, const cbn_ve_plan* p, const EvPtrs& evp, size_t dom_floats, int64_t n_rows, const GatherOuts& outs,
-               cudaStream_t s) {
-  static bool attr_set[64] = {};
-  if (!attr_set[ctx->device & 63]) {
-    CBN_CUDA(ctx, cudaFuncSetAttribute(gather_f32_kernel<CT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-    attr_set[ctx->device & 63] = true;
-  }
-  size_t smem = p->blob_bytes + dom_floats * 4;
-  int per_sm = (int)std::max<size_t>(1, std::min<size_t>(4, (200 * 1024) / (smem + 1024)));
-  gather_f32_kernel<CT><<<gather_blocks(ctx, n_rows, per_sm), GATHER_TPB, smem, s>>>(
-      p->d_blob, (int)p->blob_bytes, (int)p->desc_bytes, p->n_tables, evp, p->n_evidence, n_rows, outs);
-  CBN_CHECK_LAUNCH(ctx);
-  return CBN_OK;
-}
-
 template <int CT, int NOUT>
 int launch_inter(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, const GatherOuts& outs,
                  cudaStream_t s) {
-  static bool attr_set[64] = {};
-  if (!attr_set[ctx->device & 63]) {
-    CBN_CUDA(ctx, cudaFuncSetAttribute(gather_inter_kernel<CT, NOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-    attr_set[ctx->device & 63] = true;
-  }
-  if (p->occ[0] == 0 || p->occ_smem[0] != p->blob_bytes) {   // resident CTAs per SM for this plan (queried once)
-    int occ = 1;
-    CBN_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gather_inter_kernel<CT, NOUT>, GATHER_TPB, p->blob_bytes));
-    p->occ[0] = std::max(occ, 1); p->occ_smem[0] = p->blob_bytes;
-  }
-  const int per_sm = p->occ[0];
+  int per_sm = 1;
+  int rc = resident_ctas<gather_inter_kernel<CT, NOUT>>(ctx, p, 0, 100 * 1024, p->blob_bytes, &per_sm);
+  if (rc) return rc;
   CBN_CUDA(ctx, launch_pdl(gather_inter_kernel<CT, NOUT>, gather_blocks(ctx, n_rows, per_sm), GATHER_TPB, p->blob_bytes, s,
                            p->d_blob, (int)p->blob_bytes, (int)p->desc_bytes, ev, ld, n_rows, p->static_evidence, outs));
   return CBN_OK;
 }
 
 // tile-staged launch: persistent CTAs, as many as fit per SM for this plan's shared-memory footprint
-template <int CT, int NOUT, int QPT, bool LOGEV = false>
+template <int CT, int NOUT, int QPT, bool LOGEV>
 int launch_tiles_q(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, const GatherOuts& outs,
                    cudaStream_t s) {
   TileCols cols{};
@@ -1376,26 +1392,17 @@ int launch_tiles_q(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_
   while (n_stages > 2 && blob_pad + n_stages * stage_bytes > 56 * 1024) --n_stages;
   const int hints = 7;     // evict-first for the code and posterior streams, evict-last for the table
   const size_t smem = blob_pad + n_stages * stage_bytes;
-  static bool attr_set[64] = {};
-  if (!attr_set[ctx->device & 63]) {
-    CBN_CUDA(ctx, cudaFuncSetAttribute(gather_tiles_kernel<CT, NOUT, QPT, LOGEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-    attr_set[ctx->device & 63] = true;
-  }
-  const int slot = LOGEV ? 3 : 1;
-  if (p->occ[slot] == 0 || p->occ_smem[slot] != smem) {
-    int occ = 1;
-    CBN_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gather_tiles_kernel<CT, NOUT, QPT, LOGEV>, GATHER_TPB, smem));
-    p->occ[slot] = std::max(occ, 1); p->occ_smem[slot] = smem;
-  }
+  int per_sm = 1;
+  int rc = resident_ctas<gather_tiles_kernel<CT, NOUT, QPT, LOGEV>>(ctx, p, LOGEV ? 3 : 1, 160 * 1024, smem, &per_sm);
+  if (rc) return rc;
   const int64_t n_tiles = (n_rows + GT_TILE_ROWS - 1) / GT_TILE_ROWS;
-  const int per_sm = p->occ[slot];
   const int blocks = (int)balanced_grid(n_tiles, int64_t(ctx->sm_count) * per_sm);
   CBN_CUDA(ctx, launch_pdl(gather_tiles_kernel<CT, NOUT, QPT, LOGEV>, blocks, GATHER_TPB, smem, s, p->d_blob, (int)p->blob_bytes,
                            (int)p->desc_bytes, p->n_tables, cols, n_stages, hints, ev, ld, n_rows, p->static_evidence, outs));
   return CBN_OK;
 }
 
-template <int CT, int NOUT>
+template <int CT, int NOUT, bool LOGEV>
 int launch_tiles(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t ld, int64_t n_rows, const GatherOuts& outs,
                  cudaStream_t s) {
   if constexpr (NOUT >= 2) {
@@ -1405,13 +1412,13 @@ int launch_tiles(cbn_ctx* ctx, const cbn_ve_plan* p, const uint8_t* ev, int64_t 
     if (qpt_env < 0) { const char* e = getenv("CBN_GATHER_QPT"); qpt_env = e ? atoi(e) : 0; }
     const int64_t big_tiles = n_rows / (4 * GATHER_TPB * GT_MAX_QPT);
     const bool two = qpt_env ? qpt_env == 2 : big_tiles >= int64_t(ctx->sm_count) * 4 * 10;
-    if (two) return launch_tiles_q<CT, NOUT, 2>(ctx, p, ev, ld, n_rows, outs, s);
+    if (two) return launch_tiles_q<CT, NOUT, 2, LOGEV>(ctx, p, ev, ld, n_rows, outs, s);
   }
-  return launch_tiles_q<CT, NOUT, 1>(ctx, p, ev, ld, n_rows, outs, s);
+  return launch_tiles_q<CT, NOUT, 1, LOGEV>(ctx, p, ev, ld, n_rows, outs, s);
 }
 
 // large batches go through the tile-staged kernel (CBN_GATHER_TILES=0/1 forces the choice; default: >= 2^21 rows)
-bool use_tiles(const cbn_ve_plan* p, int64_t n_rows, bool force = false) {
+bool use_tiles(const cbn_ve_plan* p, int64_t n_rows) {
   static int mode = -2;
   if (mode == -2) { const char* e = getenv("CBN_GATHER_TILES"); mode = e ? atoi(e) : -1; }
   if (mode == 0 || p->card_t > GATHER_MAX_CT || p->n_evidence < 1) return false;
@@ -1425,52 +1432,21 @@ bool use_tiles(const cbn_ve_plan* p, int64_t n_rows, bool force = false) {
   // large tables in global memory (not staged): the tile-staged kernel carries the L2 policies that keep the table
   // resident while the streams pass through, which pays from a few hundred thousand rows on
   if (!p->staged && p->table_bytes >= (4ll << 20) && n_rows >= (int64_t(1) << 18)) return true;
-  return force || mode == 1 || n_rows >= (int64_t(1) << 21);
+  return mode == 1 || n_rows >= (int64_t(1) << 21);
 }
 
+// LOGEV: the log-evidence epilogue (cbn_ve_run_codes_log_evidence: single-target plans, card_t <= GATHER_MAX_CT)
+template <bool LOGEV = false>
 int ve_run_codes_impl(cbn_ctx* ctx, const cbn_ve_plan* plan, const uint8_t* ev_codes, int64_t ld, int64_t n_rows,
-                      const GatherOuts& outs, cudaStream_t s, bool force_tiles = false) {
-  const bool tiles = use_tiles(plan, n_rows, force_tiles);
-  if (plan->interleaved) {
-    const int key = plan->card_t * 10 + plan->interleaved;
-    if (tiles) switch (key) {
-      case 22: return launch_tiles<2, 2>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      case 23: return launch_tiles<2, 3>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      case 24: return launch_tiles<2, 4>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      case 32: return launch_tiles<3, 2>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      case 42: return launch_tiles<4, 2>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      default: break;
-    }
-    switch (key) {
-      case 22: return launch_inter<2, 2>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      case 23: return launch_inter<2, 3>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      case 24: return launch_inter<2, 4>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      case 32: return launch_inter<3, 2>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      case 42: return launch_inter<4, 2>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-      default: return cbn_fail(ctx, CBN_ERR_UNSUPPORTED, "internal: interleaved plan %d x %d", plan->card_t, plan->interleaved);
-    }
-  }
-  if (tiles) switch (plan->card_t) {
-    case 1: return launch_tiles<1, 0>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 2: return launch_tiles<2, 0>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 3: return launch_tiles<3, 0>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 4: return launch_tiles<4, 0>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 5: return launch_tiles<5, 0>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 6: return launch_tiles<6, 0>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 7: return launch_tiles<7, 0>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 8: return launch_tiles<8, 0>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    default: break;
-  }
-  switch (plan->card_t) {
-    case 1: return launch_codes<1>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 2: return launch_codes<2>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 3: return launch_codes<3>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 4: return launch_codes<4>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 5: return launch_codes<5>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 6: return launch_codes<6>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 7: return launch_codes<7>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 8: return launch_codes<8>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    default: {
+                      const GatherOuts& outs, cudaStream_t s) {
+  const bool tiles = use_tiles(plan, n_rows);
+  if constexpr (!LOGEV) {
+    if (plan->interleaved)
+      return with_interleaved(ctx, plan->card_t, plan->interleaved, [&](auto ct, auto n_out) {
+        return tiles ? launch_tiles<ct, n_out, false>(ctx, plan, ev_codes, ld, n_rows, outs, s)
+                     : launch_inter<ct, n_out>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+      });
+    if (plan->card_t > GATHER_MAX_CT) {
       int blocks = (int)std::min<int64_t>((n_rows + GATHER_TPB - 1) / GATHER_TPB, int64_t(ctx->sm_count) * 8);
       gather_codes_wide_kernel<<<blocks, GATHER_TPB, 0, s>>>(reinterpret_cast<const GTable*>(plan->d_blob), plan->n_tables,
                                                              ev_codes, ld, n_rows, plan->card_t, outs);
@@ -1478,6 +1454,17 @@ int ve_run_codes_impl(cbn_ctx* ctx, const cbn_ve_plan* plan, const uint8_t* ev_c
       return CBN_OK;
     }
   }
+  return with_card_t(plan->card_t, [&](auto ct) {
+    return tiles ? launch_tiles<ct, 0, LOGEV>(ctx, plan, ev_codes, ld, n_rows, outs, s)
+                 : launch_codes<ct, LOGEV>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+  });
+}
+
+// the evidence code matrix of the codes entry points
+int check_ev_matrix(cbn_ctx* ctx, const char* fn, const cbn_ve_plan* plan, const uint8_t* ev_codes, int64_t ld, int64_t n_rows) {
+  if (plan->n_evidence > 0 && (!ev_codes || ld < n_rows || (ld % 16) != 0 || !is_aligned(ev_codes, 16)))
+    return cbn_fail(ctx, CBN_ERR_INVALID, "%s: evidence matrix needs ld >= n_rows, ld %% 16 == 0, 16-byte aligned base", fn);
+  return CBN_OK;
 }
 
 int check_run_args(cbn_ctx* ctx, const char* fn, const cbn_ve_plan* plan, const uint8_t* ev_codes, int64_t ld, int64_t n_rows,
@@ -1485,8 +1472,8 @@ int check_run_args(cbn_ctx* ctx, const char* fn, const cbn_ve_plan* plan, const 
   if (!plan || n_rows < 0) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: bad argument", fn);
   if (n_rows == 0) return CBN_OK;            // an empty batch has no buffers to check (torch gives NULL for empty tensors)
   if (!posteriors || (plan->n_evidence > 0 && !ev_codes)) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: bad argument", fn);
-  if (plan->n_evidence > 0 && (ld < n_rows || (ld % 16) != 0 || !is_aligned(ev_codes, 16)))
-    return cbn_fail(ctx, CBN_ERR_INVALID, "%s: evidence matrix needs ld >= n_rows, ld %% 16 == 0, 16-byte aligned base", fn);
+  int rc = check_ev_matrix(ctx, fn, plan, ev_codes, ld, n_rows);
+  if (rc) return rc;
   outs->normalize_mask = plan->normalize_mask;
   outs->log_space = plan->log_space;
   for (int o = 0; o < plan->n_out; ++o) {
@@ -2230,8 +2217,8 @@ extern "C" int cbn_ve_run_codes_log_evidence(cbn_ctx* ctx, const cbn_ve_plan* pl
     return cbn_fail(ctx, CBN_ERR_UNSUPPORTED, "%s: needs a single-target plan with at most %d target values", fn, GATHER_MAX_CT);
   if (n_rows == 0) return CBN_OK;
   if (!log_out) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: log_out is NULL", fn);
-  if (plan->n_evidence > 0 && (!ev_codes || ld < n_rows || (ld % 16) != 0 || !is_aligned(ev_codes, 16)))
-    return cbn_fail(ctx, CBN_ERR_INVALID, "%s: evidence matrix needs ld >= n_rows, ld %% 16 == 0, 16-byte aligned base", fn);
+  int rc = check_ev_matrix(ctx, fn, plan, ev_codes, ld, n_rows);
+  if (rc) return rc;
   DeviceGuard g(ctx->device);
   cudaStream_t s = (cudaStream_t)stream;
   if (plan->kind == 1) return ve_run_rows_t<true, true>(ctx, plan, ev_codes, ld, n_rows, log_out, s);
@@ -2239,26 +2226,29 @@ extern "C" int cbn_ve_run_codes_log_evidence(cbn_ctx* ctx, const cbn_ve_plan* pl
   outs.out[0] = log_out;
   outs.normalize_mask = 0;
   outs.log_space = 1;
-  if (use_tiles(plan, n_rows)) switch (plan->card_t) {
-    case 1: return launch_tiles_q<1, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 2: return launch_tiles_q<2, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 3: return launch_tiles_q<3, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 4: return launch_tiles_q<4, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 5: return launch_tiles_q<5, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 6: return launch_tiles_q<6, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 7: return launch_tiles_q<7, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    default: return launch_tiles_q<8, 0, 1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+  return ve_run_codes_impl<true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
+}
+
+// float evidence columns: their check, then one gather_f32_kernel launch (the callers have checked card_t <= GATHER_MAX_CT)
+static int ve_run_f32_impl(cbn_ctx* ctx, const char* fn, const cbn_ve_plan* plan, const float* const* ev_cols,
+                           const float* const* domains, int64_t n_rows, const GatherOuts& outs, cudaStream_t s) {
+  EvPtrs evp{};
+  size_t dom_floats = 0;
+  for (int e = 0; e < plan->n_evidence; ++e) {
+    if (!ev_cols[e] || !domains[e]) return cbn_fail(ctx, CBN_ERR_INVALID, "%s: evidence column %d is NULL", fn, e);
+    evp.col[e] = ev_cols[e]; evp.dom[e] = domains[e]; evp.card[e] = plan->ev_cards[e];
+    dom_floats += plan->ev_cards[e];
   }
-  switch (plan->card_t) {
-    case 1: return launch_codes<1, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 2: return launch_codes<2, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 3: return launch_codes<3, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 4: return launch_codes<4, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 5: return launch_codes<5, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 6: return launch_codes<6, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    case 7: return launch_codes<7, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-    default: return launch_codes<8, true>(ctx, plan, ev_codes, ld, n_rows, outs, s);
-  }
+  const size_t smem = plan->blob_bytes + dom_floats * 4;
+  const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(4, (200 * 1024) / (smem + 1024)));
+  return with_card_t(plan->card_t, [&](auto ct) -> int {
+    int rc = set_smem_limit<gather_f32_kernel<ct>>(ctx, 160 * 1024);
+    if (rc) return rc;
+    gather_f32_kernel<ct><<<gather_blocks(ctx, n_rows, per_sm), GATHER_TPB, smem, s>>>(
+        plan->d_blob, (int)plan->blob_bytes, (int)plan->desc_bytes, plan->n_tables, evp, plan->n_evidence, n_rows, outs);
+    CBN_CHECK_LAUNCH(ctx);
+    return CBN_OK;
+  });
 }
 
 extern "C" int cbn_ve_run_f32(cbn_ctx* ctx, const cbn_ve_plan* plan, const float* const* ev_cols,
@@ -2277,28 +2267,11 @@ extern "C" int cbn_ve_run_f32(cbn_ctx* ctx, const cbn_ve_plan* plan, const float
   if (!is_aligned(posterior, 16)) return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_ve_run_f32: posterior must be 16-byte aligned");
   if (n_rows == 0) return CBN_OK;
   DeviceGuard g(ctx->device);
-  EvPtrs evp{};
-  size_t dom_floats = 0;
-  for (int e = 0; e < plan->n_evidence; ++e) {
-    if (!ev_cols[e] || !domains[e]) return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_ve_run_f32: evidence column %d is NULL", e);
-    evp.col[e] = ev_cols[e]; evp.dom[e] = domains[e]; evp.card[e] = plan->ev_cards[e];
-    dom_floats += plan->ev_cards[e];
-  }
   GatherOuts outs{};
   outs.out[0] = posterior;
   outs.normalize_mask = plan->normalize_mask;
   outs.log_space = plan->log_space;
-  cudaStream_t s = (cudaStream_t)stream;
-  switch (plan->card_t) {
-    case 1: return launch_f32<1>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 2: return launch_f32<2>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 3: return launch_f32<3>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 4: return launch_f32<4>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 5: return launch_f32<5>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 6: return launch_f32<6>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 7: return launch_f32<7>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    default: return launch_f32<8>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-  }
+  return ve_run_f32_impl(ctx, "cbn_ve_run_f32", plan, ev_cols, domains, n_rows, outs, (cudaStream_t)stream);
 }
 
 // ---- MAP value per row (fused posterior + argmax + domain lookup) ------------------------------------------------------
@@ -2316,8 +2289,8 @@ extern "C" int cbn_ve_run_codes_map(cbn_ctx* ctx, const cbn_ve_plan* plan, const
   int rc = check_map_plan(ctx, "cbn_ve_run_codes_map", plan, target_domain, map_out, n_rows);
   if (rc) return rc;
   if (n_rows == 0) return CBN_OK;
-  if (plan->n_evidence > 0 && (!ev_codes || ld < n_rows || (ld % 16) != 0 || !is_aligned(ev_codes, 16)))
-    return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_ve_run_codes_map: evidence matrix needs ld >= n_rows, ld %% 16 == 0, 16-byte aligned base");
+  rc = check_ev_matrix(ctx, "cbn_ve_run_codes_map", plan, ev_codes, ld, n_rows);
+  if (rc) return rc;
   DeviceGuard g(ctx->device);
   GatherOuts outs{};
   outs.out[0] = map_out;
@@ -2337,33 +2310,16 @@ extern "C" int cbn_ve_run_f32_map(cbn_ctx* ctx, const cbn_ve_plan* plan, const f
   if (plan->n_evidence > CBN_MAX_EVIDENCE_PTRS)
     return cbn_fail(ctx, CBN_ERR_UNSUPPORTED, "cbn_ve_run_f32_map: more than %d evidence columns; encode them and use cbn_ve_run_codes_map", CBN_MAX_EVIDENCE_PTRS);
   DeviceGuard g(ctx->device);
-  EvPtrs evp{};
-  size_t dom_floats = 0;
-  for (int e = 0; e < plan->n_evidence; ++e) {
-    if (!ev_cols[e] || !domains[e]) return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_ve_run_f32_map: evidence column %d is NULL", e);
-    evp.col[e] = ev_cols[e]; evp.dom[e] = domains[e]; evp.card[e] = plan->ev_cards[e];
-    dom_floats += plan->ev_cards[e];
-  }
   GatherOuts outs{};
   outs.out[0] = map_out;
   outs.normalize_mask = 0;
   outs.map_domain = target_domain;
   outs.log_space = plan->log_space;
-  cudaStream_t s = (cudaStream_t)stream;
-  switch (plan->card_t) {
-    case 1: return launch_f32<1>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 2: return launch_f32<2>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 3: return launch_f32<3>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 4: return launch_f32<4>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 5: return launch_f32<5>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 6: return launch_f32<6>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    case 7: return launch_f32<7>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-    default: return launch_f32<8>(ctx, plan, evp, dom_floats, n_rows, outs, s);
-  }
+  return ve_run_f32_impl(ctx, "cbn_ve_run_f32_map", plan, ev_cols, domains, n_rows, outs, (cudaStream_t)stream);
 }
 
 // ---- host-buffer entry point: chunked, double-buffered H2D -> gather -> D2H -----------------------
-static int ensure_io(cbn_ctx* ctx, size_t in_bytes, size_t out_bytes) {
+int cbn_ensure_io(cbn_ctx* ctx, size_t in_bytes, size_t out_bytes) {
   for (int i = 0; i < 2; ++i) {
     if (!ctx->io_stream[i]) CBN_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->io_stream[i], cudaStreamNonBlocking));
     if (!ctx->io_event[i]) CBN_CUDA(ctx, cudaEventCreateWithFlags(&ctx->io_event[i], cudaEventDisableTiming));
@@ -2387,6 +2343,19 @@ static int ensure_io(cbn_ctx* ctx, size_t in_bytes, size_t out_bytes) {
       CBN_CUDA(ctx, cudaMallocHost(&ctx->io_pin_out[i], out_bytes));
     }
     ctx->io_out_bytes = out_bytes;
+  }
+  return CBN_OK;
+}
+
+int cbn_h2d_columns(cbn_ctx* ctx, int b, const uint8_t* host, int64_t ld, int64_t r0, int64_t m, int n_cols, int64_t chunk,
+                    bool pinned) {
+  uint8_t* din = (uint8_t*)ctx->io_dev_in[b];
+  if (pinned) {   // one strided copy for all columns of the chunk
+    CBN_CUDA(ctx, cudaMemcpy2DAsync(din, size_t(chunk), host + r0, size_t(ld), size_t(m), size_t(n_cols), cudaMemcpyHostToDevice,
+                                    ctx->io_stream[b]));
+  } else {
+    for (int c = 0; c < n_cols; ++c) memcpy((uint8_t*)ctx->io_pin_in[b] + int64_t(c) * chunk, host + int64_t(c) * ld + r0, m);
+    CBN_CUDA(ctx, cudaMemcpyAsync(din, ctx->io_pin_in[b], size_t(chunk) * n_cols, cudaMemcpyHostToDevice, ctx->io_stream[b]));
   }
   return CBN_OK;
 }
@@ -2447,7 +2416,7 @@ static int ve_run_codes_host_impl(cbn_ctx* ctx, const cbn_ve_plan* plan, const u
   const int ne = std::max(plan->n_evidence, 1);
   const size_t out_stride = size_t(chunk) * ct;   // floats per output inside a staging buffer
   // compact mode: the compacted rows of all outputs sit behind the full-width ones in the same device buffer
-  int rc = ensure_io(ctx, size_t(chunk) * ne, out_stride * n_out * sizeof(float) * (compact ? 2 : 1));
+  int rc = cbn_ensure_io(ctx, size_t(chunk) * ne, out_stride * n_out * sizeof(float) * (compact ? 2 : 1));
   if (rc) return rc;
   // Pageable or pinned caller memory: pinned callers get direct DMA, pageable ones go through pinned staging.
   cudaPointerAttributes attr{};
@@ -2471,22 +2440,15 @@ static int ve_run_codes_host_impl(cbn_ctx* ctx, const cbn_ve_plan* plan, const u
       if (!out_pinned) drain(b);
       pending_row[b] = -1;
     }
-    uint8_t* din = (uint8_t*)ctx->io_dev_in[b];
     if (plan->n_evidence > 0) {
-      if (in_pinned) {   // one strided copy for all columns of the chunk
-        CBN_CUDA(ctx, cudaMemcpy2DAsync(din, size_t(chunk), ev_codes_host + r0, size_t(ld), size_t(m), size_t(plan->n_evidence),
-                                        cudaMemcpyHostToDevice, s));
-      } else {
-        for (int e = 0; e < plan->n_evidence; ++e)
-          memcpy((uint8_t*)ctx->io_pin_in[b] + int64_t(e) * chunk, ev_codes_host + int64_t(e) * ld + r0, m);
-        CBN_CUDA(ctx, cudaMemcpyAsync(din, ctx->io_pin_in[b], size_t(chunk) * plan->n_evidence, cudaMemcpyHostToDevice, s));
-      }
+      rc = cbn_h2d_columns(ctx, b, ev_codes_host, ld, r0, m, plan->n_evidence, chunk, in_pinned);
+      if (rc) return rc;
     }
     GatherOuts go{};
     for (int o = 0; o < n_out; ++o) go.out[o] = (float*)ctx->io_dev_out[b] + o * out_stride;
     go.normalize_mask = plan->normalize_mask;
     go.log_space = plan->log_space;
-    rc = ve_run_codes_impl(ctx, plan, din, chunk, m, go, s);
+    rc = ve_run_codes_impl(ctx, plan, (const uint8_t*)ctx->io_dev_in[b], chunk, m, go, s);
     if (rc) return rc;
     for (int o = 0; o < n_out; ++o) {
       const float* src = go.out[o];
