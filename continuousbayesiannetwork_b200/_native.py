@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(PKG, "libcbn_b200.so")
 MAX_FAMILY_VARS = 12
 MAX_CARD = 255
 UNSEEN = 255
+MISSING = 254
 MAX_CONTRACT_DIMS = 24
 MAX_CONTRACT_INPUTS = 16
 MAX_GATHER_TABLES = 16
@@ -123,6 +124,33 @@ class EssDest(C.Structure):
     ]
 
 
+JT_MAX_MEMBERS = 24
+
+
+class JtClique(C.Structure):
+    _fields_ = [
+        ("n_members", C.c_int32),
+        ("member", C.c_int32 * JT_MAX_MEMBERS),
+        ("table_offset", C.c_int64),
+    ]
+
+
+class JtOp(C.Structure):
+    _fields_ = [
+        ("kind", C.c_int32),
+        ("clique", C.c_int32),
+        ("out_size", C.c_int32),
+        ("perm", C.c_int32),
+        ("n_in", C.c_int32),
+        ("in_at", C.c_int32),
+        ("out", C.c_int32),
+        ("needed", C.c_int32),
+        ("n_out_vars", C.c_int32),
+        ("out_var", C.c_int32 * MAX_FAMILY_VARS),
+        ("table_offset", C.c_int64),
+    ]
+
+
 MPE_MAX_SLOTS = 512
 ESS_MAX_DESTS = 64
 ESS_MAX_CONFIGS = 65536
@@ -195,6 +223,12 @@ SIGNATURES = {
     "cbn_ess_plan_destroy": (None, [_P]),
     "cbn_ess_run": (C.c_int, [_P, _P, C.POINTER(_P), _P, C.c_int64, C.c_int64, _P, _P]),
     "cbn_ess_plan_smem_dests": (C.c_int, [_P]),
+    "cbn_jt_plan_create": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(JtClique), _P, C.c_int64,
+                                     C.c_int32, C.POINTER(JtOp), C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int16),
+                                     C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, C.POINTER(_P)]),
+    "cbn_jt_plan_destroy": (None, [_P]),
+    "cbn_jt_run": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, _P, _P, _P]),
+    "cbn_jt_plan_stats": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int32)]),
     "cbn_ve_run_codes_host": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P]),
     "cbn_ve_run_codes_host_multi": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P)]),
     "cbn_ve_run_codes_host_multi_ex": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P), C.c_int32]),

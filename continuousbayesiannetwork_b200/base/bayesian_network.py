@@ -17,7 +17,9 @@ or undefined, SURVEY.md section 3.3):
 * ``most_probable_explanation(data)`` gives, per row, the jointly most probable values of every node not in ``data`` and
   their log-probability ``log max_h P(h, e)`` (missing-value completion, diagnosis); the reference has no such query.
 * ``latent={"Z": k}`` / ``fit_em(data)`` fit networks with hidden nodes (no column in the data) by exact EM; the reference
-  can only fit complete data.
+  can only fit complete data.  ``fit_em(data, missing="marginalize")`` also takes NaN cells (per-row missing values).
+* ``posterior_marginals(data)`` gives every node's posterior given each row's own observed cells (NaN: not observed) and
+  ``log P`` of those cells; the reference has no such query.
 """
 from __future__ import annotations
 
@@ -38,7 +40,8 @@ class BayesianNetwork:
         """``latent``: hidden nodes, which have no column in ``data``: name -> cardinality k (domain 0.0 .. k-1) or the list
         of domain values.  With it the network is fitted by ``fit_em``, with the settings read from
         ``parameters_learning_config`` keys ``em_max_iter`` (100), ``em_tol`` (1e-6), ``em_seed`` (0) and
-        ``em_pseudo_count`` (0); ``self.em_result`` holds the ``EMResult``."""
+        ``em_pseudo_count`` (0) and ``em_missing`` ("error"; "marginalize" accepts NaN cells); ``self.em_result`` holds the
+        ``EMResult``."""
         if not nx.is_directed_acyclic_graph(dag):
             raise ValueError("The provided graph is not a directed acyclic graph (DAG).")
 
@@ -58,7 +61,8 @@ class BayesianNetwork:
         self._latent_domains = self._parse_latent(latent)
         cfg = parameters_learning_config or {}
         self._em_settings = {"max_iter": int(cfg.get("em_max_iter", 100)), "tol": float(cfg.get("em_tol", 1e-6)),
-                             "seed": int(cfg.get("em_seed", 0)), "pseudo_count": float(cfg.get("em_pseudo_count", 0.0))}
+                             "seed": int(cfg.get("em_seed", 0)), "pseudo_count": float(cfg.get("em_pseudo_count", 0.0)),
+                             "missing": str(cfg.get("em_missing", "error"))}
         self.em_result = None
 
         self._setup_inference(inference_config)
@@ -212,13 +216,23 @@ class BayesianNetwork:
         self._attach_all()
 
     def fit_em(self, data, max_iter: int = 100, tol: float = 1e-6, seed: int = 0, init: str = "random",
-               pseudo_count: float = 0.0):
+               pseudo_count: float = 0.0, missing: str = "error"):
         """Fit by expectation-maximisation: every node without a column in ``data`` is hidden in every row.
 
         :param data: a DataFrame or a dict name -> values, as ``log_likelihood`` takes them; the observed domains are
                      discovered from it, as the ordinary fit does (a re-fit, like ``update_knowledge``).  A hidden node
                      keeps the domain the network has for it (from ``latent=`` or an earlier fit).  Every row observes
-                     the same nodes: NaN in a column raises ``ValueError`` (per-row missing values are not supported).
+                     the same nodes unless ``missing="marginalize"``.
+        :param missing: ``"error"``: NaN in a column raises ``ValueError``.  ``"marginalize"``: a NaN cell is hidden in its
+                     row only (domains are discovered from the other cells; a column of NaN only raises ``ValueError``).
+                     When NaN cells are present the E-step is a junction-tree calibration per row (``cbn_jt_run``), with
+                     the rows in which a family is fully observed counted as in the ordinary fit; without NaN the E-step
+                     is the one of ``"error"``.  The log-likelihood is that of each row's observed cells.  A node with a
+                     NaN cell is then treated like a latent node by the fitted tables: it is in ``tables.hidden``, so
+                     ``mle_tensor`` refuses its families (``tables.counts`` holds only the complete rows; the expected
+                     counts are in ``tables.expected_counts``) and ``update_knowledge`` re-fits by EM with the stored
+                     settings.  With ``init="random"`` only families with a latent member start from Dirichlet(1) rows;
+                     a family with NaN cells but no latent member starts from the MLE of its complete rows.
         :param init: ``"random"``: every CPT with a hidden member starts from Dirichlet(1) rows drawn with ``seed``;
                      ``"current"``: from the network's current CPTs (the data's domains must be the current ones).  Fully
                      observed families always get their exact MLE.
@@ -230,7 +244,7 @@ class BayesianNetwork:
                  expected counts of every family.
         """
         from .. import _native as N
-        from ..em import EM, MAX_ROWS
+        from ..em import EM, JTEM, MAX_ROWS
 
         if getattr(self.inference_obj, "evidence_plan", None) is None:
             raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not compute posteriors for EM")
@@ -238,13 +252,20 @@ class BayesianNetwork:
             raise ValueError(f"init must be 'random' or 'current', got {init!r}")
         if not pseudo_count >= 0:
             raise ValueError("pseudo_count must not be negative")
+        if missing not in ("error", "marginalize"):
+            raise ValueError(f"missing must be 'error' or 'marginalize', got {missing!r}")
         cols, n_rows = self._observed_columns(data)
         given = [n for n in cols if n in self._latent_domains]
         if given:
             raise ValueError(f"data has columns for the latent nodes {given}")
         if not 0 < n_rows < MAX_ROWS:
             raise ValueError(f"EM needs 1 .. 2^31 - 1 rows, got {n_rows}")
-        if cols and int(sum(torch.isnan(c).sum() for c in cols.values()).item()):
+        nan_cells = int(sum(torch.isnan(c).sum() for c in cols.values()).item()) if cols else 0
+        if nan_cells and missing == "marginalize":
+            empty = [n for n, c in cols.items() if bool(torch.isnan(c).all().item())]
+            if empty:
+                raise ValueError(f"columns {empty} hold only NaN: they have no observed value to take a domain from")
+        if nan_cells and missing == "error":
             raise ValueError("an observed column holds NaN: per-row missing values are not supported (every row observes "
                              "the same nodes; a node without a column is hidden in every row)")
         names = list(self.initial_dag.nodes)
@@ -265,23 +286,35 @@ class BayesianNetwork:
             current = old.cond.clone()
         t = DiscreteTables(names, {n: self.get_parents(self.initial_dag, n) for n in names}, device=self.device)
         observed = [n for n in names if n in cols]
-        domains.update(zip(observed, t.discover_domains([cols[n] for n in observed])))
+        for n, d in zip(observed, t.discover_domains([cols[n] for n in observed])):
+            if nan_cells and d.numel() and bool(torch.isnan(d[-1]).item()):
+                d = d[:-1]                 # the domain kernel keeps a collapsed NaN last: a missing cell, not a value
+            if d.numel() == 0:
+                raise ValueError(f"column {n} holds only NaN: it has no observed value to take a domain from")
+            domains[n] = d
         t.set_domains([domains[n] for n in names])
         if current is not None and not all(torch.equal(a, b.to(a.device)) for a, b in zip(t.domains, old.domains)):
             raise ValueError("init='current': the data's domains differ from the network's, so its CPTs do not apply")
         codes = t.new_code_matrix(n_rows)
-        codes.fill_(N.UNSEEN)              # hidden rows: the count kernel skips every family with a hidden member
+        # hidden rows: the count kernel skips every family with a hidden member (both codes are >= every cardinality)
+        codes.fill_(N.MISSING if nan_cells else N.UNSEEN)
         for n in observed:
             t.encode(cols[n], t.index[n], codes[t.index[n]])
+            if nan_cells:
+                codes[t.index[n], :n_rows].masked_fill_(torch.isnan(cols[n]), N.MISSING)
         t.count(codes, n_rows)
         t.hidden = {t.index[n] for n in hidden}
         self.tables = t
         self._attach_all()
-        em = EM(t, self.inference_obj, codes, n_rows, sorted(t.hidden))
+        em = (JTEM if nan_cells else EM)(t, self.inference_obj, codes, n_rows, sorted(t.hidden))
+        if nan_cells:
+            # a node with a missing cell has no exact counts of its own (its families start from the complete rows' MLE)
+            t.hidden |= {t.index[n] for n in observed if bool(torch.isnan(cols[n]).any().item())}
         em.initialise(init, seed, current)
         result = em.fit(max_iter, tol, pseudo_count)
         t.expected_counts = em.expected_counts()
-        self._em_settings = {"max_iter": int(max_iter), "tol": float(tol), "seed": int(seed), "pseudo_count": float(pseudo_count)}
+        self._em_settings = {"max_iter": int(max_iter), "tol": float(tol), "seed": int(seed), "pseudo_count": float(pseudo_count),
+                             "missing": missing}
         self._attach_all()
         self.em_result = result
         return result
@@ -380,6 +413,27 @@ class BayesianNetwork:
         if mpe is None:
             raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not compute explanations")
         return mpe(cols)
+
+    def posterior_marginals(self, data, nodes: Sequence[str] = None) -> Tuple[Dict[str, torch.Tensor], torch.Tensor]:
+        """Posterior marginal of every node given each row's own observed cells, and ``log P`` of those cells: for tabular
+        data whose rows each miss different cells (imputation, per-row diagnosis, held-out scoring with gaps).
+
+        :param data: a DataFrame or a dict name -> values holding domain VALUES; NaN means "not observed in this row", and
+                     a node without a column is unobserved in every row.  A column that is not a node raises ``ValueError``.
+        :param nodes: the nodes whose marginals are returned (default: every node); the others are not written.
+        :return: ``(marginals, log_evidence)``.  ``marginals`` maps each node to float32 [n_rows, card] on the device (rows
+                 sum to 1; an observed node is one-hot); these are column views of one [n_rows, sum of the cards] buffer,
+                 not contiguous tensors (``.contiguous()`` copies one out); ``log_evidence`` is float32 [n_rows], ``log P(observed cells)``
+                 (natural log).  A value outside the fitted domain or observed cells of probability zero give -inf and NaN
+                 marginals.  With no columns the result is one row, the prior marginals.  The value of a row depends on
+                 that row only.  Exact, by a junction-tree calibration per row; a network whose junction tree is over the
+                 kernel's budgets raises ``PlanTooLarge``, and a node of cardinality 255 is refused the same way.
+        """
+        cols, _ = self._observed_columns(data)
+        marginals = getattr(self.inference_obj, "posterior_marginals", None)
+        if marginals is None:
+            raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not compute posterior marginals")
+        return marginals(cols, nodes)
 
     def sample_posterior(self, data, n_draws: int = 1, seed: int = 0,
                          first_row: int = 0) -> Tuple[Dict[str, torch.Tensor], torch.Tensor]:

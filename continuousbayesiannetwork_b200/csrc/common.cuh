@@ -161,6 +161,16 @@ __device__ __forceinline__ uint64_t splitmix64(uint64_t z) {
   return z ^ (z >> 31);
 }
 
+// Add a fixed-point weight (at most 2^32) to a privatised int64 table cell held as two 32-bit words in shared memory
+// (em.cu, jt.cu).  sm_100a has no native 64-bit shared-memory atomic add (nvcc lowers it to a load / CAS loop): the low
+// word takes ATOMS.ADD and, only when that add wraps, the high word takes the carry.
+__device__ __forceinline__ void smem_add_fixed(uint2* cell, unsigned long long v) {
+  const uint32_t lo = uint32_t(v);
+  const uint32_t old = atomicAdd(&cell->x, lo);
+  const uint32_t hi = uint32_t(v >> 32) + (old + lo < old ? 1u : 0u);
+  if (hi) atomicAdd(&cell->y, hi);
+}
+
 // ---- mbarrier + 1-D bulk async copy (TMA engine) ----------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {

@@ -41,13 +41,6 @@ struct EssChain {
   int card[ESS_MAX_H];
 };
 
-__device__ __forceinline__ void smem_add_fixed(uint2* cell, unsigned long long v) {
-  const uint32_t lo = uint32_t(v);
-  const uint32_t old = atomicAdd(&cell->x, lo);
-  const uint32_t hi = uint32_t(v >> 32) + (old + lo < old ? 1u : 0u);
-  if (hi) atomicAdd(&cell->y, hi);
-}
-
 __global__ void __launch_bounds__(ESS_TPB) ess_kernel(const __grid_constant__ EssChain chain, int m, int card_h,
                                                       const EssDest* __restrict__ dests, int n_dests,
                                                       const int* __restrict__ maps, int smem_cells,

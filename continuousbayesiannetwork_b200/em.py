@@ -13,6 +13,11 @@ Fully observed families enter the same int64 buffer as ``count << 32`` from the 
 CPT kernel with ``n_total = n_rows << 32``: fp32 division is invariant under the common power-of-two scale, so with
 complete data the CPTs are bit for bit those of the ordinary fit.
 
+With per-row missing values (``fit_em(missing="marginalize")`` on data with NaN cells) the observed set differs from row
+to row, and ``JTEM`` replaces the chain: one junction-tree calibration per row (``jt.py``, ``cbn_jt_run``) gives every
+family's posterior in each row where the family has a missing member, into the same int64 buffer, and the rows where the
+family is fully observed stay with the count kernel.  The M-step is the same.
+
 Python here loops over groups, chain steps, assignments and row chunks only: each iteration of those loops is a
 launch.  No loop touches row data.
 """
@@ -164,14 +169,9 @@ class EM:
 
     def __init__(self, tables, inference, codes: torch.Tensor, n_rows: int, hidden: Sequence[int],
                  chunk_rows: int = CHUNK_ROWS):
-        t = self.t = tables
-        self.infer = inference
-        self.codes = codes
-        self.n = int(n_rows)
-        self.hidden = sorted(set(hidden))
+        t = self._bind(tables, inference, codes, n_rows, hidden)
         self.observed = [v for v in range(len(t.names)) if v not in set(self.hidden)]
         self.groups = plan_groups(t.cards, [t.family_vars(n) for n in t.names], self.hidden)
-        self.stream = N.stream_ptr(t.device)
         self.ess = [EssPlan(t, g, self.stream) for g in self.groups]
         floats = max([chain_floats(g.hidden, t.cards) for g in self.groups], default=1)
         # chunks start on 16-row boundaries (the code matrix's alignment); the factor buffers stay below 2^30 bytes
@@ -180,9 +180,20 @@ class EM:
         self.ev = t.new_code_matrix(self.n, len(self.observed) + max(len(self.hidden), 1))
         self.ev[: len(self.observed)] = codes[self.observed, : self.ev.shape[1]]
         self.ev_names = [t.names[v] for v in self.observed]
-        # counts of the fully observed families, << 32 (the hidden families' tables hold 0: their rows were skipped)
+
+    def _bind(self, tables, inference, codes: torch.Tensor, n_rows: int, hidden: Sequence[int]):
+        """What every E-step shares: the tables, the engine, the code matrix, the hidden (latent) nodes, the stream, and
+        ``base``: the counts of the fully observed rows of every family, << 32 (the count kernel skips a row of a family
+        when a member's code is not below its cardinality)."""
+        t = self.t = tables
+        self.infer = inference
+        self.codes = codes
+        self.n = int(n_rows)
+        self.hidden = sorted(set(hidden))
+        self.stream = N.stream_ptr(t.device)
         self.base = t.allreduce_buffer()[: t.total_cells].clone() * FIXED_ONE
         self.acc = torch.empty_like(self.base)
+        return t
 
     # ------------------------------------------------------------------ E-step
     def e_step(self):
@@ -245,6 +256,10 @@ class EM:
     def expected_counts(self) -> torch.Tensor:
         return self.acc.double() / FIXED_ONE
 
+    def has_hidden(self) -> bool:
+        """Whether any family has a hidden member (else the first M-step is the fit)."""
+        return bool(self.groups)
+
     # ------------------------------------------------------------------ the loop
     def initialise(self, init: str, seed: int, current: Optional[torch.Tensor]):
         """Every family gets its complete-data MLE (exact for fully observed families, zeros for the rest); families with
@@ -273,7 +288,7 @@ class EM:
             res.log_likelihood.append(float(total.item()))
             self.m_step(pseudo_count)
             res.n_iter = it + 1
-            if not self.groups:               # complete data: the first M-step is the fit
+            if not self.has_hidden():         # complete data: the first M-step is the fit
                 res.converged = True
                 break
             if it > 0:
@@ -287,3 +302,48 @@ class EM:
         res.log_likelihood.append(float(total.item()))
         res.n_dead_rows = int(dead.item())
         return res
+
+
+class JTEM(EM):
+    """EM with per-row missing values: ``codes`` holds ``CBN_MISSING`` in every missing cell and in the rows of the
+    ``hidden`` (latent) nodes.  The E-step is one ``cbn_jt_run`` per row chunk, with the log-likelihood of the observed
+    part of each row from the same launch; the count kernel has already put the fully observed rows of every family into
+    ``base`` (it skips codes >= the cardinality, CBN_MISSING among them)."""
+
+    def __init__(self, tables, inference, codes: torch.Tensor, n_rows: int, hidden: Sequence[int],
+                 chunk_rows: int = CHUNK_ROWS):
+        t = self._bind(tables, inference, codes, n_rows, hidden)
+        self.groups = []
+        self.chunk = max(16, int(chunk_rows) // 16 * 16)
+        self.log_p = torch.empty(min(self.chunk, self.n), dtype=torch.float32, device=t.device)
+
+    def has_hidden(self) -> bool:
+        """Always: this E-step runs for data with missing cells, so some family is hidden in some row."""
+        return True
+
+    def plan(self):
+        """The junction tree of the current CPTs, with no node outputs.  After an M-step only its clique tables are
+        rebuilt: the structure and the schedule are kept by the compiler."""
+        from . import jt
+
+        return jt.compile_tree(self.infer.compiler).plan([])
+
+    def e_step(self):
+        self.acc.copy_(self.base)
+        sums = self._new_sums()
+        plan = self.plan()
+        for s in range(0, self.n, self.chunk):
+            c = min(self.chunk, self.n - s)
+            plan.run(self.codes[:, s:], c, log_out=self.log_p, acc=self.acc)
+            self._add_log_p(c, sums)
+        return sums
+
+    def _add_log_p(self, c: int, sums):
+        ll = self.log_p[:c]
+        live = ll > float("-inf")
+        sums[0].add_(torch.where(live, ll.double(), 0.0).sum())
+        sums[1].add_((~live).sum())
+
+    def _log_likelihood(self, s: int, c: int, sums):
+        self.plan().run(self.codes[:, s:], c, log_out=self.log_p)
+        self._add_log_p(c, sums)

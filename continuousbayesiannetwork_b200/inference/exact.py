@@ -150,6 +150,57 @@ class ExactInference(BaseInference):
         nh = len(plan.hidden)          # row d * nh + h of the code matrix: draw d of plan.hidden[h]
         return {t.names[v]: self._values(v, hidden[h::nh][:n_draws, :nq]) for h, v in enumerate(plan.hidden)}, log_evidence
 
+    def junction_tree(self):
+        """The network's junction tree (``jt.JunctionTree``), compiled once per set of CPTs."""
+        from .. import jt
+
+        assert self.compiler is not None, "inference engine is not bound to a fitted network"
+        return jt.compile_tree(self.compiler)
+
+    def missing_codes(self, evidence: Dict[str, torch.Tensor]):
+        """``evidence`` (name -> tensor [n_rows] or [n_rows, 1] of category VALUES, NaN: not observed in that row) as a
+        uint8 code matrix with a row per network variable: ``encode``, then NaN -> CBN_MISSING; a node without a column
+        is CBN_MISSING in every row.  Returns (codes, number of rows; 1 when there is no column)."""
+        t = self.tables
+        names = list(evidence or {})
+        cols, nq = self._columns(evidence, names, mismatch="all evidence columns must have the same number of rows")
+        codes = t.new_code_matrix(nq)
+        codes.fill_(N.MISSING)
+        for n, col in zip(names, cols):
+            v = t.index[n]
+            t.encode(col, v, codes[v])
+            codes[v, :nq].masked_fill_(torch.isnan(col), N.MISSING)
+        return codes, nq
+
+    def posterior_marginals(self, evidence: Dict[str, torch.Tensor], nodes: Optional[Sequence[str]] = None):
+        """Posterior marginal of every node (or of ``nodes``) given each row's own observed cells, and ``log P`` of those
+        cells: ``(marginals, log_evidence)``.  ``evidence``: name -> tensor [n_rows] or [n_rows, 1] of category VALUES,
+        NaN where the row does not observe the node; a node without a column is unobserved in every row.
+        ``marginals`` maps each node to float32 [n_rows, card] (an observed node is one-hot), a column view of ONE
+        float32 [n_rows, sum of the cards] buffer the kernel writes (not contiguous: ``.contiguous()`` copies a node's
+        block out; writing into a view writes that buffer); ``log_evidence`` is float32
+        [n_rows] (natural log).  A value outside the fitted domain, or observed cells of probability zero, give -inf and
+        NaN marginals.  No columns give one row, the prior marginals.  One junction-tree calibration per row
+        (``cbn_jt_run``); the value of a row depends on that row only.  Not part of the reference's surface."""
+        t = self.tables
+        if nodes is None:
+            ids = list(range(len(t.names)))
+        else:
+            for n in nodes:
+                if n not in t.index:
+                    raise ValueError(f"{n} is not a node of the network")
+            ids = [t.index[n] for n in nodes]
+            if len(set(ids)) != len(ids):
+                raise ValueError("a node is listed twice")
+        codes, nq = self.missing_codes(evidence)
+        plan = self.junction_tree().plan(ids)
+        run = plan.schedule.marg_floats
+        marg = torch.empty((nq, run), dtype=torch.float32, device=t.device)
+        log_evidence = torch.empty(nq, dtype=torch.float32, device=t.device)
+        plan.run(codes, nq, marg_out=marg if run else None, log_out=log_evidence)
+        at = plan.schedule.node_out
+        return {t.names[v]: marg[:, at[v]: at[v] + t.cards[v]] for v in ids}, log_evidence
+
     def infer_map(self, target_node: str, evidence: Dict[str, torch.Tensor]) -> Optional[torch.Tensor]:
         """MAP value of the target per row through the fused kernel (``cbn_ve_run_f32_map``); ``None`` when the plan is
         not a single-target gather plan with at most 8 target values (the caller then takes posterior + argmax)."""

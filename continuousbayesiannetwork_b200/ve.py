@@ -617,6 +617,7 @@ class VECompiler:
         self.mpe_argmax_budget = int(mpe_argmax_budget_bytes)    # argmax tables of one MPE plan, in bytes
         self.sample_table_budget = int(sample_table_budget_bytes)    # threshold tables of one posterior sampler, in bytes
         self._plans: Dict[tuple, object] = {}           # (mode, key) -> plan
+        self.structures: Dict[tuple, object] = {}       # host schedules that depend on the graph only (kept across CPTs)
         self._plans_version = None
         self._has_zero: Dict[int, bool] = {}
         self.last_row_schedule: Optional[dict] = None

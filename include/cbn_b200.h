@@ -49,6 +49,7 @@ extern "C" {
 #define CBN_MAX_FAMILY_VARS 12
 #define CBN_MAX_CARD 255
 #define CBN_UNSEEN 255
+#define CBN_MISSING 254          /* cbn_jt_run: not observed in this row (summed out); no other entry point gives it a meaning */
 #define CBN_MAX_CONTRACT_DIMS 24
 #define CBN_MAX_CONTRACT_INPUTS 16
 #define CBN_MAX_GATHER_TABLES 16
@@ -493,6 +494,70 @@ CBN_API void cbn_ess_plan_destroy(cbn_ess_plan* plan);
 CBN_API int cbn_ess_run(cbn_ctx* ctx, const cbn_ess_plan* plan, const float* const* factors, const uint8_t* codes, int64_t ld,
                         int64_t n_rows, unsigned long long* acc, cbn_stream stream);
 CBN_API int cbn_ess_plan_smem_dests(const cbn_ess_plan* plan);
+
+/* ---- junction-tree calibration per row: marginals, log P(e) and expected counts with per-row missing values ---------
+ * One structure per network (a junction tree over the moral graph; built by jt.py), calibrated per row with that row's
+ * own observed set.  Row r's codes are codes[v * ld + r] for every network variable v: a code below the cardinality is
+ * observed, CBN_MISSING is summed out, anything else (CBN_UNSEEN, a code >= the cardinality) makes the row dead.
+ *
+ * The plan is a list of cliques and a program of ops.  A clique's members are ascending network ids; its table (device
+ * float, at clique_tables + table_offset) is row-major over them, last fastest.  Every op is one product-sum over one
+ * clique c (cells(c) = out_size * fiber):
+ *     out[o] = sum_f psi[x] * ev(x) * prod_i msg[in_i.message + maps[in_i.map + x]],   x = maps[perm + o * fiber + f]
+ *                                                                                    (x = o * fiber + f when perm = -1)
+ * where ev(x) is 1 when the cell agrees with every observed member of the row, and inputs (n_in pairs of int32 at
+ * inputs + 2 * in_at) name per-row message offsets and the map of every clique cell to that message's cell.  The program
+ * is every CBN_JT_UP op (collect; the output is a message, divided by its maximum, whose log is added to the row's
+ * log-scale), one CBN_JT_ROOT op (out_size 1: log P(e) = log-scales + log Z), then CBN_JT_DOWN (distribute; a message
+ * divided by its maximum, run when `needed` has bit 1 and marginals are requested or bit 2 and counts are), CBN_JT_NODE
+ * (the marginal of out_var[0], normalised, at marg_out + row * marg_floats + out) and CBN_JT_FAMILY ops (the posterior of
+ * the family out_var[0..n_out_vars), in family-table order: each cell w = x / sum (correctly rounded) adds
+ * rint(double(w) * 2^32) to acc[table_offset + cell], only in rows where a member of the family is CBN_MISSING; a
+ * fully observed row is the count kernel's, as count << 32).  Nothing in the reference computes this.
+ *
+ * cbn_jt_plan_create: range-checks everything (cardinalities 1..CBN_MISSING - 1, ascending members, at most 32767 cells
+ * per clique, every map entry inside its clique / the messages, outputs inside their buffers; CBN_ERR_INVALID otherwise),
+ * copies the host tables and the clique tables (which may be freed after it returns), and needs the whole plan plus one
+ * row's messages (msg_floats + scratch_floats floats, scratch: the largest NODE / FAMILY output) to fit in shared memory
+ * (CBN_ERR_UNSUPPORTED otherwise).  Uploads run on `stream`, and the function returns when it has drained.
+ * cbn_jt_run: every output is nullable: marg_out float [n_rows][marg_floats] (NaN in dead rows), log_out float [n_rows]
+ * (-inf in dead rows), acc the uint64 layout of cbn_count_run / cbn_ess_run (accumulates).  A row's values depend on that
+ * row only and acc is an integer sum: any grid or batch split gives the same bits.  Launched without programmatic
+ * dependent launch.
+ * cbn_jt_plan_stats: shared memory per CTA and warps per CTA (one row per warp at a time). */
+#define CBN_JT_MAX_MEMBERS 24
+#define CBN_JT_UP 0
+#define CBN_JT_ROOT 1
+#define CBN_JT_DOWN 2
+#define CBN_JT_NODE 3
+#define CBN_JT_FAMILY 4
+typedef struct cbn_jt_plan cbn_jt_plan;
+typedef struct cbn_jt_clique {
+  int32_t n_members;
+  int32_t member[CBN_JT_MAX_MEMBERS];        /* network ids, ascending */
+  int64_t table_offset;                      /* first cell of the clique's table in clique_tables */
+} cbn_jt_clique;
+typedef struct cbn_jt_op {
+  int32_t kind;                              /* CBN_JT_* */
+  int32_t clique;
+  int32_t out_size;                          /* output cells; divides the clique's cells */
+  int32_t perm;                              /* offset in maps of the [out_size][fiber] layout, -1: identity */
+  int32_t n_in, in_at;                       /* input pairs inputs[2 * in_at ..] */
+  int32_t out;                               /* UP / DOWN: message offset; NODE: offset in the row's marginals */
+  int32_t needed;                            /* DOWN: 1 on the way to a NODE op, 2 to a FAMILY op */
+  int32_t n_out_vars;                        /* NODE: 1; FAMILY: the family's size; else 0 */
+  int32_t out_var[CBN_MAX_FAMILY_VARS];      /* NODE: the node; FAMILY: parents ..., node */
+  int64_t table_offset;                      /* FAMILY: first cell of the family's table in acc */
+} cbn_jt_op;
+CBN_API int cbn_jt_plan_create(cbn_ctx* ctx, int32_t n_vars, const int32_t* cards, int32_t n_cliques,
+                               const cbn_jt_clique* cliques, const float* clique_tables, int64_t n_table_cells, int32_t n_ops,
+                               const cbn_jt_op* ops, const int32_t* inputs, int32_t n_inputs, const int16_t* maps,
+                               int64_t n_maps, int32_t msg_floats, int32_t scratch_floats, int32_t marg_floats,
+                               cbn_stream stream, cbn_jt_plan** out);
+CBN_API void cbn_jt_plan_destroy(cbn_jt_plan* plan);
+CBN_API int cbn_jt_run(cbn_ctx* ctx, const cbn_jt_plan* plan, const uint8_t* codes, int64_t ld, int64_t n_rows,
+                       float* marg_out, float* log_out, unsigned long long* acc, cbn_stream stream);
+CBN_API int cbn_jt_plan_stats(const cbn_jt_plan* plan, int64_t* smem_bytes, int32_t* warps_per_cta);
 
 /* ---- ancestral sampling (synthetic workloads; BruteForce._sample's network analogue,
  * brute_force.py:246-265).  Counter-based: sample i of variable v depends only on
