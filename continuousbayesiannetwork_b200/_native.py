@@ -125,6 +125,7 @@ class EssDest(C.Structure):
 
 
 JT_MAX_MEMBERS = 24
+JT_DECODE_MAX, JT_DECODE_SAMPLE = 0, 1
 
 
 class JtClique(C.Structure):
@@ -229,6 +230,8 @@ SIGNATURES = {
     "cbn_jt_plan_destroy": (None, [_P]),
     "cbn_jt_run": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P, _P, _P, _P]),
     "cbn_jt_plan_stats": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int32)]),
+    "cbn_jt_decode": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.c_int32, C.c_uint64, C.c_int64, C.c_int32, _P,
+                                C.c_int64, _P, _P]),
     "cbn_ve_run_codes_host": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, _P]),
     "cbn_ve_run_codes_host_multi": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P)]),
     "cbn_ve_run_codes_host_multi_ex": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.POINTER(_P), C.c_int32]),

@@ -458,6 +458,37 @@ class BayesianNetwork:
             raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not sample posteriors")
         return sample(cols, n_draws=n_draws, seed=seed, first_row=first_row)
 
+    def impute(self, data, method: str = "mpe", n_draws: int = 1, seed: int = 0,
+               first_row: int = 0) -> Tuple[Dict[str, torch.Tensor], torch.Tensor]:
+        """Complete each row's missing cells with values that are jointly consistent: the single most probable
+        completion (``method="mpe"``) or joint draws from ``P(missing | observed)`` for multiple imputation
+        (``method="sample"``).  Unlike per-node argmaxes or draws of ``posterior_marginals``, a completion never has
+        probability zero.
+
+        :param data: a DataFrame or a dict name -> values holding domain VALUES; NaN means "not observed in this row", and
+                     a node without a column is unobserved in every row.  A column that is not a node raises ``ValueError``.
+        :param method: ``"mpe"`` or ``"sample"``; anything else raises ``ValueError``.
+        :param n_draws: draws per row for ``"sample"`` (at least 1); ``"mpe"`` takes 1 only.
+        :param seed, first_row: draw d of row i depends only on ``(seed, first_row + i, d)``, so a batch split over calls
+                     (pass each part's offset as ``first_row``) or a smaller ``n_draws`` gives the same bits.  These draws
+                     are not ``sample_posterior``'s: the two factorise the posterior differently.
+        :return: ``"mpe"``: ``(completed, log_prob)``.  ``completed`` maps EVERY node to float32 [n_rows] domain values on
+                 the device (observed cells unchanged); ``log_prob`` is float32 [n_rows], ``log max P(completion)`` over
+                 the completions of the row (natural log).  The result is checkable: ``log_likelihood(completed)`` equals
+                 ``log_prob`` within fp32 rounding.  ``"sample"``: ``(draws, log_evidence)``.  ``draws`` maps every node
+                 to float32 [n_draws, n_rows]; ``log_evidence`` is ``log P(observed cells)``, the bits of
+                 ``posterior_marginals``'.  A value outside the fitted domain or observed cells of probability zero give
+                 -inf and NaN in every column of the row (never a NaN log value).  With no columns the result is one row:
+                 the explanation of the prior, or draws from it.  The value of a row depends on that row only.  Exact, by
+                 a junction-tree pass per row; a network whose junction tree is over the kernel's budgets raises
+                 ``PlanTooLarge`` before any device work.
+        """
+        cols, _ = self._observed_columns(data)
+        impute = getattr(self.inference_obj, "impute", None)
+        if impute is None:
+            raise NotImplementedError(f"inference engine {self.inference_obj_name!r} does not impute")
+        return impute(cols, method=method, n_draws=n_draws, seed=seed, first_row=first_row)
+
     def _observed_columns(self, data) -> Tuple[Dict[str, torch.Tensor], int]:
         """``_columns`` for a subset of the nodes: (name -> float32 device column, number of rows)."""
         dev = self.device

@@ -23,6 +23,10 @@
 // a fixed shuffle tree.  Every sum has a fixed order, so a row's values depend on that row only, and the counts are
 // integer sums: any grid or batch split gives the same bits.  Family tables are privatised in shared memory with the
 // split 32-bit carry of the ESS kernel (smem_add_fixed).
+//
+// jt_decode_kernel (cbn_jt_decode) runs the same collect pass, with max in place of + for the most probable
+// completion, then decodes the cliques top-down: each clique's unobserved members are fixed by argmax or by one
+// inverse-CDF draw over its cells' collect terms, given the values fixed above it (rules in cbn_b200.h).
 #include <algorithm>
 #include <cmath>
 #include <new>
@@ -74,11 +78,16 @@ struct JtView {
   const float* psi;
   const int16_t* maps;
   const uint8_t* dig;
-  const uint8_t* tile;                                // [n_vars][JT_TILE]
+  uint8_t* tile;                                      // [n_vars][JT_TILE]; the decode fixes values in its row's column
   int k;                                              // the row's column in the tile
 };
 
+// the fiber reduction of an op: + (sum-product: calibration, log P(e), sampling) or max (max-product: MPE)
+template <bool MAX>
+__device__ __forceinline__ float jt_reduce(float a, float b) { return MAX ? fmaxf(a, b) : __fadd_rn(a, b); }
+
 // out[o] for every output cell of op o (into shared memory); ends with __syncwarp
+template <bool MAX = false>
 __device__ __forceinline__ void jt_products(const JtView& V, const JtOpD& o, const float* msg, float* out, int lane) {
   const JtCl q = V.cl[o.clique];
   const int lpo = o.out_size >= 32 ? 1 : (1 << (31 - __clz(32 / o.out_size)));
@@ -103,10 +112,10 @@ __device__ __forceinline__ void jt_products(const JtView& V, const JtOpD& o, con
           const int2 e = V.in[o.in_at + i];
           v = __fmul_rn(v, msg[e.x + V.maps[e.y + c]]);
         }
-        s = __fadd_rn(s, v);
+        s = jt_reduce<MAX>(s, v);
       }
     }
-    for (int off = lpo >> 1; off > 0; off >>= 1) s = __fadd_rn(s, __shfl_xor_sync(FULL, s, off));
+    for (int off = lpo >> 1; off > 0; off >>= 1) s = jt_reduce<MAX>(s, __shfl_xor_sync(FULL, s, off));
     if (sub == 0 && oc < o.out_size) out[oc] = s;
   }
   __syncwarp();
@@ -129,6 +138,35 @@ __device__ __forceinline__ float jt_warp_sum(const float* x, int n, int lane) {
 __device__ __forceinline__ void jt_divide(float* x, int n, float d, int lane) {
   for (int i = lane; i < n; i += 32) x[i] = __fdiv_rn(x[i], d);
   __syncwarp();
+}
+
+// a code neither below the cardinality nor CBN_MISSING makes the row dead
+__device__ __forceinline__ bool jt_row_dead(const JtView& V, int n_vars, int lane) {
+  bool bad = false;
+  for (int v = lane; v < n_vars; v += 32) {
+    const int c = V.tile[v * JT_TILE + V.k];
+    bad |= !(c < V.cards[v] || c == CBN_MISSING);
+  }
+  return __any_sync(FULL, bad);
+}
+
+// the collect pass of one row: every UP op (a message divided by its maximum) and the ROOT op, sum- or max-product.
+// Adds the log of every maximum and of the ROOT value to logp and leaves i at the first op after ROOT; false (with i at
+// the failing op) when a maximum or the ROOT value is 0
+template <bool MAX = false>
+__device__ __forceinline__ bool jt_collect(const JtView& V, int n_ops, float* msg, float* scratch, int lane, int& i,
+                                           float& logp) {
+  for (; i < n_ops; ++i) {
+    const JtOpD& o = V.ops[i];
+    if (o.kind > CBN_JT_ROOT) break;
+    float* dst = o.kind == CBN_JT_UP ? msg + o.out : scratch;
+    jt_products<MAX>(V, o, msg, dst, lane);
+    const float mx = o.kind == CBN_JT_UP ? jt_warp_max(dst, o.out_size, lane) : dst[0];
+    if (!(mx > 0.0f)) return false;
+    if (o.kind == CBN_JT_UP) jt_divide(dst, o.out_size, mx, lane);
+    logp += logf(mx);
+  }
+  return true;
 }
 
 __global__ void __launch_bounds__(JT_MAX_WARPS * 32) jt_kernel(const __grid_constant__ JtArgs a) {
@@ -164,26 +202,10 @@ __global__ void __launch_bounds__(JT_MAX_WARPS * 32) jt_kernel(const __grid_cons
     for (int k = warp; k < JT_TILE && base + k < a.n; k += warps) {
       const int64_t r = base + k;
       V.k = k;
-      bool bad = false;
-      for (int v = lane; v < a.n_vars; v += 32) {
-        const int c = tile[v * JT_TILE + k];
-        bad |= !(c < V.cards[v] || c == CBN_MISSING);
-      }
-      bad = __any_sync(FULL, bad);
+      bool bad = jt_row_dead(V, a.n_vars, lane);
       float logp = 0.0f;
       int i = 0;
-      if (!bad) {
-        for (; i < a.n_ops; ++i) {
-          const JtOpD& o = V.ops[i];
-          if (o.kind > CBN_JT_ROOT) break;
-          float* dst = o.kind == CBN_JT_UP ? msg + o.out : scratch;
-          jt_products(V, o, msg, dst, lane);
-          const float mx = o.kind == CBN_JT_UP ? jt_warp_max(dst, o.out_size, lane) : dst[0];
-          if (!(mx > 0.0f)) { bad = true; break; }
-          if (o.kind == CBN_JT_UP) jt_divide(dst, o.out_size, mx, lane);
-          logp += logf(mx);
-        }
-      }
+      if (!bad) bad = !jt_collect(V, a.n_ops, msg, scratch, lane, i, logp);
       if (a.logp && lane == 0) a.logp[r] = bad ? -INFINITY : logp;
       if (bad) {
         if (a.marg)
@@ -240,6 +262,154 @@ __global__ void __launch_bounds__(JT_MAX_WARPS * 32) jt_kernel(const __grid_cons
   }
 }
 
+
+// ---- decoding: the most probable completion (MAX) or joint posterior draws (SAMPLE) of the row's missing cells ----------
+struct JtDecodeArgs {
+  JtArgs a;                                           // a.logp: log_out
+  uint8_t* out;
+  int64_t out_ld;
+  uint64_t seed;
+  int64_t first_row;
+  int n_draws;
+};
+
+// the collect term of canonical cell c of op o's clique against the row's working column (observed and fixed codes):
+// psi[c] * ev(c) * prod_k m_k[map_k[c]], multiplied in the op's input order, so it has the bits of the cell's term in
+// jt_products
+__device__ __forceinline__ float jt_cell_weight(const JtView& V, const JtOpD& o, const JtCl& q, const float* msg, int c) {
+  for (int m = 0; m < q.n_members; ++m) {
+    const int w = V.tile[V.members[q.member_at + m] * JT_TILE + V.k];
+    if (w != CBN_MISSING && V.dig[q.dig_at + m * q.cells + c] != w) return 0.0f;
+  }
+  float v = V.psi[q.psi_at + c];
+  for (int i = 0; i < o.n_in; ++i) {
+    const int2 e = V.in[o.in_at + i];
+    v = __fmul_rn(v, msg[e.x + V.maps[e.y + c]]);
+  }
+  return v;
+}
+
+// fixes the unfixed members of op o's clique in the working column: the cell of maximal weight (the smallest canonical
+// index among equals), or the first cell whose cumulative weight exceeds u * total (lane j sums the contiguous chunk
+// [j * per, (j + 1) * per), the lane totals are combined by a shuffle scan, the owning lane rescans its chunk; if rounding
+// leaves no such cell, the last cell of positive weight of the owning chunk).  false when every weight is 0
+template <int MODE>
+__device__ __forceinline__ bool jt_decode_clique(const JtView& V, const JtOpD& o, const float* msg, int lane,
+                                                 uint64_t draw_base) {
+  const JtCl q = V.cl[o.clique];
+  bool open = false;
+  for (int m = lane; m < q.n_members; m += 32) open |= V.tile[V.members[q.member_at + m] * JT_TILE + V.k] == CBN_MISSING;
+  if (!__any_sync(FULL, open)) return true;
+  int x;
+  if (MODE == CBN_JT_DECODE_MAX) {
+    float best = -1.0f;
+    x = 0;
+    for (int c = lane; c < q.cells; c += 32) {
+      const float w = jt_cell_weight(V, o, q, msg, c);
+      if (w > best) { best = w; x = c; }
+    }
+    for (int off = 16; off > 0; off >>= 1) {
+      const float ob = __shfl_xor_sync(FULL, best, off);
+      const int ox = __shfl_xor_sync(FULL, x, off);
+      if (ob > best || (ob == best && ox < x)) { best = ob; x = ox; }
+    }
+    if (!(best > 0.0f)) return false;
+  } else {
+    const int per = (q.cells + 31) / 32, c0 = min(lane * per, q.cells), c1 = min(c0 + per, q.cells);
+    float t = 0.0f;
+    for (int c = c0; c < c1; ++c) t = __fadd_rn(t, jt_cell_weight(V, o, q, msg, c));
+    float inc = t;
+    for (int off = 1; off < 32; off <<= 1) {
+      const float y = __shfl_up_sync(FULL, inc, off);
+      if (lane >= off) inc = __fadd_rn(inc, y);
+    }
+    const float up1 = __shfl_up_sync(FULL, inc, 1);
+    const float before = lane ? up1 : 0.0f;
+    const float total = __shfl_sync(FULL, inc, 31);
+    const unsigned pos = __ballot_sync(FULL, t > 0.0f);
+    if (!pos) return false;
+    const uint64_t h = splitmix64(draw_base + uint64_t(o.clique));
+    const float target = __fmul_rn(float(uint32_t(h >> 40)) * (1.0f / 16777216.0f), total);
+    const unsigned hit = __ballot_sync(FULL, inc > target && t > 0.0f);     // a tree scan: inc can grow by rounding alone
+    const int owner = hit ? __ffs(hit) - 1 : 31 - __clz(pos);
+    x = 0;
+    if (lane == owner) {
+      float cum = before;
+      int last = c0;
+      for (int c = c0; c < c1; ++c) {
+        const float w = jt_cell_weight(V, o, q, msg, c);
+        if (!(w > 0.0f)) continue;
+        last = c;
+        cum = __fadd_rn(cum, w);
+        if (cum > target) break;
+      }
+      x = last;
+    }
+    x = __shfl_sync(FULL, x, owner);
+  }
+  __syncwarp();
+  for (int m = lane; m < q.n_members; m += 32)
+    V.tile[V.members[q.member_at + m] * JT_TILE + V.k] = V.dig[q.dig_at + m * q.cells + x];
+  __syncwarp();
+  return true;
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(JT_MAX_WARPS * 32, 4) jt_decode_kernel(const __grid_constant__ JtDecodeArgs d) {
+  extern __shared__ __align__(16) unsigned char jt_smem[];
+  const JtArgs& a = d.a;
+  for (int i = threadIdx.x; i < a.blob_bytes / 16; i += blockDim.x)
+    reinterpret_cast<int4*>(jt_smem)[i] = reinterpret_cast<const int4*>(a.blob)[i];
+  __syncthreads();
+  JtView V;
+  V.ops = reinterpret_cast<const JtOpD*>(jt_smem + a.ops_at);
+  V.cl = reinterpret_cast<const JtCl*>(jt_smem + a.cl_at);
+  V.members = reinterpret_cast<const int*>(jt_smem + a.mem_at);
+  V.cards = reinterpret_cast<const int*>(jt_smem + a.cards_at);
+  V.in = reinterpret_cast<const int2*>(jt_smem + a.in_at);
+  V.psi = reinterpret_cast<const float*>(jt_smem + a.psi_at);
+  V.maps = reinterpret_cast<const int16_t*>(jt_smem + a.maps_at);
+  V.dig = jt_smem + a.dig_at;
+  uint8_t* tile = jt_smem + a.tile_at;
+  V.tile = tile;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, warps = blockDim.x >> 5;
+  float* msg = reinterpret_cast<float*>(jt_smem + a.warp_at) + size_t(warp) * a.row_floats;
+  float* scratch = msg + a.msg_floats;
+  for (int64_t base = int64_t(blockIdx.x) * JT_TILE; base < a.n; base += int64_t(gridDim.x) * JT_TILE) {
+    __syncthreads();                                          // the previous tile's rows are done
+    for (int i = threadIdx.x; i < a.n_vars * JT_TILE; i += blockDim.x) {
+      const int64_t r = base + (i % JT_TILE);
+      tile[i] = r < a.n ? a.codes[int64_t(i / JT_TILE) * a.ld + r] : uint8_t(CBN_UNSEEN);
+    }
+    __syncthreads();
+    for (int k = warp; k < JT_TILE && base + k < a.n; k += warps) {
+      const int64_t r = base + k;
+      V.k = k;
+      bool bad = jt_row_dead(V, a.n_vars, lane);
+      float logp = 0.0f;
+      int end = 0;                                            // the collect ops are [0, end): UP ..., ROOT
+      if (!bad) bad = !jt_collect<MODE == CBN_JT_DECODE_MAX>(V, a.n_ops, msg, scratch, lane, end, logp);
+      for (int dr = 0; dr < d.n_draws && !bad; ++dr) {
+        if (dr) {                                             // back to the row's own codes
+          __syncwarp();
+          for (int v = lane; v < a.n_vars; v += 32) tile[v * JT_TILE + k] = a.codes[int64_t(v) * a.ld + r];
+          __syncwarp();
+        }
+        const uint64_t draw_base = splitmix64(splitmix64(d.seed ^ (uint64_t(d.first_row + r) * 0xD1B54A32D192ED03ull)) ^
+                                              (uint64_t(dr) * 0x9E6C63D0676A9A99ull));
+        for (int j = end - 1; j >= 0 && !bad; --j) bad = !jt_decode_clique<MODE>(V, V.ops[j], msg, lane, draw_base);
+        if (bad) break;
+        for (int v = lane; v < a.n_vars; v += 32)
+          d.out[(int64_t(dr) * a.n_vars + v) * d.out_ld + r] = tile[v * JT_TILE + k];
+      }
+      if (a.logp && lane == 0) a.logp[r] = bad ? -INFINITY : logp;
+      if (bad)
+        for (int dr = 0; dr < d.n_draws; ++dr)
+          for (int v = lane; v < a.n_vars; v += 32) d.out[(int64_t(dr) * a.n_vars + v) * d.out_ld + r] = CBN_UNSEEN;
+    }
+  }
+}
+
 size_t align16(size_t x) { return (x + 15) / 16 * 16; }
 }  // namespace
 
@@ -250,6 +420,7 @@ struct cbn_jt_plan {
   size_t smem = 0;
   int warps = 0;
   int per_sm = 1;
+  int per_sm_decode[2] = {1, 1};                      // CTAs per SM of jt_decode_kernel<MAX> and <SAMPLE>
 };
 
 extern "C" void cbn_jt_plan_destroy(cbn_jt_plan* p) {
@@ -419,8 +590,19 @@ extern "C" int cbn_jt_plan_create(cbn_ctx* ctx, int32_t n_vars, const int32_t* c
   // with a smaller footprint does not lower it below what an earlier (cached) plan launches with
   if (e == cudaSuccess) e = cudaFuncSetAttribute(jt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)optin);
   if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&p->per_sm, jt_kernel, warps * 32, p->smem);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(jt_decode_kernel<CBN_JT_DECODE_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)optin);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(jt_decode_kernel<CBN_JT_DECODE_SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)optin);
+  if (e == cudaSuccess)
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&p->per_sm_decode[0], jt_decode_kernel<CBN_JT_DECODE_MAX>, warps * 32,
+                                                      p->smem);
+  if (e == cudaSuccess)
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&p->per_sm_decode[1], jt_decode_kernel<CBN_JT_DECODE_SAMPLE>,
+                                                      warps * 32, p->smem);
   if (e != cudaSuccess) { cbn_jt_plan_destroy(p); return cbn_fail(ctx, CBN_ERR_CUDA, "JT plan: %s", cudaGetErrorString(e)); }
   p->per_sm = std::max(p->per_sm, 1);
+  for (int& k : p->per_sm_decode) k = std::max(k, 1);
   A.blob = p->d_blob;
   p->args = A;
   *out = p;
@@ -455,6 +637,53 @@ extern "C" int cbn_jt_run(cbn_ctx* ctx, const cbn_jt_plan* plan, const uint8_t* 
   const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(tiles, int64_t(ctx->sm_count) * plan->per_sm));
   // launched without programmatic dependent launch: acc may come from the count kernel right before it
   jt_kernel<<<blocks, plan->warps * 32, plan->smem, s>>>(A);
+  CBN_CHECK_LAUNCH(ctx);
+  return CBN_OK;
+}
+
+extern "C" int cbn_jt_decode(cbn_ctx* ctx, const cbn_jt_plan* plan, const uint8_t* codes, int64_t ld, int64_t n_rows,
+                             int32_t mode, uint64_t seed, int64_t first_row, int32_t n_draws, uint8_t* out_codes,
+                             int64_t out_ld, float* log_out, cbn_stream stream) {
+  if (!ctx) return cbn_fail(nullptr, CBN_ERR_INVALID, "cbn_jt_decode: ctx is NULL");
+  if (!plan || (mode != CBN_JT_DECODE_MAX && mode != CBN_JT_DECODE_SAMPLE))
+    return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_jt_decode: no plan, or mode is not CBN_JT_DECODE_MAX / CBN_JT_DECODE_SAMPLE");
+  if (n_draws < 1 || (mode == CBN_JT_DECODE_MAX && n_draws != 1))
+    return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_jt_decode: n_draws is %d (1 for CBN_JT_DECODE_MAX, at least 1 to sample)",
+                    n_draws);
+  if (first_row < 0 || n_rows < 0 || n_rows >= (int64_t(1) << 31))
+    return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_jt_decode: bad argument (first_row >= 0, 0 <= n_rows < 2^31)");
+  if (n_rows == 0) return CBN_OK;
+  if (!codes || ld < n_rows || (ld % 16) != 0 || !is_aligned(codes, 16))
+    return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_jt_decode: code matrix needs ld >= n_rows, ld %% 16 == 0, 16-byte aligned base");
+  if (!out_codes || out_ld < n_rows || (out_ld % 16) != 0 || !is_aligned(out_codes, 16))
+    return cbn_fail(ctx, CBN_ERR_INVALID,
+                    "cbn_jt_decode: output needs a pointer, out_ld >= n_rows, out_ld %% 16 == 0, 16-byte aligned base");
+  const int n_vars = plan->args.n_vars;
+  const uintptr_t c0 = uintptr_t(codes), c1 = c0 + uintptr_t(n_vars) * uintptr_t(ld);
+  const uintptr_t o0 = uintptr_t(out_codes), o1 = o0 + uintptr_t(n_draws) * uintptr_t(n_vars) * uintptr_t(out_ld);
+  if (o0 < c1 && c0 < o1) return cbn_fail(ctx, CBN_ERR_INVALID, "cbn_jt_decode: out_codes overlaps codes");
+  JtDecodeArgs D{};
+  D.a = plan->args;
+  D.a.codes = codes;
+  D.a.ld = ld;
+  D.a.n = n_rows;
+  D.a.marg = nullptr;
+  D.a.logp = log_out;
+  D.a.acc = nullptr;
+  D.out = out_codes;
+  D.out_ld = out_ld;
+  D.seed = seed;
+  D.first_row = first_row;
+  D.n_draws = n_draws;
+  DeviceGuard g(ctx->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t tiles = (n_rows + JT_TILE - 1) / JT_TILE;
+  const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(tiles, int64_t(ctx->sm_count) * plan->per_sm_decode[mode]));
+  // launched without programmatic dependent launch, as cbn_jt_run
+  if (mode == CBN_JT_DECODE_MAX)
+    jt_decode_kernel<CBN_JT_DECODE_MAX><<<blocks, plan->warps * 32, plan->smem, s>>>(D);
+  else
+    jt_decode_kernel<CBN_JT_DECODE_SAMPLE><<<blocks, plan->warps * 32, plan->smem, s>>>(D);
   CBN_CHECK_LAUNCH(ctx);
   return CBN_OK;
 }

@@ -201,6 +201,37 @@ class ExactInference(BaseInference):
         at = plan.schedule.node_out
         return {t.names[v]: marg[:, at[v]: at[v] + t.cards[v]] for v in ids}, log_evidence
 
+    def impute(self, evidence: Dict[str, torch.Tensor], method: str = "mpe", n_draws: int = 1, seed: int = 0,
+               first_row: int = 0):
+        """Completions of each row's unobserved cells, jointly consistent: ``(completed, log_prob)`` for ``method="mpe"``,
+        ``(draws, log_evidence)`` for ``method="sample"``.  ``evidence``: name -> tensor [n_rows] or [n_rows, 1] of
+        category VALUES, NaN where the row does not observe the node; a node without a column is unobserved in every row.
+        ``"mpe"``: ``completed`` maps EVERY node to float32 [n_rows] domain values, ``argmax_h P(h, e_row)`` filled in and
+        the observed cells unchanged; ``log_prob`` is float32 [n_rows] ``log max_h P(h, e_row)`` (natural log).
+        ``"sample"``: ``draws`` maps every node to float32 [n_draws, n_rows], each draw a joint sample of the row's
+        unobserved cells from ``P(h | e_row)``; ``log_evidence`` is float32 [n_rows] ``log P(e_row)``, the bits of
+        ``posterior_marginals``'.  Draw d of row i depends only on ``(seed, first_row + i, d)``.  A value outside the
+        fitted domain, or observed cells of probability zero, give -inf and NaN in every column.  No columns give one row.
+        One collect pass and one top-down decode of the junction tree per row (``cbn_jt_decode``).  Not part of the
+        reference's surface."""
+        if method not in ("mpe", "sample"):
+            raise ValueError(f"method must be 'mpe' or 'sample', got {method!r}")
+        if n_draws < 1 or (method == "mpe" and n_draws != 1):
+            raise ValueError(f"n_draws must be 1 for 'mpe' and at least 1 for 'sample', got {n_draws}")
+        if first_row < 0:
+            raise ValueError("first_row must not be negative")
+        t = self.tables
+        codes, nq = self.missing_codes(evidence)
+        plan = self.junction_tree().collect_plan()
+        nv = len(t.names)
+        out = t.new_code_matrix(nq, n_draws * nv)
+        log_out = torch.empty(nq, dtype=torch.float32, device=t.device)
+        mode = N.JT_DECODE_MAX if method == "mpe" else N.JT_DECODE_SAMPLE
+        plan.decode(codes, nq, mode, n_draws, seed, first_row, out, log_out)
+        if method == "mpe":
+            return {t.names[v]: self._values(v, out[v, :nq]) for v in range(nv)}, log_out
+        return {t.names[v]: self._values(v, out[v: n_draws * nv: nv, :nq]) for v in range(nv)}, log_out
+
     def infer_map(self, target_node: str, evidence: Dict[str, torch.Tensor]) -> Optional[torch.Tensor]:
         """MAP value of the target per row through the fused kernel (``cbn_ve_run_f32_map``); ``None`` when the plan is
         not a single-target gather plan with at most 8 target values (the caller then takes posterior + argmax)."""

@@ -15,6 +15,8 @@ evidence enters each row as indicators:
 ``cbn_jt_run`` (csrc/jt.cu) calibrates the tree per row by Shafer-Shenoy message passing: a collect pass towards the
 root (which yields ``log P(observed part of the row)``), a distribute pass towards the cliques that host an output, then
 every requested node marginal and, for EM, every family posterior of a row in which the family has a missing member.
+``cbn_jt_decode`` runs the collect pass only (sum- or max-product) and decodes the cliques top-down: the most probable
+completion of the row's missing cells, or joint draws of them; its plan is the collect-only schedule (UP and ROOT ops).
 Host work here is graph logic and int32 / int16 index tables only.
 
 Evidence codes per row: below the cardinality is observed, ``MISSING`` (254) is summed out, anything else makes the row
@@ -251,7 +253,10 @@ class Schedule:
 
 
 def build_schedule(st: Structure, nodes: Sequence[int], row_floats_budget: int = 5000,
-                   smem_budget: int = SMEM_BUDGET_BYTES) -> Schedule:
+                   smem_budget: int = SMEM_BUDGET_BYTES, collect_only: bool = False) -> Schedule:
+    """The per-row program with ``nodes`` as outputs; ``collect_only``: the UP ops and the ROOT op alone (no down
+    messages, ``nodes`` must be empty), the program ``cbn_jt_decode`` runs."""
+    assert not (collect_only and len(nodes)), "a collect-only schedule has no outputs"
     cards = st.cards
     nodes = list(nodes)
     n_cl = len(st.cliques)
@@ -273,7 +278,8 @@ def build_schedule(st: Structure, nodes: Sequence[int], row_floats_budget: int =
             msg += s
     # which down messages an output needs: every clique on the way from the root to its home
     need = [0] * n_cl
-    for bit, homes in ((NEED_NODES, [st.home[v] for v in nodes]), (NEED_FAMILIES, list(st.assign))):
+    outputs = () if collect_only else ((NEED_NODES, [st.home[v] for v in nodes]), (NEED_FAMILIES, list(st.assign)))
+    for bit, homes in outputs:
         for h in homes:
             while h >= 0 and not need[h] & bit:
                 need[h] |= bit
@@ -321,7 +327,7 @@ def build_schedule(st: Structure, nodes: Sequence[int], row_floats_budget: int =
         node_out[v] = run
         ops.append(op(NODE, st.home[v], [v], None, run))
         run += cards[v]
-    for v, fv in enumerate(st.family_vars):
+    for v, fv in enumerate([] if collect_only else st.family_vars):
         ops.append(op(FAMILY, st.assign[v], fv, None, v))
     scratch = max([o["out_size"] for o in ops if o["kind"] in (NODE, FAMILY)] + [1])
     sch = Schedule(st, ops, np.concatenate(maps) if maps else np.zeros(0, np.int16), msg, scratch, nodes, node_out, run)
@@ -391,6 +397,16 @@ class JTPlan:
         N.check(N.lib().cbn_jt_run(t.ctx.handle, self.handle, codes.data_ptr(), codes.stride(0), int(n_rows), ptr(marg_out),
                                    ptr(log_out), ptr(acc), N.stream_ptr(t.device)), t.ctx.handle)
 
+    def decode(self, codes, n_rows: int, mode: int, n_draws: int, seed: int, first_row: int, out_codes, log_out=None):
+        """``cbn_jt_decode``: ``codes`` as in ``run``; ``mode`` ``N.JT_DECODE_MAX`` or ``N.JT_DECODE_SAMPLE``;
+        ``out_codes``: uint8 [n_draws * n_vars, out_ld] (row ``d * n_vars + v``: draw d of variable v); ``log_out``: float32
+        [n_rows] or None."""
+        t = self.t
+        N.check(N.lib().cbn_jt_decode(t.ctx.handle, self.handle, codes.data_ptr(), codes.stride(0), int(n_rows), int(mode),
+                                      int(seed) & ((1 << 64) - 1), int(first_row), int(n_draws), out_codes.data_ptr(),
+                                      out_codes.stride(0), None if log_out is None else log_out.data_ptr(),
+                                      N.stream_ptr(t.device)), t.ctx.handle)
+
     def __del__(self):
         try:
             if self.handle is not None:
@@ -439,6 +455,12 @@ class JunctionTree:
             self._plans[key] = JTPlan(self, schedule_for(self.compiler, key))
         return self._plans[key]
 
+    def collect_plan(self) -> JTPlan:
+        """The plan of the collect-only schedule (``cbn_jt_decode``), cached like ``plan``."""
+        if "collect" not in self._plans:
+            self._plans["collect"] = JTPlan(self, collect_schedule(self.compiler))
+        return self._plans["collect"]
+
 
 def schedule_for(compiler, nodes: Optional[Sequence[int]] = None) -> Schedule:
     """The schedule of the compiler's network with ``nodes`` as outputs (default: every node).  It depends on the structure
@@ -454,6 +476,17 @@ def schedule_for(compiler, nodes: Optional[Sequence[int]] = None) -> Schedule:
         st = compiler.structures[base + (full,)].structure
         compiler.structures[base + (key,)] = build_schedule(st, key, compiler.row_temp_floats)
     return compiler.structures[base + (key,)]
+
+
+def collect_schedule(compiler) -> Schedule:
+    """The collect-only schedule (UP and ROOT ops; ``msg_floats`` counts the up messages only) of the compiler's network,
+    kept in ``compiler.structures`` beside the others.  The full schedule is built first, so the same budgets refuse a
+    network here as in ``posterior_marginals``."""
+    key = ("jt", tuple(compiler.t.cards), "collect")
+    if key not in compiler.structures:
+        st = schedule_for(compiler).structure
+        compiler.structures[key] = build_schedule(st, [], compiler.row_temp_floats, collect_only=True)
+    return compiler.structures[key]
 
 
 def compile_tree(compiler, dry: bool = False):

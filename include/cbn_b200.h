@@ -559,6 +559,41 @@ CBN_API int cbn_jt_run(cbn_ctx* ctx, const cbn_jt_plan* plan, const uint8_t* cod
                        float* marg_out, float* log_out, unsigned long long* acc, cbn_stream stream);
 CBN_API int cbn_jt_plan_stats(const cbn_jt_plan* plan, int64_t* smem_bytes, int32_t* warps_per_cta);
 
+/* ---- junction-tree decoding per row: the most probable completion, or joint posterior draws, of the missing cells -----
+ * Runs the plan's CBN_JT_UP ops and its CBN_JT_ROOT op as cbn_jt_run does (any plan; the ops after ROOT are not run, so a
+ * plan whose program ends at ROOT has the smallest footprint), then decodes the row top-down.
+ *   CBN_JT_DECODE_MAX: the fiber reduction of the collect is max instead of + (the shuffle tree too); log_out[r] is the
+ *     sum of the logs of the UP maxima plus the log of the ROOT maximum, log max_h P(h, e_row).  n_draws must be 1.
+ *   CBN_JT_DECODE_SAMPLE: log_out[r] is log P(e_row), bit-identical to cbn_jt_run's log_out on the same plan.  The collect
+ *     runs once per row; every draw restarts from the row's own codes.
+ * Decode order: the ROOT op's clique first, then the clique of every UP op in reverse program order (parents before
+ * children).  The weight of canonical cell c of a clique is psi[c] * ev(c) * prod_k m_k[map_k[c]] over the op's own inputs
+ * (the messages of the clique's children), multiplied in the collect's order, so each weight has the bits of its collect
+ * term; ev(c) tests the row's working codes: the observed cells plus every value fixed by the cliques decoded before.
+ * The chosen cell's digits are then fixed, so a child's separator is fixed when it is decoded; a clique with no unfixed
+ * member is skipped.
+ *   MAX: the cell of maximal weight, the smallest canonical index among equals.
+ *   SAMPLE: the first cell, in canonical order, whose inclusive cumulative weight is > u * total, so a cell of weight 0 is
+ *     never drawn.  Summation order: lane j of the row's warp sums the contiguous chunk [j * ceil(cells / 32), ..) in
+ *     order, the lane totals are combined by an inclusive Hillis-Steele shuffle scan, the first lane with a positive total
+ *     whose inclusive sum is > u * total rescans its chunk from the sum of the lanes before it.  If rounding leaves no
+ *     such cell, the last cell of positive weight of that chunk (of the last lane with a positive total, when no lane
+ *     qualifies).  u is cbn_psample_run's counter hash with the clique index in place of the variable:
+ *     h = splitmix64(splitmix64(splitmix64(seed ^ (first_row + r) * 0xD1B54A32D192ED03) ^ d * 0x9E6C63D0676A9A99) + clique),
+ *     u = (h >> 40) * 2^-24.  Draw d of row r depends only on (seed, first_row + r, d): a batch split through first_row or
+ *     a smaller n_draws gives the same bits.  The draws are not those of cbn_psample_run (another factorisation).
+ * Output: every variable v of draw d at out_codes[(d * n_vars + v) * out_ld + r] (uint8 codes; observed cells copied).  A
+ * dead row (a code neither below the cardinality nor CBN_MISSING, a collect maximum or ROOT value of 0, or, which exact
+ * arithmetic rules out, a clique of total weight 0 in the decode) gets -inf in log_out and CBN_UNSEEN in every column of
+ * every draw.  log_out is nullable.  CBN_ERR_INVALID for a bad mode, n_draws < 1 (or != 1 with MAX), first_row < 0,
+ * n_rows outside [0, 2^31), ld or out_ld below n_rows or not a multiple of 16 or an unaligned base, or out_codes NULL or
+ * overlapping codes.  Launched without programmatic dependent launch. */
+#define CBN_JT_DECODE_MAX 0
+#define CBN_JT_DECODE_SAMPLE 1
+CBN_API int cbn_jt_decode(cbn_ctx* ctx, const cbn_jt_plan* plan, const uint8_t* codes, int64_t ld, int64_t n_rows,
+                          int32_t mode, uint64_t seed, int64_t first_row, int32_t n_draws, uint8_t* out_codes,
+                          int64_t out_ld, float* log_out, cbn_stream stream);
+
 /* ---- ancestral sampling (synthetic workloads; BruteForce._sample's network analogue,
  * brute_force.py:246-265).  Counter-based: sample i of variable v depends only on
  * (seed, first_sample + i, v), so any sharding of the sample range yields the same data.
